@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c4|c5|c1|c2cn|mnist_img] [--precision fp32|tf32|bf16]
     python bench.py --impl reference ...      # the reference algorithm's CPU path (oracle port) on host cores
     python bench.py --workload c5 --sweep-full   # the 1 K - 64 M point sweep of BASELINE config 5 on its own
+    python bench.py --dump-outputs DIR ...       # also write the log-probs of the last timed step to DIR/log_prob.npy
 
 Contract (one JSON line on stdout, printed by rank 0): metric/value/unit/n_gpus/steps/warmup/ms_per_step/
 higher_is_better/scaling/vs_baseline/dtype/data/config + roofline, cpu_baseline, e2e, clocks, gpu_launches.
@@ -27,6 +28,7 @@ Besides the headline numbers the default line carries, so that the driver's N = 
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import subprocess
@@ -73,6 +75,25 @@ MODE_PRODUCTS = {"fp32": 3.0, "fp32_tf32": 6.0, "tf32": 2.0, "bf16": 1.0}   # te
 SWEEP_POINTS = [1 << 10, 1 << 13, 1 << 16, 1 << 19, 1 << 22, 1 << 26]      # C5: total points of one pass (all ranks)
 SWEEP_BLOCK = 1 << 16                                                       # rows generated on the device at a time
 SWEEP_DEFAULT_MAX_PER_GPU = 1 << 23                                         # default line: skip points above this per rank
+DUMP_MAX_BYTES = 64 << 20                                                   # --dump-outputs: all files together
+
+
+def dump_outputs(directory: str, arrays: dict) -> None:
+    """Writes each output as `directory/<name>.npy` in float32, so that two builds can be compared output for output.
+    An output too large for the budget is cut to a fixed, seeded sample of its rows; the chosen row indices go to
+    `<name>_rows.npy` (float64, exact for any row count that fits in memory)."""
+    import numpy as np
+    import torch
+    os.makedirs(directory, exist_ok=True)
+    budget = DUMP_MAX_BYTES // max(1, len(arrays))
+    for name, t in arrays.items():
+        a = t.detach().float().cpu()
+        if a.numel() * 4 > budget:
+            keep = budget // (a[0].numel() * 4 + 8)           # every kept row also stores its float64 index
+            rows = torch.randperm(a.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            a = a[rows]
+            np.save(os.path.join(directory, name + "_rows.npy"), rows.numpy().astype(np.float64))
+        np.save(os.path.join(directory, name + ".npy"), a.numpy())
 
 
 def algorithmic_flops_per_sample(spec) -> float:
@@ -137,8 +158,14 @@ class ClockSampler:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits",
                                           "-lms", "100", "-i", str(self.idx)], stdout=subprocess.PIPE, text=True)
             threading.Thread(target=self._pump, daemon=True).start()
+            atexit.register(self._end)            # a run that fails before stop() leaves no sampler behind
         except OSError:
             self.proc = None
+
+    def _end(self):
+        if self.proc.poll() is None:
+            self.proc.terminate()
+        self.proc.wait()
 
     def _pump(self):
         for line in self.proc.stdout:
@@ -147,7 +174,7 @@ class ClockSampler:
     def stop(self):
         if self.proc is None:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
-        self.proc.terminate()
+        self._end()
         sm, smax, reasons, power = [], None, set(), []
         for ln in self.lines:
             f = [x.strip() for x in ln.split(",")]
@@ -453,7 +480,11 @@ def main():
     ap.add_argument("--no-train", action="store_true", help="skip the C3 training leg")
     ap.add_argument("--no-extra", action="store_true", help="skip the C4 lines and the C5 sweep")
     ap.add_argument("--sweep-full", action="store_true", help="C5 sweep: run every point (64 M on one GPU takes ~2 min)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the log-probs of the last timed step (rank 0) to DIR/log_prob.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -539,7 +570,10 @@ def main():
         reprep.append(((t1 - t0) - (time.perf_counter() - t1)) * 1e3)
     prep_ms = sorted(reprep)[1]
 
-    step = lambda: flow.log_prob(x)                    # noqa: E731
+    last = {}
+
+    def step():
+        last["log_prob"] = flow.log_prob(x)
     for _ in range(args.warmup):
         step()
     sampler = ClockSampler(local_rank)
@@ -553,6 +587,8 @@ def main():
     if ranged:
         torch.cuda.profiler.stop()
     launches = ops.LAUNCHES
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last)
     if args.only_logprob:
         if rank == 0:
             sampler.stop()

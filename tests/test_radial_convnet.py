@@ -132,7 +132,9 @@ def test_training_pass_matches_oracle_gradients(fake_ops, name):
     loss = -training.log_prob_autograd(flow, x).mean()
     loss.backward()
     p = {k: v.clone().requires_grad_(v.is_floating_point()) for k, v in params.items()}
-    want_loss = -O.flow_log_prob(x, spec, p).mean()
+    # the oracle runs in float64: its float32 run can round a first-layer weight gradient off by ~1e-3 on its own, more
+    # than the tolerance below, depending on the CPU kernels of the torch build
+    want_loss = -O.flow_log_prob(x, spec, p, torch.float64).mean()
     want_loss.backward()
     assert abs(float(loss) - float(want_loss)) <= 2e-5 * max(1.0, abs(float(want_loss)))
     got = dict(flow.named_parameters())
