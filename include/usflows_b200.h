@@ -190,6 +190,28 @@ int usf_ingest_f16(const float* x, int64_t ldx, int64_t rows, int32_t d, const f
                    const float* sub, void* out_h16, void* out_l16, int64_t ld_16, int32_t* overflow_flag,
                    void* stream);
 
+/* 8-bit inputs (dequantisation of image data, the reference's DequantizedDataset: x = pixel / 256 + U(0, 1/256)).
+ * Value k in 0..255 at flat event index j (row-major over the event, e.g. c*H*W + h*W + w) of GLOBAL row r becomes
+ *   USF_DEQUANT_UNIFORM:  x = (k + u) / 256,  u = (2m + 1) / 2^16,  m = Philox4x32-10(key = seed, counter = (r, j >> 2))[j & 3] >> 17
+ *   USF_DEQUANT_MIDPOINT: x = (k + 0.5) / 256
+ * (counter words and rounds as usf_base_sample's).  Every x is exact in fp32 and lies strictly inside (k/256, (k+1)/256); the
+ * noise depends on (seed, r, j) only.  r = row0 + the row's index in the call; when dev_params (device memory, 2 x int64) is
+ * given, the kernel reads {seed, row base} there at run time: seed is replaced, row base is added to row0 (a captured graph
+ * can then be replayed with new values). */
+#define USF_DEQUANT_UNIFORM 0
+#define USF_DEQUANT_MIDPOINT 1
+typedef struct usf_dequant {
+  int32_t mode;
+  int32_t reserved0;
+  uint64_t seed;
+  int64_t row0;
+  const int64_t* dev_params;
+} usf_dequant;
+/* usf_ingest / usf_ingest_f16 reading 8-bit rows x [rows, ldx] (bytes): out = ((dequant(x) / div) * mul) - sub into every
+ * non-NULL plane of `out` (+ the fp16 range flag, may be NULL).  With only the fp32 plane it is the plain dequantisation. */
+int usf_ingest_u8(const uint8_t* x, int64_t ldx, int64_t rows, int32_t d, const usf_dequant* dq, const float* div,
+                  const float* mul, const float* sub, const usf_planes* out, int32_t* overflow_flag, void* stream);
+
 /* out[r] = sum_j logpdf_base(z[r,j]; loc[j], scale[j]) + add_const  (z = z_hi [+ z_lo]).
  * Replaces DistributionModule.log_prob (distributions.py:150-151; torch Laplace/Normal.log_prob +
  * Independent sum) and the `+ log_det` of Flow.log_prob (flows.py:234-245). */
@@ -247,6 +269,10 @@ int usf_gate_norm(const float* o, int64_t ldo, const float* xres, int64_t ldx, i
  * over [C, H, W] (transforms.py:105-125). */
 int usf_layout_transpose(const float* in, int64_t n, int32_t a, int32_t b, const float* scale, int32_t scale_mode,
                          int32_t scale_on_input, float* out, void* stream);
+/* the NCHW -> channels-last direction of usf_layout_transpose (A = c, B = hw, scale on the input side) reading 8-bit images
+ * in [n, c, hw], dequantised as usf_ingest_u8 does (j = c_index * hw + pixel, r = dq->row0 + image index) */
+int usf_layout_transpose_u8(const uint8_t* in, int64_t n, int32_t c, int32_t hw, const usf_dequant* dq, const float* scale,
+                            int32_t scale_mode, float* out, void* stream);
 /* Operand rows of a k x k convolution (stride 1, zero padding 'same', dilation) over channels-last rows:
  *   out[r, (kh*k + kw)*C + c] = g(in[pixel (h + (kh - k/2) dil, w + (kw - k/2) dil) of r's image, c]), 0 outside;
  *   g = optional multiply by mask[(h'*W + w')*C + c] (the coupling's x * mask, transforms.py:286), then optional ReLU.
@@ -422,6 +448,9 @@ int usf_flow_apply(const usf_plan* plan, const float* x, int64_t ldx, int64_t ro
 /* out[r] = log p(x[r, :]) = base.log_prob(stack(x[r, :])) + add_const   (Flow.log_prob, flows.py:225-245) */
 int usf_flow_logprob(const usf_plan* plan, const float* x, int64_t ldx, int64_t rows, float* out, int32_t* overflow_flag,
                      void* stream);
+/* the same for 8-bit rows x [rows, ldx] (bytes), dequantised as usf_ingest_u8 does by the plan's first ingest */
+int usf_flow_logprob_u8(const usf_plan* plan, const uint8_t* x, int64_t ldx, int64_t rows, const usf_dequant* dq, float* out,
+                        int32_t* overflow_flag, void* stream);
 int usf_plan_destroy(usf_plan* plan);
 
 /* ------------------------------------------------------------------------------------------------

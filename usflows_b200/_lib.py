@@ -85,6 +85,15 @@ class PlanLinear(C.Structure):
     ]
 
 
+class Dequant(C.Structure):
+    """Mirror of `usf_dequant` (include/usflows_b200.h)."""
+
+    _fields_ = [
+        ("mode", C.c_int32), ("reserved0", C.c_int32), ("seed", C.c_uint64), ("row0", C.c_int64), ("dev_params", C.c_void_p),
+    ]
+
+
+DEQUANT_UNIFORM, DEQUANT_MIDPOINT = 0, 1
 MODE_CODES = {"fp32": 0, "fp32_tf32": 1, "fp32_simt": 2, "tf32": 3, "bf16": 4}
 PLAN_SRC_STREAM, PLAN_SRC_HIDDEN = 0, 1
 PLAN_DST_STREAM, PLAN_DST_HIDDEN, PLAN_DST_SEGMENT = 0, 1, 2
@@ -117,6 +126,9 @@ SIGNATURES = {
     "usf_linear": (C.c_int, [C.POINTER(LinearArgs), _P]),
     "usf_ingest": (C.c_int, [_P, _I64, _I64, _I32, _P, _P, _P, _P, _I64, _P, _P, _I64, _P, _I64, _P]),
     "usf_ingest_f16": (C.c_int, [_P, _I64, _I64, _I32, _P, _P, _P, _P, _P, _I64, _P, _P]),
+    "usf_ingest_u8": (C.c_int, [_P, _I64, _I64, _I32, C.POINTER(Dequant), _P, _P, _P, C.POINTER(Planes), _P, _P]),
+    "usf_layout_transpose_u8": (C.c_int, [_P, _I64, _I32, _I32, C.POINTER(Dequant), _P, _I32, _P, _P]),
+    "usf_flow_logprob_u8": (C.c_int, [_P, _P, _I64, _I64, C.POINTER(Dequant), _P, _P, _P]),
     "usf_split_f16": (C.c_int, [_P, _I64, _I32, _I64, _P, _P, _I64, _P, _P]),
     "usf_base_logprob": (C.c_int, [_P, _P, _I64, _I64, _I32, _P, _P, _I32, _F, _P, _P]),
     "usf_flow_small": (C.c_int, [_P, _I64, _I64, _I32, _P, _I32, _P, _I32, _I32, _I32, _P, _I64, _P]),

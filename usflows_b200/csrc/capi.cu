@@ -111,6 +111,21 @@ int make_epilogue(const usf_linear_args* a, Epilogue* ep) {
 
 static inline cudaStream_t S(void* s) { return reinterpret_cast<cudaStream_t>(s); }
 
+static OutPlanes to_out_planes(const usf_planes* p, int32_t* overflow_flag) {
+  OutPlanes o{nullptr, nullptr, nullptr, nullptr, 0, 0, 0};
+  if (!p) return o;
+  o.f32 = p->f32; o.ld_f32 = p->ld_f32;
+  o.hi = p->hi; o.lo = p->lo; o.ld_split = p->ld_split;
+  o.bf16 = reinterpret_cast<__nv_bfloat16*>(p->bf16); o.ld_bf16 = p->ld_bf16;
+  o.h16 = reinterpret_cast<__half*>(p->h16); o.l16 = reinterpret_cast<__half*>(p->l16); o.ld_16 = p->ld_16;
+  o.overflow_flag = overflow_flag;
+  return o;
+}
+
+static inline bool dequant_ok(const usf_dequant* dq) {
+  return dq && (dq->mode == USF_DEQUANT_UNIFORM || dq->mode == USF_DEQUANT_MIDPOINT);
+}
+
 // Scope in which this thread's stream-capture interaction mode is "relaxed", so an allocation / release issued while the
 // thread happens to be capturing a CUDA graph neither fails nor invalidates the capture.
 struct RelaxedCaptureMode {
@@ -217,9 +232,9 @@ int usf_ingest(const float* x, int64_t ldx, int64_t rows, int32_t d, const float
   const bool vec = planes_vec_ok(o) && aligned16(x) && ldx % 4 == 0 && d % 4 == 0 && (!dv || aligned16(dv)) &&
                    (!mul || aligned16(mul)) && (!sub || aligned16(sub)) && (!out_bf16 || d % 8 == 0 || true);
   if (vec)
-    USF_CUDA_OK(launch_chain(ingest_kernel<true>, dim3(ew_grid(rows * (d / 4), 256)), dim3(256), 0, S(stream), x, (long long)ldx, (long long)rows, (int)d, dv, mul, sub, o));
+    USF_CUDA_OK(launch_chain(ingest_kernel<true, LoadF32>, dim3(ew_grid(rows * (d / 4), 256)), dim3(256), 0, S(stream), LoadF32{x, (long long)ldx}, (long long)rows, (int)d, dv, mul, sub, o));
   else
-    USF_CUDA_OK(launch_chain(ingest_kernel<false>, dim3(ew_grid(rows * d, 256)), dim3(256), 0, S(stream), x, (long long)ldx, (long long)rows, (int)d, dv, mul, sub, o));
+    USF_CUDA_OK(launch_chain(ingest_kernel<false, LoadF32>, dim3(ew_grid(rows * d, 256)), dim3(256), 0, S(stream), LoadF32{x, (long long)ldx}, (long long)rows, (int)d, dv, mul, sub, o));
   USF_CUDA_OK(cudaGetLastError());
   return USF_OK;
 }
@@ -236,9 +251,29 @@ int usf_ingest_f16(const float* x, int64_t ldx, int64_t rows, int32_t d, const f
   const bool vec = planes_vec_ok(o) && aligned16(x) && ldx % 4 == 0 && d % 4 == 0 && (!dv || aligned16(dv)) &&
                    (!mul || aligned16(mul)) && (!sub || aligned16(sub));
   if (vec)
-    USF_CUDA_OK(launch_chain(ingest_kernel<true>, dim3(ew_grid(rows * (d / 4), 256)), dim3(256), 0, S(stream), x, (long long)ldx, (long long)rows, (int)d, dv, mul, sub, o));
+    USF_CUDA_OK(launch_chain(ingest_kernel<true, LoadF32>, dim3(ew_grid(rows * (d / 4), 256)), dim3(256), 0, S(stream), LoadF32{x, (long long)ldx}, (long long)rows, (int)d, dv, mul, sub, o));
   else
-    USF_CUDA_OK(launch_chain(ingest_kernel<false>, dim3(ew_grid(rows * d, 256)), dim3(256), 0, S(stream), x, (long long)ldx, (long long)rows, (int)d, dv, mul, sub, o));
+    USF_CUDA_OK(launch_chain(ingest_kernel<false, LoadF32>, dim3(ew_grid(rows * d, 256)), dim3(256), 0, S(stream), LoadF32{x, (long long)ldx}, (long long)rows, (int)d, dv, mul, sub, o));
+  USF_CUDA_OK(cudaGetLastError());
+  return USF_OK;
+}
+
+int usf_ingest_u8(const uint8_t* x, int64_t ldx, int64_t rows, int32_t d, const usf_dequant* dq, const float* dv,
+                  const float* mul, const float* sub, const usf_planes* out, int32_t* overflow_flag, void* stream) {
+  USF_REQUIRE(x && out && rows >= 0 && d > 0 && ldx >= d, "bad input");
+  USF_REQUIRE(dequant_ok(dq), "bad dequantisation (null, or mode not USF_DEQUANT_UNIFORM / USF_DEQUANT_MIDPOINT)");
+  USF_REQUIRE((out->hi == nullptr) == (out->lo == nullptr) && (out->h16 == nullptr) == (out->l16 == nullptr), "planes come as pairs");
+  USF_REQUIRE(out->f32 || out->hi || out->bf16 || out->h16, "usf_ingest_u8 needs an output plane");
+  if (rows == 0) return USF_OK;
+  const OutPlanes o = to_out_planes(out, overflow_flag);
+  const LoadU8 in{x, (long long)ldx, (unsigned long long)dq->seed, (long long)dq->row0,
+                  reinterpret_cast<const long long*>(dq->dev_params), (int)dq->mode};
+  const bool vec = planes_vec_ok(o) && (reinterpret_cast<uintptr_t>(x) & 3u) == 0 && ldx % 4 == 0 && d % 4 == 0 &&
+                   (!dv || aligned16(dv)) && (!mul || aligned16(mul)) && (!sub || aligned16(sub));
+  if (vec)
+    USF_CUDA_OK(launch_chain(ingest_kernel<true, LoadU8>, dim3(ew_grid(rows * (d / 4), 256)), dim3(256), 0, S(stream), in, (long long)rows, (int)d, dv, mul, sub, o));
+  else
+    USF_CUDA_OK(launch_chain(ingest_kernel<false, LoadU8>, dim3(ew_grid(rows * d, 256)), dim3(256), 0, S(stream), in, (long long)rows, (int)d, dv, mul, sub, o));
   USF_CUDA_OK(cudaGetLastError());
   return USF_OK;
 }
@@ -320,17 +355,6 @@ int usf_radial_sample(int64_t rows, int32_t d, const float* loc, int32_t p_kind,
   return USF_OK;
 }
 
-static OutPlanes to_out_planes(const usf_planes* p, int32_t* overflow_flag) {
-  OutPlanes o{nullptr, nullptr, nullptr, nullptr, 0, 0, 0};
-  if (!p) return o;
-  o.f32 = p->f32; o.ld_f32 = p->ld_f32;
-  o.hi = p->hi; o.lo = p->lo; o.ld_split = p->ld_split;
-  o.bf16 = reinterpret_cast<__nv_bfloat16*>(p->bf16); o.ld_bf16 = p->ld_bf16;
-  o.h16 = reinterpret_cast<__half*>(p->h16); o.l16 = reinterpret_cast<__half*>(p->l16); o.ld_16 = p->ld_16;
-  o.overflow_flag = overflow_flag;
-  return o;
-}
-
 int usf_gate_norm(const float* o, int64_t ldo, const float* xres, int64_t ldx, int64_t rows, int32_t n, int32_t gated,
                   int32_t pre_relu, const float* gamma, const float* beta, float eps, float* y_f32, int64_t ldy, const usf_planes* act,
                   int32_t act_relu, const usf_planes* raw, int32_t* overflow_flag, void* stream) {
@@ -369,7 +393,21 @@ int usf_layout_transpose(const float* in, int64_t n, int32_t a, int32_t b, const
   USF_REQUIRE(scale_mode >= 0 && scale_mode <= 2 && (scale_mode == 0 || scale), "scale_mode 0 (none), 1 (multiply) or 2 (divide)");
   if (n == 0) return USF_OK;
   const long long tiles = (long long)n * ((a + 31) / 32) * ((b + 31) / 32);
-  layout_kernel<<<ew_grid(tiles * 256, 256), 256, 0, S(stream)>>>(in, n, a, b, scale, scale_mode, scale_on_input, out);
+  layout_kernel<float><<<ew_grid(tiles * 256, 256), 256, 0, S(stream)>>>(in, n, a, b, scale, scale_mode, scale_on_input, out,
+                                                                         LayoutU8{0, 0, nullptr, 0});
+  USF_CUDA_OK(cudaGetLastError());
+  return USF_OK;
+}
+
+int usf_layout_transpose_u8(const uint8_t* in, int64_t n, int32_t c, int32_t hw, const usf_dequant* dq, const float* scale,
+                            int32_t scale_mode, float* out, void* stream) {
+  USF_REQUIRE(in && out && n >= 0 && c > 0 && hw > 0, "bad input");
+  USF_REQUIRE(dequant_ok(dq), "bad dequantisation (null, or mode not USF_DEQUANT_UNIFORM / USF_DEQUANT_MIDPOINT)");
+  USF_REQUIRE(scale_mode >= 0 && scale_mode <= 2 && (scale_mode == 0 || scale), "scale_mode 0 (none), 1 (multiply) or 2 (divide)");
+  if (n == 0) return USF_OK;
+  const long long tiles = (long long)n * ((c + 31) / 32) * ((hw + 31) / 32);
+  layout_kernel<uint8_t><<<ew_grid(tiles * 256, 256), 256, 0, S(stream)>>>(
+      in, n, c, hw, scale, scale_mode, 1, out, LayoutU8{dq->seed, dq->row0, reinterpret_cast<const long long*>(dq->dev_params), dq->mode});
   USF_CUDA_OK(cudaGetLastError());
   return USF_OK;
 }
@@ -680,13 +718,24 @@ int usf_plan_finalize(usf_plan* p) {
 
 int usf_flow_apply(const usf_plan* p, const float* x, int64_t ldx, int64_t rows, float* z, int64_t ldz, int32_t* overflow_flag,
                    void* stream) {
-  return plan_run(p, x, ldx, rows, z, ldz, overflow_flag, stream);
+  return plan_run(p, PlanInput{x, nullptr, nullptr}, ldx, rows, z, ldz, overflow_flag, stream);
 }
 
 int usf_flow_logprob(const usf_plan* p, const float* x, int64_t ldx, int64_t rows, float* out, int32_t* overflow_flag,
                      void* stream) {
   USF_REQUIRE(p && p->finalized && p->base_kind >= 0 && out, "plan without a base density (usf_plan_set_base)");
-  int rc = plan_run(p, x, ldx, rows, p->fin, p->ld_fin, overflow_flag, stream);
+  int rc = plan_run(p, PlanInput{x, nullptr, nullptr}, ldx, rows, p->fin, p->ld_fin, overflow_flag, stream);
+  if (rc) return rc;
+  return usf_base_logprob(p->fin, nullptr, p->ld_fin, rows, p->out_width, p->loc, p->scale, p->base_kind, p->add_const, out,
+                          stream);
+}
+
+int usf_flow_logprob_u8(const usf_plan* p, const uint8_t* x, int64_t ldx, int64_t rows, const usf_dequant* dq, float* out,
+                        int32_t* overflow_flag, void* stream) {
+  USF_REQUIRE(p && p->finalized && p->base_kind >= 0 && out, "plan without a base density (usf_plan_set_base)");
+  USF_REQUIRE(x && ldx >= p->d_in, "bad input (x null or ldx < d_in)");
+  USF_REQUIRE(dequant_ok(dq), "bad dequantisation (null, or mode not USF_DEQUANT_UNIFORM / USF_DEQUANT_MIDPOINT)");
+  int rc = plan_run(p, PlanInput{nullptr, x, dq}, ldx, rows, p->fin, p->ld_fin, overflow_flag, stream);
   if (rc) return rc;
   return usf_base_logprob(p->fin, nullptr, p->ld_fin, rows, p->out_width, p->loc, p->scale, p->base_kind, p->add_const, out,
                           stream);

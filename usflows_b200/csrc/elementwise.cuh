@@ -105,21 +105,90 @@ inline bool planes_vec_ok(const OutPlanes& o) {
   return ok;
 }
 
+// ---- Philox4x32-10 (base sampling, dequantisation noise) ------------------------------------------------------------------
+__device__ __forceinline__ void philox_round(uint32_t (&c)[4], uint32_t k0, uint32_t k1) {
+  const uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
+  const uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
+  const uint32_t n0 = hi1 ^ c[1] ^ k0, n1 = lo1, n2 = hi0 ^ c[3] ^ k1, n3 = lo0;
+  c[0] = n0; c[1] = n1; c[2] = n2; c[3] = n3;
+}
+__device__ __forceinline__ void philox4x32_10(uint64_t seed, uint64_t ctr_lo, uint64_t ctr_hi, uint32_t (&out)[4]) {
+  uint32_t c[4] = {(uint32_t)ctr_lo, (uint32_t)(ctr_lo >> 32), (uint32_t)ctr_hi, (uint32_t)(ctr_hi >> 32)};
+  uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
+#pragma unroll
+  for (int i = 0; i < 10; ++i) {
+    philox_round(c, k0, k1);
+    k0 += 0x9E3779B9u;
+    k1 += 0xBB67AE85u;
+  }
+  out[0] = c[0]; out[1] = c[1]; out[2] = c[2]; out[3] = c[3];
+}
+// ---- 8-bit dequantisation (usf_dequant) -----------------------------------------------------------------
+// Value k in 0..255 at flat event index j of GLOBAL row r becomes x = (k + u) / 256 with u = (2m + 1) / 2^16,
+// m = Philox4x32-10(key = seed, counter = (r, j >> 2))[j & 3] >> 17 (15 bits), or u = 1/2 for the midpoint mode.
+// k * 2^16 + (2m + 1) < 2^24, so x is exact in fp32 and lies strictly inside (k/256, (k+1)/256); the noise depends on
+// (seed, r, j) only, so chunking, graph replay and sharding cannot change a bit.
+__device__ __forceinline__ float dequant_value(uint32_t k, uint32_t rnd, int mode) {
+  const uint32_t low = mode == USF_DEQUANT_MIDPOINT ? 0x8000u : (((rnd >> 17) << 1) | 1u);
+  return (float)((k << 16) | low) * (1.0f / 16777216.0f);
+}
+// out[i] with a run-time i in 0..3, kept in registers (an indexed load would put the array in local memory)
+__device__ __forceinline__ uint32_t pick4(const uint32_t (&out)[4], int i) {
+  return i == 0 ? out[0] : i == 1 ? out[1] : i == 2 ? out[2] : out[3];
+}
+
+// input loaders of ingest_kernel: fp32 rows, or 8-bit rows dequantised on the fly
+struct LoadF32 {
+  const float* x;
+  long long ldx;
+  __device__ __forceinline__ void init() {}
+  __device__ __forceinline__ void load4(long long r, int j, float (&v)[4]) const {
+    const float4 t = __ldcs(reinterpret_cast<const float4*>(x + r * ldx + j));
+    v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
+  }
+  __device__ __forceinline__ float load1(long long r, int j) const { return __ldg(x + r * ldx + j); }
+};
+struct LoadU8 {
+  const uint8_t* x;
+  long long ldx;
+  unsigned long long seed;
+  long long row0;                  // global row of local row 0
+  const long long* params;         // optional device {seed, row base}: replaces seed, adds to row0
+  int mode;
+  __device__ __forceinline__ void init() {
+    if (params) { seed = (unsigned long long)__ldg(params); row0 += __ldg(params + 1); }
+  }
+  // j % 4 == 0: one 4-byte load and one Philox call for 4 elements
+  __device__ __forceinline__ void load4(long long r, int j, float (&v)[4]) const {
+    const uint32_t k = __ldcs(reinterpret_cast<const unsigned int*>(x + r * ldx + j));
+    uint32_t rnd[4] = {0u, 0u, 0u, 0u};
+    if (mode != USF_DEQUANT_MIDPOINT) philox4x32_10(seed, (uint64_t)(row0 + r), (uint64_t)(j >> 2), rnd);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) v[i] = dequant_value((k >> (8 * i)) & 0xFFu, rnd[i], mode);
+  }
+  __device__ __forceinline__ float load1(long long r, int j) const {
+    uint32_t rnd[4] = {0u, 0u, 0u, 0u};
+    if (mode != USF_DEQUANT_MIDPOINT) philox4x32_10(seed, (uint64_t)(row0 + r), (uint64_t)(j >> 2), rnd);
+    return dequant_value(x[r * ldx + j], pick4(rnd, j & 3), mode);
+  }
+};
+
 // ---- ingest: out = ((x / div) * mul) - sub --------------------------------------------------------
-template <bool VEC>
+template <bool VEC, class Load>
 __global__ void __launch_bounds__(256)
-ingest_kernel(const float* __restrict__ x, long long ldx, long long rows, int d, const float* __restrict__ dv,
+ingest_kernel(Load in, long long rows, int d, const float* __restrict__ dv,
               const float* __restrict__ mul, const float* __restrict__ sub, OutPlanes o) {
   griddep_launch_dependents();
   griddep_wait();
+  in.init();
   if (VEC) {
     const int d4 = d >> 2;
     const long long total = rows * d4;
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
       const long long r = i / d4;
       const int j = (int)(i - r * d4) * 4;
-      float4 t = __ldcs(reinterpret_cast<const float4*>(x + r * ldx + j));
-      float v[4] = {t.x, t.y, t.z, t.w};
+      float v[4];
+      in.load4(r, j, v);
       if (dv) { float4 s = __ldg(reinterpret_cast<const float4*>(dv + j)); v[0] = v[0] / s.x; v[1] = v[1] / s.y; v[2] = v[2] / s.z; v[3] = v[3] / s.w; }
       if (mul) { float4 s = __ldg(reinterpret_cast<const float4*>(mul + j)); v[0] *= s.x; v[1] *= s.y; v[2] *= s.z; v[3] *= s.w; }
       if (sub) { float4 s = __ldg(reinterpret_cast<const float4*>(sub + j)); v[0] -= s.x; v[1] -= s.y; v[2] -= s.z; v[3] -= s.w; }
@@ -130,7 +199,7 @@ ingest_kernel(const float* __restrict__ x, long long ldx, long long rows, int d,
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
       const long long r = i / d;
       const int j = (int)(i - r * d);
-      float v = x[r * ldx + j];
+      float v = in.load1(r, j);
       if (dv) v = v / __ldg(dv + j);
       if (mul) v *= __ldg(mul + j);
       if (sub) v -= __ldg(sub + j);
@@ -183,24 +252,7 @@ base_logprob_kernel(const float* __restrict__ z, const float* __restrict__ z_lo,
   }
 }
 
-// ---- Philox4x32-10 base sampling ------------------------------------------------------------------
-__device__ __forceinline__ void philox_round(uint32_t (&c)[4], uint32_t k0, uint32_t k1) {
-  const uint32_t hi0 = __umulhi(0xD2511F53u, c[0]), lo0 = 0xD2511F53u * c[0];
-  const uint32_t hi1 = __umulhi(0xCD9E8D57u, c[2]), lo1 = 0xCD9E8D57u * c[2];
-  const uint32_t n0 = hi1 ^ c[1] ^ k0, n1 = lo1, n2 = hi0 ^ c[3] ^ k1, n3 = lo0;
-  c[0] = n0; c[1] = n1; c[2] = n2; c[3] = n3;
-}
-__device__ __forceinline__ void philox4x32_10(uint64_t seed, uint64_t ctr_lo, uint64_t ctr_hi, uint32_t (&out)[4]) {
-  uint32_t c[4] = {(uint32_t)ctr_lo, (uint32_t)(ctr_lo >> 32), (uint32_t)ctr_hi, (uint32_t)(ctr_hi >> 32)};
-  uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
-#pragma unroll
-  for (int i = 0; i < 10; ++i) {
-    philox_round(c, k0, k1);
-    k0 += 0x9E3779B9u;
-    k1 += 0xBB67AE85u;
-  }
-  out[0] = c[0]; out[1] = c[1]; out[2] = c[2]; out[3] = c[3];
-}
+// ---- base sampling --------------------------------------------------------------------------------------
 // 23 random bits + 1/2: every value is exactly representable in fp32, so the result stays inside (0,1)
 // (24 bits + 1/2 would round up to 1.0 for the top value and give log1p(-1) = -inf in the Laplace inverse CDF)
 __device__ __forceinline__ float u01_open(uint32_t x) { return ((float)(x >> 9) + 0.5f) * (1.0f / 8388608.0f); }

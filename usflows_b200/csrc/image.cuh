@@ -16,10 +16,20 @@ namespace usf {
 // out[n, b, a] = f(in[n, a, b]) for in [N, A, B];  f multiplies / divides by s indexed in the order of the NCHW side:
 // s_on_input != 0: s[a * B + b] (the input is NCHW: A = C, B = HW), else s[b * A + a] (the output is NCHW: B = C, A = HW).
 // 32 x 32 shared-memory tiles, both global accesses coalesced; 1-D grid-stride loop over (n, tile_a, tile_b).
+// A uint8 input (NCHW side) is dequantised as it is read: element a * B + b of image n is event index j of global row
+// dq.row0 + n (dequant_value, one Philox call per element: neighbours in a tile row may belong to different counters).
+struct LayoutU8 {
+  unsigned long long seed;
+  long long row0;
+  const long long* params;
+  int mode;
+};
+template <class T>
 __global__ void __launch_bounds__(256)
-layout_kernel(const float* __restrict__ in, long long N, int A, int B, const float* __restrict__ s, int s_mode, int s_on_input,
-              float* __restrict__ out) {
+layout_kernel(const T* __restrict__ in, long long N, int A, int B, const float* __restrict__ s, int s_mode, int s_on_input,
+              float* __restrict__ out, LayoutU8 dq) {
   __shared__ float tile[32][33];
+  if (sizeof(T) == 1 && dq.params) { dq.seed = (unsigned long long)__ldg(dq.params); dq.row0 += __ldg(dq.params + 1); }
   const int ta = (A + 31) >> 5, tb = (B + 31) >> 5;
   const long long tiles = N * ta * tb;
   const int tx = threadIdx.x & 31, ty = threadIdx.x >> 5;      // 32 x 8
@@ -27,14 +37,21 @@ layout_kernel(const float* __restrict__ in, long long N, int A, int B, const flo
     const long long n = t / (ta * tb);
     const int rem = (int)(t - n * (ta * tb));
     const int a0 = (rem / tb) << 5, b0 = (rem % tb) << 5;
-    const float* src = in + n * (long long)A * B;
+    const T* src = in + n * (long long)A * B;
     float* dst = out + n * (long long)A * B;
 #pragma unroll
     for (int i = 0; i < 32; i += 8) {
       const int a = a0 + ty + i, b = b0 + tx;
       float v = 0.f;
       if (a < A && b < B) {
-        v = src[(long long)a * B + b];
+        const long long j = (long long)a * B + b;
+        if (sizeof(T) == 1) {
+          uint32_t rnd[4] = {0u, 0u, 0u, 0u};
+          if (dq.mode != USF_DEQUANT_MIDPOINT) philox4x32_10(dq.seed, (uint64_t)(dq.row0 + n), (uint64_t)(j >> 2), rnd);
+          v = dequant_value((uint32_t)src[j], pick4(rnd, (int)(j & 3)), dq.mode);
+        } else {
+          v = (float)src[j];
+        }
         if (s_mode) {
           const float f = __ldg(s + (s_on_input ? (long long)a * B + b : (long long)b * A + a));
           v = s_mode == 1 ? v * f : v / f;

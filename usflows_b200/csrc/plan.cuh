@@ -109,16 +109,24 @@ inline int plan_ingest(const float* x, int64_t ldx, int64_t rows, int32_t d, con
   return usf_ingest(x, ldx, rows, d, nullptr, nullptr, nullptr, o.f32, o.ld_f32, o.hi, o.lo, o.ld_split, o.bf16, o.ld_bf16, stream);
 }
 
+// the caller's rows: fp32, or 8-bit values with their dequantisation (then step 0 always ingests: no fp32 tensor to read)
+struct PlanInput {
+  const float* f32;
+  const uint8_t* u8;
+  const usf_dequant* dq;
+};
+
 // runs the contraction chain; the last step writes fp32 into (z_out, ldz)
-inline int plan_run(const usf_plan* p, const float* x, int64_t ldx, int64_t rows, float* z_out, int64_t ldz, int32_t* flag,
+inline int plan_run(const usf_plan* p, PlanInput in, int64_t ldx, int64_t rows, float* z_out, int64_t ldz, int32_t* flag,
                     void* stream) {
   USF_REQUIRE(p && p->finalized, "plan not finalized");
-  USF_REQUIRE(x && z_out && rows >= 0 && rows <= p->max_rows, "bad input (rows must not exceed the plan's max_rows)");
+  USF_REQUIRE((in.f32 || in.u8) && z_out && rows >= 0 && rows <= p->max_rows, "bad input (rows must not exceed the plan's max_rows)");
   if (rows == 0) return USF_OK;
   const int mode = p->mode;
+  const float* x = in.f32;
   usf_planes src;
   memset(&src, 0, sizeof(src));
-  src.f32 = const_cast<float*>(x);
+  src.f32 = const_cast<float*>(x);           // NULL for 8-bit rows: no plane satisfies a consumer, so they are ingested
   src.ld_f32 = ldx;
   usf_planes cur = src, hid;
   memset(&hid, 0, sizeof(hid));
@@ -134,7 +142,7 @@ inline int plan_run(const usf_plan* p, const float* x, int64_t ldx, int64_t rows
       const int need = in_coupling ? stream_planes(mode) : operand_planes(mode);
       const bool direct_ok = st.engine == USF_ENGINE_SIMT || (aligned16(x) && ldx % 4 == 0);
       if (!has_planes(cur, need) || (cur_is_src && !direct_ok)) {
-        USF_REQUIRE(cur.f32 != nullptr, "internal: activation has no fp32 plane to re-encode from");
+        USF_REQUIRE(cur.f32 != nullptr || (cur_is_src && in.u8), "internal: activation has no fp32 plane to re-encode from");
         xf ^= 1;
         usf_planes b = p->x[xf];
         // only the planes this consumer needs
@@ -142,7 +150,8 @@ inline int plan_run(const usf_plan* p, const float* x, int64_t ldx, int64_t rows
         if (!(need & 2)) { b.hi = b.lo = nullptr; }
         if (!(need & 4)) { b.bf16 = nullptr; }
         if (!(need & 8)) { b.h16 = b.l16 = nullptr; }
-        int rc = plan_ingest(cur.f32, cur.ld_f32, rows, cur_width, b, flag, stream);
+        int rc = cur_is_src && in.u8 ? usf_ingest_u8(in.u8, ldx, rows, cur_width, in.dq, nullptr, nullptr, nullptr, &b, flag, stream)
+                                     : plan_ingest(cur.f32, cur.ld_f32, rows, cur_width, b, flag, stream);
         if (rc) return rc;
         cur = b;
         cur_is_src = false;

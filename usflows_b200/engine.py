@@ -540,10 +540,12 @@ class Program:
 
     def run(self, x: torch.Tensor, mode: Optional[str] = None, chunk_rows: Optional[int] = None,
             out: Optional[torch.Tensor] = None, sink=None,
-            flag_out: Optional[torch.Tensor] = None, ladj_rows: Optional[torch.Tensor] = None) -> Optional[torch.Tensor]:
+            flag_out: Optional[torch.Tensor] = None, ladj_rows: Optional[torch.Tensor] = None,
+            dq: Optional[ops.Dequant] = None) -> Optional[torch.Tensor]:
         """Evaluate the program on x [rows, d].  With `sink`, the final stream value of each chunk is handed
-        to `sink(chunk_f32 [r, width], r0, r1)` from a reused workspace buffer instead of being stored."""
-        ops.require_cuda(x, "input")
+        to `sink(chunk_f32 [r, width], r0, r1)` from a reused workspace buffer instead of being stored.  With `dq`, x is
+        uint8 and its first ingest dequantises it (ops.Dequant)."""
+        ops.require_cuda(x, "input", torch.float32 if dq is None else torch.uint8)
         if x.dim() != 2:
             raise RuntimeError("usflows_b200: expected a [rows, d] input")
         x = x.contiguous()
@@ -551,6 +553,8 @@ class Program:
         width = self.out_width(x.shape[1])
         if rows == 0:                       # empty batch: nothing to launch
             return None if sink is not None else torch.empty(0, width, dtype=torch.float32, device=x.device)
+        if dq is not None and self.small is not None and x.shape[1] == self.small["d"]:
+            x, dq = _dequantized(x, dq), None                   # one launch for the whole stack: it reads fp32
         if self.small is not None and x.shape[1] == self.small["d"]:
             sm = self.small
             res = out if (out is not None and sink is None) else torch.empty(rows, sm["d"], dtype=torch.float32, device=x.device)
@@ -560,7 +564,7 @@ class Program:
                 return None
             return res
         if self.force_fallback:
-            return self._fallback().run(x, chunk_rows=chunk_rows, out=out, sink=sink, ladj_rows=ladj_rows)
+            return self._fallback().run(x, chunk_rows=chunk_rows, out=out, sink=sink, ladj_rows=ladj_rows, dq=dq)
         cap = chunk_rows or _default_chunk_rows
         n_chunks = (rows + cap - 1) // cap
         chunk = min(rows, ((rows + n_chunks - 1) // n_chunks + 255) // 256 * 256)
@@ -573,12 +577,13 @@ class Program:
             r1 = min(rows, r0 + chunk)
             flag = flags[ci:ci + 1] if own_flags else flag_out
             lr = None if ladj_rows is None else ladj_rows[r0:r1]
+            cdq = None if dq is None else dq.shifted(r0)
             if sink is not None:
                 fin = _workspace.planes(x.device, "final", r1 - r0, width, "f32")
-                self._run_chunk(x[r0:r1], fin, flag, lr)
+                self._run_chunk(x[r0:r1], fin, flag, lr, cdq)
                 sink(fin, r0, r1)
             else:
-                self._run_chunk(x[r0:r1], out[r0:r1], flag, lr)
+                self._run_chunk(x[r0:r1], out[r0:r1], flag, lr, cdq)
         if own_flags:
             # one device->host read per call: chunks whose activations left the fp16 range are recomputed with the
             # tf32-split engine (same accuracy class, no range limit)
@@ -589,12 +594,13 @@ class Program:
                 lr = None if ladj_rows is None else ladj_rows[r0:r1]
                 if lr is not None:
                     lr.zero_()                                  # the abandoned pass already added its log-scales
+                cdq = None if dq is None else dq.shifted(r0)
                 if sink is not None:
                     fin = _workspace.planes(x.device, "final", r1 - r0, width, "f32")
-                    fb._run_chunk(x[r0:r1], fin, None, lr)
+                    fb._run_chunk(x[r0:r1], fin, None, lr, cdq)
                     sink(fin, r0, r1)
                 else:
-                    fb._run_chunk(x[r0:r1], out[r0:r1], None, lr)
+                    fb._run_chunk(x[r0:r1], out[r0:r1], None, lr, cdq)
         return None if sink is not None else out
 
     def _stream_planes(self) -> set:
@@ -604,7 +610,8 @@ class Program:
         return {"fp32": {"h16", "l16"}, "fp32_tf32": {"hi", "lo"}, "bf16": {"bf16"}}.get(self.mode, {"f32"})
 
     def _run_chunk(self, x: torch.Tensor, final_out: torch.Tensor, flag: Optional[torch.Tensor] = None,
-                   ladj_rows: Optional[torch.Tensor] = None) -> None:
+                   ladj_rows: Optional[torch.Tensor] = None, dq: Optional[ops.Dequant] = None) -> None:
+        """One chunk x [rows, d]; with `dq`, x is uint8 and is dequantised by the first kernel that reads it."""
         dev, rows = x.device, x.shape[0]
         steps = self.steps
         flip = {"x": 0, "h": 0}
@@ -632,8 +639,18 @@ class Program:
                     setattr(v, pl, t[:, c0:c0 + w])
             return v
 
-        src_f32 = Act(rows, x.shape[1], f32=x)   # the user's tensor: read-only
+        def ingest(src: Act, out: Act, **kw) -> None:
+            if src is src_f32 and dq is not None:
+                ops.ingest_u8(x, dq, out, **kw)
+            else:
+                ops.ingest(src.f32, out, **kw)
+
+        # the user's tensor: read-only.  8-bit rows have no plane a consumer could read: the first step ingests them
+        src_f32 = Act(rows, x.shape[1], f32=x if dq is None else None)
         cur = src_f32
+        if dq is not None and steps and steps[0].kind in ("leaky", "permute"):    # kernels that read fp32 only
+            cur = new_act("x", x.shape[1], {"f32"})
+            ingest(src_f32, cur)
         for i, st in enumerate(steps):
             nxt = steps[i + 1] if i + 1 < len(steps) else None
             if st.kind == "mm":
@@ -642,10 +659,10 @@ class Program:
                     need = self._stream_planes() if in_coupling else self._operand_planes()
                     direct_ok = st.engine == ENGINE_SIMT or (x.data_ptr() % 16 == 0 and x.stride(0) % 4 == 0)
                     if not all(getattr(cur, pl) is not None for pl in need) or (cur is src_f32 and not direct_ok):
-                        if cur.f32 is None:
+                        if cur.f32 is None and not (cur is src_f32 and dq is not None):
                             raise RuntimeError("internal: activation has no fp32 plane to re-encode from")
                         b = new_act("x", cur.width, need)
-                        ops.ingest(cur.f32, b, overflow_flag=flag)
+                        ingest(cur, b, overflow_flag=flag)
                         cur = b
                     a = seg_view(cur, st.in_seg)
                 else:
@@ -711,18 +728,18 @@ class Program:
             elif st.kind == "affine":                                  # x_seg <- x_seg * exp(s) + t  (or the inverse), in place
                 if cur is src_f32:                                     # never update the caller's tensor
                     b = new_act("x", cur.width, self._stream_planes())
-                    ops.ingest(cur.f32, b, overflow_flag=flag)
+                    ingest(cur, b, overflow_flag=flag)
                     cur = b
                 target = seg_view(cur, st.out_seg)
                 ops.affine_couple(st_buf, target, st.sign, st.clip[0], st.clip[1], row_ladj=ladj_rows, overflow_flag=flag)
                 if nxt is not None and nxt.kind in ("leaky", "permute", "vec") and cur.f32 is None:
                     raise NotImplementedError("usflows_b200: an elementwise layer directly after an affine coupling is not built")
             else:                                                      # elementwise kernels on the fp32 plane
-                if cur.f32 is None:
+                if cur.f32 is None and not (st.kind == "vec" and cur is src_f32 and dq is not None):
                     raise RuntimeError("internal: elementwise step needs an fp32 stream plane")
                 out = Act(rows, cur.width, f32=final_out) if st.final else new_act("x", cur.width, {"f32"})
                 if st.kind == "vec":
-                    ops.ingest(cur.f32, out, div=st.vec_div, mul=st.vec_mul)
+                    ingest(cur, out, div=st.vec_div, mul=st.vec_mul)
                 elif st.kind == "leaky":
                     ops.leaky_relu(cur.f32, st.slope, out.f32)
                 else:
@@ -838,12 +855,20 @@ class CPlan:
         except Exception:                      # noqa: BLE001  (interpreter shutdown)
             pass
 
-    def log_prob(self, x: torch.Tensor, out: torch.Tensor, flag: Optional[torch.Tensor] = None) -> None:
-        """out[r] = log p(x[r]) for r < rows <= max_rows on the current stream."""
+    def log_prob(self, x: torch.Tensor, out: torch.Tensor, flag: Optional[torch.Tensor] = None,
+                 dq: Optional[ops.Dequant] = None) -> None:
+        """out[r] = log p(x[r]) for r < rows <= max_rows on the current stream; with `dq`, x is uint8 (usf_flow_logprob_u8)."""
         ops.LAUNCHES += len(self.prog.steps) + 2
         from . import _lib
-        _lib.check(self._lib.usf_flow_logprob(self.handle, x.data_ptr(), ops._ld(x), x.shape[0], out.data_ptr(),
-                                              None if flag is None else flag.data_ptr(), ops._stream()))
+        fl = None if flag is None else flag.data_ptr()
+        if dq is not None:
+            import ctypes as C
+            s = dq.struct()
+            _lib.check(self._lib.usf_flow_logprob_u8(self.handle, x.data_ptr(), ops._ld(x), x.shape[0], C.byref(s),
+                                                     out.data_ptr(), fl, ops._stream()))
+            return
+        _lib.check(self._lib.usf_flow_logprob(self.handle, x.data_ptr(), ops._ld(x), x.shape[0], out.data_ptr(), fl,
+                                              ops._stream()))
 
     def apply(self, x: torch.Tensor, z: torch.Tensor, flag: Optional[torch.Tensor] = None) -> None:
         ops.LAUNCHES += len(self.prog.steps) + 1
@@ -894,8 +919,16 @@ _workspace = _Workspace()
 # --------------------------------------------------------------------------------------------------
 # public helpers used by the layer / flow classes
 # --------------------------------------------------------------------------------------------------
-def _flatten_rows(x: torch.Tensor, event_ndim: int = 1):
-    ops.require_cuda(x, "input")
+def _dequantized(x: torch.Tensor, dq: ops.Dequant) -> torch.Tensor:
+    """fp32 copy of the 8-bit rows x [rows, d] (for the routes that read fp32 only)."""
+    out = torch.empty(x.shape, dtype=torch.float32, device=x.device)
+    if x.numel():
+        ops.ingest_u8(x, dq, Act(x.shape[0], x.shape[1], f32=out))
+    return out
+
+
+def _flatten_rows(x: torch.Tensor, event_ndim: int = 1, dtype=torch.float32):
+    ops.require_cuda(x, "input", dtype)
     batch_shape = x.shape[:x.dim() - event_ndim]
     return x.reshape(math.prod(batch_shape), math.prod(x.shape[x.dim() - event_ndim:])), batch_shape
 

@@ -190,16 +190,28 @@ class Flow(torch.nn.Module):
         """data -> latent through every layer's `backward` in reverse order (flows.py:57-67)."""
         return self._run("backward", x)
 
-    def log_prob(self, x: torch.Tensor, context: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """log p(x) = base.log_prob(z) - sum_k log|det J_k|  (flows.py:225-245)."""
+    def log_prob(self, x: torch.Tensor, context: Optional[torch.Tensor] = None, *, dequantize: Optional[str] = None,
+                 seed: Optional[int] = None) -> torch.Tensor:
+        """log p(x) = base.log_prob(z) - sum_k log|det J_k|  (flows.py:225-245).
+
+        With `dequantize` ("uniform" or "midpoint"), x is a uint8 batch [*batch, *event] of 8-bit values that the first kernel
+        reading it dequantises, exactly as `usflows_b200.dequantize(x.reshape(-1, *event), dequantize, seed)` would (the
+        reference's DequantizedDataset for "uniform"); `seed=None` draws a fresh seed from torch.default_generator."""
+        return self._log_prob_any(x, context, ops.dequant_spec(x, dequantize, seed))
+
+    def _log_prob_any(self, x: torch.Tensor, context, dq: Optional[ops.Dequant]) -> torch.Tensor:
         if self.soft_training:
             self._require_conditional()
         elif self._context_needs_soft_training:
             context = None                    # USFlow.log_prob drops the context unless soft_training (flows.py:559-567)
         if context is not None or self._layer_route:
+            if dq is not None:                # the layer-by-layer route reads fp32
+                x2, _ = engine._flatten_rows(x, len(self._event_shape()), torch.uint8)
+                with ops.on_device(x):
+                    x = engine._dequantized(x2.contiguous(), dq).reshape(x.shape)
             return self._with_context("log_prob", x, context)
         with ops.on_device(x):                # no context = context 0 (flows.py:559-565): the conditional conditioners
-            return self._log_prob(x)          # are lowered without their context input, which is exact
+            return self._log_prob(x, dq)      # are lowered without their context input, which is exact
 
     def _require_conditional(self) -> None:
         """Soft training hands a context to every coupling's conditioner (transforms.py:284-289), which only the
@@ -227,33 +239,36 @@ class Flow(torch.nn.Module):
                 return training.log_prob_autograd(self, x2, context).reshape(batch_shape)
             return training.apply_autograd(self, x2, what, context).reshape(*batch_shape, *x2.shape[1:])
 
-    def _log_prob(self, x: torch.Tensor) -> torch.Tensor:
+    def _log_prob(self, x: torch.Tensor, dq: Optional[ops.Dequant] = None) -> torch.Tensor:
+        """`dq`: x is uint8 (ops.Dequant); every route below reaches the same result as on the dequantised fp32 rows."""
         prog, ladj = self._program("backward", self._zero_ctx)
         base = self._base_module()
         base._prepared()                  # parameter-side work happens here, outside any graph capture
-        x2, batch_shape = engine._flatten_rows(x, len(self._event_shape()))
+        x2, batch_shape = engine._flatten_rows(x, len(self._event_shape()), torch.float32 if dq is None else torch.uint8)
+        if dq is not None:
+            x2 = x2.contiguous()
         d = x2.shape[1]
         rows = x2.shape[0]
         if isinstance(prog, image_engine.ImageProgram):      # image-shaped event: the latent arrives channels-last
             if x2.is_cuda and 0 < rows <= SMALL_BATCH_GRAPH_IMAGES and not prog.force_fallback \
                     and not torch.cuda.is_current_stream_capturing():
-                lp = self._log_prob_small_batch(prog, ladj, x2)     # ~100 launches per step: one graph replay instead
-                if lp is not None:
+                lp = self._log_prob_small_batch(prog, ladj, x2 if dq is None else engine._dequantized(x2, dq))
+                if lp is not None:                                  # ~100 launches per step: one graph replay instead
                     return lp.reshape(batch_shape)
             out = torch.empty(rows, dtype=torch.float32, device=x2.device)
             perm = self._channels_last_perm(x2.device)
             with torch.no_grad():
                 prog.run(x2, sink=lambda z, r0, r1: base._density_into(ops.Act(r1 - r0, d, f32=z), -ladj, out[r0:r1],
-                                                                       perm=perm))
+                                                                       perm=perm), dq=dq)
             return out.reshape(batch_shape)
         if x2.is_cuda and 0 < rows <= SMALL_BATCH_GRAPH_ROWS and getattr(prog, "small", None) is None \
                 and not prog.force_fallback and not prog.has_row_ladj and not torch.cuda.is_current_stream_capturing():
-            lp = self._log_prob_small_batch(prog, ladj, x2)
+            lp = self._log_prob_small_batch(prog, ladj, x2 if dq is None else engine._dequantized(x2, dq))
             if lp is not None:
                 return lp.reshape(batch_shape)
         if USE_C_PLAN and x2.is_cuda and rows > 0 and prog.plan_able() and getattr(base, "base_kind", -1) >= 0 \
                 and not torch.cuda.is_current_stream_capturing():
-            return self._log_prob_plan(prog, base, ladj, x2).reshape(batch_shape)
+            return self._log_prob_plan(prog, base, ladj, x2, dq).reshape(batch_shape)
         out = torch.empty(rows, dtype=torch.float32, device=x2.device)
 
         def sink(z_chunk, r0, r1):
@@ -262,11 +277,11 @@ class Flow(torch.nn.Module):
         with torch.no_grad():
             if prog.has_row_ladj:          # affine couplings: per-row log-determinants next to the model constant
                 row_ladj = torch.zeros(rows, dtype=torch.float32, device=x2.device)
-                prog.run(x2, sink=sink, ladj_rows=row_ladj)
+                prog.run(x2, sink=sink, ladj_rows=row_ladj, dq=dq)
                 if rows:
                     ops.sub_rows(out, row_ladj)
             else:
-                prog.run(x2, sink=sink)
+                prog.run(x2, sink=sink, dq=dq)
         return out.reshape(batch_shape)
 
     @staticmethod
@@ -281,7 +296,7 @@ class Flow(torch.nn.Module):
             size *= 2
         return chunk, min(size, max(cap, chunk))
 
-    def _log_prob_plan(self, prog, base, ladj: float, x2: torch.Tensor) -> torch.Tensor:
+    def _log_prob_plan(self, prog, base, ladj: float, x2: torch.Tensor, dq: Optional[ops.Dequant] = None) -> torch.Tensor:
         """`log_prob` through the whole-stack C entry: one `usf_flow_logprob` call per chunk (ingest, every contraction and
         the base density are launched by the library).  Same kernels, same order, same bits as the launch-by-launch route."""
         rows, d = x2.shape
@@ -294,13 +309,14 @@ class Flow(torch.nn.Module):
             flags = torch.zeros(len(starts), dtype=torch.int32, device=x2.device) if prog.mode == "fp32" else None
             for ci, r0 in enumerate(starts):
                 r1 = min(rows, r0 + chunk)
-                plan.log_prob(x2[r0:r1], out[r0:r1], None if flags is None else flags[ci:ci + 1])
+                plan.log_prob(x2[r0:r1], out[r0:r1], None if flags is None else flags[ci:ci + 1],
+                              None if dq is None else dq.shifted(r0))
             if flags is not None:                       # chunks that left the fp16 range: tf32-split engine, launch by launch
                 for ci in torch.nonzero(flags).reshape(-1).tolist():
                     r0 = starts[ci]
                     r1 = min(rows, r0 + chunk)
                     prog._fallback().run(x2[r0:r1], sink=lambda z, a, b, r0=r0: base._density_into(
-                        ops.Act(b - a, z.shape[1], f32=z), -ladj, out[r0 + a:r0 + b]))
+                        ops.Act(b - a, z.shape[1], f32=z), -ladj, out[r0 + a:r0 + b]), dq=None if dq is None else dq.shifted(r0))
         return out
 
     def _log_prob_small_batch(self, prog, ladj: float, x2: torch.Tensor):
@@ -354,10 +370,11 @@ class Flow(torch.nn.Module):
                 return None
             return ent["out"].clone()
 
-    def _chunk_graph(self, prog, slot: int, buf: torch.Tensor, d: int) -> dict:
-        """CUDA graph of the launch program of one full-size chunk reading host-staging buffer `slot`."""
+    def _chunk_graph(self, prog, slot: int, buf: torch.Tensor, d: int, dq_mode: Optional[str] = None) -> dict:
+        """CUDA graph of the launch program of one full-size chunk reading host-staging buffer `slot`.  With `dq_mode`, the
+        buffer holds 8-bit rows; the graph reads their {seed, global row} from its `params` tensor, written before a replay."""
         cache = prog.__dict__.setdefault("_host_graphs", {})     # on the Program: see _log_prob_small_batch
-        key = (slot, buf.data_ptr(), tuple(buf.shape))
+        key = (slot, buf.data_ptr(), tuple(buf.shape), dq_mode)
         ent = cache.get(key)
         if ent is not None and ent["gen"] == engine._workspace.generation:
             return ent
@@ -365,13 +382,15 @@ class Flow(torch.nn.Module):
         rows, width = buf.shape[0], prog.out_width(d)
         flag = torch.zeros(1, dtype=torch.int32, device=dev) if prog.mode == "fp32" else None
         fin = engine._workspace.planes(dev, f"final_host{slot}", rows, width, "f32")
-        prog._run_chunk(buf, fin, flag)                   # eager pass: sizes every workspace buffer before capture
+        params = None if dq_mode is None else torch.zeros(2, dtype=torch.int64, device=dev)
+        dq = None if dq_mode is None else ops.Dequant(dq_mode, 0, 0, params)
+        prog._run_chunk(buf, fin, flag, None, dq)         # eager pass: sizes every workspace buffer before capture
         torch.cuda.synchronize(dev)
         graph = torch.cuda.CUDAGraph()
         with _plain_stream_order(), torch.cuda.graph(graph, stream=capture_stream(dev), capture_error_mode="thread_local"):
-            prog._run_chunk(buf, fin, flag)
-        ent = dict(graph=graph, fin=fin, flag=flag, gen=engine._workspace.generation)
-        for k in [k for k in cache if k[0] == slot and (k[1] != key[1] or cache[k]["gen"] != ent["gen"])]:
+            prog._run_chunk(buf, fin, flag, None, dq)
+        ent = dict(graph=graph, fin=fin, flag=flag, params=params, gen=engine._workspace.generation)
+        for k in [k for k in cache if k[0] == slot and ((k[1] != key[1] and k[3] == dq_mode) or cache[k]["gen"] != ent["gen"])]:
             del cache[k]                                  # graphs of a replaced staging buffer / of stale workspaces
         while sum(1 for k in cache if k[0] == slot) >= 6:  # a few chunk sizes per staging buffer; drop the oldest
             del cache[next(k for k in cache if k[0] == slot)]
@@ -379,22 +398,29 @@ class Flow(torch.nn.Module):
         return ent
 
     def log_prob_host(self, x_host: torch.Tensor, out_host: Optional[torch.Tensor] = None,
-                      chunk_rows: Optional[int] = None) -> torch.Tensor:
+                      chunk_rows: Optional[int] = None, *, dequantize: Optional[str] = None, seed: Optional[int] = None,
+                      row_offset: int = 0) -> torch.Tensor:
         """`log_prob` for rows living in HOST memory (pinned for full copy speed): the batch is streamed
         through the device in chunks -- H2D copy of chunk i+1 on a side stream overlaps the kernels of
-        chunk i -- and the log-probs are copied back into `out_host`.  Returns `out_host`."""
+        chunk i -- and the log-probs are copied back into `out_host`.  Returns `out_host`.
+
+        With `dequantize` (see `log_prob`), x_host is a uint8 batch: a quarter of the bytes cross to the device, and the
+        ingest kernels dequantise.  Row r of x_host is global row `row_offset + r` of the noise (a caller that splits one
+        batch over several calls passes each part's offset and one seed to get the noise of a single call)."""
         if x_host.is_cuda:
             raise RuntimeError("log_prob_host expects a host tensor; use log_prob for device tensors")
+        dq = ops.dequant_spec(x_host, dequantize, seed, row_offset)
         with ops.on_device(next(self.parameters())):
-            return self._log_prob_host(x_host, out_host, chunk_rows)
+            return self._log_prob_host(x_host, out_host, chunk_rows, dq)
 
-    def _log_prob_host(self, x_host, out_host, chunk_rows):
+    def _log_prob_host(self, x_host, out_host, chunk_rows, dq: Optional[ops.Dequant] = None):
         dev = next(self.parameters()).device
         if self._layer_route:                 # no launch program to overlap the copies with: plain chunks
             out = torch.empty(x_host.shape[0], dtype=torch.float32) if out_host is None else out_host
             step = max(1, chunk_rows or 8192)
             for r0 in range(0, x_host.shape[0], step):
-                out[r0:r0 + step].copy_(self.log_prob(x_host[r0:r0 + step].to(dev)))
+                out[r0:r0 + step].copy_(self._log_prob_any(x_host[r0:r0 + step].to(dev), None,
+                                                           None if dq is None else dq.shifted(r0)))
             return out
         prog, ladj = self._program("backward", self._zero_ctx)
         base = self._base_module()
@@ -408,9 +434,11 @@ class Flow(torch.nn.Module):
             # kernels of chunk i, one D2H copy of all log-probs at the end
             step = max(1, chunk_rows or HOST_CHUNK_ROWS)
             main = torch.cuda.current_stream(dev)
-            if getattr(self, "_img_stage", None) is None or self._img_stage.shape[1:] != (min(step, max(rows, 1)), d) \
-                    or self._img_stage.device != dev:
-                self._img_stage = torch.empty(2, min(step, max(rows, 1)), d, dtype=torch.float32, device=dev)
+            attr = "_img_stage" if dq is None else "_img_stage_u8"      # 8-bit rows are staged as they are
+            stage = getattr(self, attr, None)
+            if stage is None or stage.shape[1:] != (min(step, max(rows, 1)), d) or stage.device != dev:
+                stage = torch.empty(2, min(step, max(rows, 1)), d, dtype=torch.float32 if dq is None else torch.uint8, device=dev)
+                setattr(self, attr, stage)
                 self._copy_stream = torch.cuda.Stream(device=dev)
             out_dev = torch.empty(rows, dtype=torch.float32, device=dev)
             starts = list(range(0, rows, step))
@@ -424,7 +452,7 @@ class Flow(torch.nn.Module):
                 with torch.cuda.stream(self._copy_stream):
                     if i >= 2:
                         self._copy_stream.wait_event(consumed[i % 2])
-                    self._img_stage[i % 2, :n].copy_(x2[r0:r0 + n], non_blocking=True)
+                    stage[i % 2, :n].copy_(x2[r0:r0 + n], non_blocking=True)
                     copied[i % 2].record(self._copy_stream)
 
             if starts:
@@ -434,7 +462,8 @@ class Flow(torch.nn.Module):
                 if i + 1 < len(starts):
                     issue_copy(i + 1)
                 main.wait_event(copied[i % 2])
-                out_dev[r0:r0 + n] = self._log_prob(self._img_stage[i % 2, :n].reshape(n, *self._event_shape()))
+                out_dev[r0:r0 + n] = self._log_prob(stage[i % 2, :n].reshape(n, *self._event_shape()),
+                                                    None if dq is None else dq.shifted(r0))
                 consumed[i % 2].record(main)
             out_host.reshape(-1)[:rows].copy_(out_dev, non_blocking=True)
             main.synchronize()
@@ -455,18 +484,22 @@ class Flow(torch.nn.Module):
         starts = [sum(sizes[:i]) for i in range(len(sizes))]
         # staging: one device buffer per chunk (slices of one allocation holding the whole batch) when that fits -- the
         # copies then run back to back on the copy stream, independent of the kernels --, else two buffers used in turn
-        whole = rows * d * 4 <= HOST_STAGE_BYTES and len(sizes) <= HOST_MAX_STAGE_SLICES
+        # 8-bit rows are staged as they are (a quarter of the bytes), in a buffer of their own: fp32 and uint8 calls in turn
+        # keep their staging buffers and captured graphs
+        sdt, attr = (torch.float32, "_host_stage") if dq is None else (torch.uint8, "_host_stage_u8")
+        whole = rows * d * sdt.itemsize <= HOST_STAGE_BYTES and len(sizes) <= HOST_MAX_STAGE_SLICES
         need = max(rows, 1) if whole else 2 * chunk
-        if getattr(self, "_host_stage", None) is None or self._host_stage.shape[0] < need \
-                or self._host_stage.shape[1] != d or self._host_stage.device != dev:
-            self._host_stage = torch.empty(need, d, dtype=torch.float32, device=dev)
+        stage = getattr(self, attr, None)
+        if stage is None or stage.shape[0] < need or stage.shape[1] != d or stage.device != dev:
+            stage = torch.empty(need, d, dtype=sdt, device=dev)
+            setattr(self, attr, stage)
             self._host_out = torch.empty(0, dtype=torch.float32, device=dev)
             self._copy_stream = torch.cuda.Stream(device=dev)
         n_buf = max(1, len(sizes)) if whole else 2
         if whole:
-            bufs = [self._host_stage[starts[i]:starts[i] + sizes[i]] for i in range(len(sizes))] or [self._host_stage[:0]]
+            bufs = [stage[starts[i]:starts[i] + sizes[i]] for i in range(len(sizes))] or [stage[:0]]
         else:
-            bufs = [self._host_stage[:chunk], self._host_stage[chunk:2 * chunk]]
+            bufs = [stage[:chunk], stage[chunk:2 * chunk]]
         if self._host_out.numel() < rows:
             self._host_out = torch.empty(rows, dtype=torch.float32, device=dev)
         out_dev = self._host_out[:rows]
@@ -491,12 +524,15 @@ class Flow(torch.nn.Module):
                 for _ in range(2):                        # a workspace that grew while capturing invalidates earlier graphs
                     for i in sorted(range(len(sizes)), key=lambda j: -sizes[j]):
                         if sizes[i] >= unit // 2:
-                            graphs[(i % n_buf, sizes[i])] = self._chunk_graph(prog, i % n_buf, bufs[i % n_buf][:sizes[i]], d)
+                            graphs[(i % n_buf, sizes[i])] = self._chunk_graph(prog, i % n_buf, bufs[i % n_buf][:sizes[i]], d,
+                                                                              None if dq is None else dq.mode)
                     if all(g["gen"] == engine._workspace.generation for g in graphs.values()):
                         break
                 for g in graphs.values():
                     if g["flag"] is not None:
                         g["flag"].zero_()
+            if graphs and dq is not None:                 # {seed, global row} of every chunk, read by the graphs' ingest
+                params = torch.tensor([[dq.seed, dq.row0 + r0] for r0 in starts], dtype=torch.int64).to(dev)
             self._copy_stream.wait_stream(main)
             for i, r0 in enumerate(starts):
                 r1 = r0 + sizes[i]
@@ -512,12 +548,14 @@ class Flow(torch.nn.Module):
                 if g is not None:
                     # one graph launch replaces the ~23 kernel launches of the chunk: the host-side launch cost
                     # (~40 us per launch through ctypes + tensor-map encoding) is what bounds small chunks otherwise
+                    if g["params"] is not None:
+                        g["params"].copy_(params[i])
                     g["graph"].replay()
                     make_sink(r0)(g["fin"], 0, sizes[i])
                 else:
                     prog.run(buf, chunk_rows=chunk, sink=make_sink(r0),
                              flag_out=flags[i:i + 1] if guarded else None,
-                             ladj_rows=None if row_ladj is None else row_ladj[r0:r1])
+                             ladj_rows=None if row_ladj is None else row_ladj[r0:r1], dq=None if dq is None else dq.shifted(r0))
                 consumed[slot].record(main)
             if guarded:                                   # one sync; out-of-range chunks go through the tf32 split
                 redo = set(torch.nonzero(flags).reshape(-1).tolist())
@@ -531,7 +569,8 @@ class Flow(torch.nn.Module):
                     if row_ladj is not None:
                         row_ladj[r0:r1].zero_()
                     prog._fallback().run(buf, chunk_rows=chunk, sink=make_sink(r0),
-                                         ladj_rows=None if row_ladj is None else row_ladj[r0:r1])
+                                         ladj_rows=None if row_ladj is None else row_ladj[r0:r1],
+                                         dq=None if dq is None else dq.shifted(r0))
             if row_ladj is not None and rows:
                 ops.sub_rows(out_dev, row_ladj)
             out_host.reshape(-1)[:rows].copy_(out_dev, non_blocking=True)

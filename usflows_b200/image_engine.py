@@ -311,16 +311,20 @@ class ImageProgram:
         return d_in
 
     # ----------------------------------------------------------------------------------------------
-    def _run_chunk(self, x: torch.Tensor, out: torch.Tensor, nchw_out: bool, flag) -> None:
-        """x [n, C*H*W] (NCHW, read-only) -> out [n, C*H*W]: NCHW when `nchw_out`, else channels-last ([n, H*W*C])."""
+    def _run_chunk(self, x: torch.Tensor, out: torch.Tensor, nchw_out: bool, flag, dq: Optional[ops.Dequant] = None) -> None:
+        """x [n, C*H*W] (NCHW, read-only) -> out [n, C*H*W]: NCHW when `nchw_out`, else channels-last ([n, H*W*C]).  With
+        `dq`, x is uint8 and the NCHW -> channels-last conversion dequantises it."""
         dev, n = x.device, x.shape[0]
         rows, C, HW = n * self.HW, self.C, self.HW
         direct = not nchw_out and self.exit_scale is None    # the channels-last stream itself is the result
         bufs = [_dense(dev, "img_x0", rows, C), _dense(dev, "img_x1", rows, C)]
         which, cur = 0, bufs[0]
         es = self.entry_scale
-        ops.layout_transpose(x, n, C, HW, cur, scale=None if es is None else es[0], scale_mode=0 if es is None else es[1],
-                             scale_on_input=True)
+        if dq is not None:
+            ops.layout_transpose_u8(x, dq, n, C, HW, cur, scale=None if es is None else es[0], scale_mode=0 if es is None else es[1])
+        else:
+            ops.layout_transpose(x, n, C, HW, cur, scale=None if es is None else es[0], scale_mode=0 if es is None else es[1],
+                                 scale_on_input=True)
         for idx, op in enumerate(self.ops):
             if op[0] == "aff":
                 g = op[1]
@@ -355,9 +359,11 @@ class ImageProgram:
             ops.layout_transpose(cur, n, HW, C, tmp, scale=xs[0], scale_mode=xs[1], scale_on_input=False)
             ops.layout_transpose(tmp, n, C, HW, out)
 
-    def run(self, x: torch.Tensor, nchw_out: bool = True, sink=None, chunk_rows: Optional[int] = None) -> Optional[torch.Tensor]:
-        """x [N, C*H*W] -> [N, C*H*W] (NCHW order), or per chunk `sink(channels_last_chunk [n, H*W*C], r0, r1)`."""
-        ops.require_cuda(x, "input")
+    def run(self, x: torch.Tensor, nchw_out: bool = True, sink=None, chunk_rows: Optional[int] = None,
+            dq: Optional[ops.Dequant] = None) -> Optional[torch.Tensor]:
+        """x [N, C*H*W] -> [N, C*H*W] (NCHW order), or per chunk `sink(channels_last_chunk [n, H*W*C], r0, r1)`; with `dq`, x
+        is uint8 (see _run_chunk)."""
+        ops.require_cuda(x, "input", torch.float32 if dq is None else torch.uint8)
         x = x.contiguous()
         N, d = x.shape
         if d != self.C * self.HW:
@@ -366,7 +372,7 @@ class ImageProgram:
         if N == 0:
             return out
         if self.force_fallback:
-            return self._fallback().run(x, nchw_out, sink, chunk_rows)
+            return self._fallback().run(x, nchw_out, sink, chunk_rows, dq)
         all_pix = all(op[0] != "coupling" or op[1].pix is not None for op in self.ops)
         per = max(1, (chunk_rows or (IMAGE_CHUNK_ROWS_PIX if all_pix else IMAGE_CHUNK_ROWS)) // self.HW)
         starts = list(range(0, N, per))
@@ -374,12 +380,13 @@ class ImageProgram:
 
         def one(prog, i, r0, flag):
             r1 = min(N, r0 + per)
+            cdq = None if dq is None else dq.shifted(r0)
             if sink is not None:
                 fin = _dense(x.device, "img_final", r1 - r0, d)
-                prog._run_chunk(x[r0:r1], fin, False, flag)
+                prog._run_chunk(x[r0:r1], fin, False, flag, cdq)
                 sink(fin, r0, r1)
             else:
-                prog._run_chunk(x[r0:r1], out[r0:r1], nchw_out, flag)
+                prog._run_chunk(x[r0:r1], out[r0:r1], nchw_out, flag, cdq)
 
         for i, r0 in enumerate(starts):
             one(self, i, r0, None if flags is None else flags[i:i + 1])

@@ -6,6 +6,7 @@ path in this package (the CPU oracle lives in oracle/ and is test infrastructure
 from __future__ import annotations
 
 import ctypes as C
+import math
 from dataclasses import dataclass
 from typing import Optional
 
@@ -146,6 +147,76 @@ def ingest(x: torch.Tensor, out: Act, *, div=None, mul=None, sub=None,
         _ptr(out.bf16), _ld(out.bf16) if out.bf16 is not None else 0, _stream()))
 
 
+# ---- 8-bit inputs ---------------------------------------------------------------------------------------------------------
+DEQUANT_MODES = {"uniform": _lib.DEQUANT_UNIFORM, "midpoint": _lib.DEQUANT_MIDPOINT}
+
+
+@dataclass(frozen=True)
+class Dequant:
+    """How 8-bit rows become fp32 (usf_dequant): `mode` ("uniform" / "midpoint"), the Philox key `seed`, the global row of
+    local row 0 `row0`, and optionally `params`, a device int64 [2] tensor {seed, row base} read at run time (seed replaced,
+    row base added to row0) so that one captured graph serves every call."""
+
+    mode: str
+    seed: int
+    row0: int = 0
+    params: Optional[torch.Tensor] = None
+
+    def shifted(self, rows: int) -> "Dequant":
+        return Dequant(self.mode, self.seed, self.row0 + int(rows), self.params)
+
+    def struct(self):
+        s = _lib.Dequant()
+        s.mode, s.seed, s.row0 = DEQUANT_MODES[self.mode], self.seed & (2**64 - 1), self.row0
+        s.dev_params = _ptr(self.params)
+        return s
+
+
+def draw_seed() -> int:
+    """One 63-bit dequantisation seed from torch.default_generator (`torch.manual_seed` reproduces it)."""
+    return int(torch.empty((), dtype=torch.int64).random_(0, 2**63 - 1, generator=torch.default_generator))
+
+
+def dequant_spec(x, mode, seed=None, row0: int = 0) -> Optional[Dequant]:
+    """Validates a `dequantize=` argument against the input; None when `mode` is None (fp32 input)."""
+    if mode is None:
+        return None
+    if mode not in DEQUANT_MODES:
+        raise ValueError(f"usflows_b200: unknown dequantize mode {mode!r}; choose from {tuple(DEQUANT_MODES)}")
+    if not isinstance(x, torch.Tensor) or x.dtype != torch.uint8:
+        raise ValueError(f"usflows_b200: dequantize={mode!r} takes a uint8 input, got "
+                         f"{x.dtype if isinstance(x, torch.Tensor) else type(x).__name__}")
+    return Dequant(mode, draw_seed() if seed is None else int(seed), int(row0))
+
+
+def ingest_u8(x: torch.Tensor, dq: Dequant, out: Act, *, div=None, mul=None, sub=None,
+              overflow_flag: Optional[torch.Tensor] = None) -> None:
+    """`ingest` reading 8-bit rows x [rows, d] (uint8), dequantised as `dq` says; see usf_ingest_u8."""
+    global LAUNCHES
+    LAUNCHES += 1
+    rows, d = x.shape
+    p, s = _planes_struct(out), dq.struct()
+    check(_lib.load().usf_ingest_u8(_ptr(x), _ld(x), rows, d, C.byref(s), _ptr(div), _ptr(mul), _ptr(sub), C.byref(p),
+                                    _ptr(overflow_flag), _stream()))
+
+
+def dequantize(x_u8: torch.Tensor, mode: str = "uniform", seed: Optional[int] = None, row_offset: int = 0) -> torch.Tensor:
+    """fp32 values of the 8-bit CUDA tensor `x_u8` [rows, *event] (a 1-D tensor is one row): element j (flat index within
+    the row) of row r becomes (k + u) / 256 with Philox noise u keyed by (seed, row_offset + r, j) ("uniform", the
+    reference's DequantizedDataset), or (k + 0.5) / 256 ("midpoint").  `seed=None` draws one from torch.default_generator.
+    The values are exactly those `Flow.log_prob(x_u8, dequantize=mode, seed=seed)` evaluates."""
+    dq = dequant_spec(x_u8, mode, seed, row_offset)
+    require_cuda(x_u8, "x_u8", torch.uint8)
+    x2 = x_u8.reshape(1, -1) if x_u8.dim() <= 1 else x_u8.reshape(x_u8.shape[0], math.prod(x_u8.shape[1:]))
+    if x2.shape[1] > 0 and x2.stride(1) != 1:
+        x2 = x2.contiguous()
+    out = torch.empty(x2.shape, dtype=torch.float32, device=x_u8.device)
+    if out.numel():
+        with on_device(x_u8):
+            ingest_u8(x2, dq, Act(x2.shape[0], x2.shape[1], f32=out))
+    return out.reshape(x_u8.shape)
+
+
 def base_logprob(z: Act, loc, scale, kind: int, add_const: float, out: torch.Tensor) -> None:
     global LAUNCHES
     LAUNCHES += 1
@@ -240,6 +311,16 @@ def layout_transpose(x: torch.Tensor, n: int, a: int, b: int, out: torch.Tensor,
     LAUNCHES += 1
     check(_lib.load().usf_layout_transpose(_ptr(x), n, a, b, _ptr(scale), scale_mode if scale is not None else 0,
                                            int(scale_on_input), _ptr(out), _stream()))
+
+
+def layout_transpose_u8(x: torch.Tensor, dq: Dequant, n: int, c: int, hw: int, out: torch.Tensor, scale=None,
+                        scale_mode: int = 0) -> None:
+    """8-bit NCHW images x [n, c*hw] -> dequantised channels-last fp32 out (x| /) scale; see usf_layout_transpose_u8."""
+    global LAUNCHES
+    LAUNCHES += 1
+    s = dq.struct()
+    check(_lib.load().usf_layout_transpose_u8(_ptr(x), n, c, hw, C.byref(s), _ptr(scale), scale_mode if scale is not None else 0,
+                                              _ptr(out), _stream()))
 
 
 def im2col(x: torch.Tensor, n_images: int, h: int, w: int, c: int, k: int, dilation: int, out: Act, *, mask=None,

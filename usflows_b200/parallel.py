@@ -24,9 +24,10 @@ from typing import List, Optional, Sequence
 
 import torch
 
-from . import engine
+from . import engine, ops
 
-_UNCOPIED = ("_programs", "_host_stage", "_host_out", "_img_stage", "_copy_stream", "_cl_perm", "_cl_perm_key", "_sharded")
+_UNCOPIED = ("_programs", "_host_stage", "_host_stage_u8", "_host_out", "_img_stage", "_img_stage_u8", "_copy_stream", "_cl_perm",
+             "_cl_perm_key", "_sharded")
 
 
 def shard_bounds(n: int, rank: int, world: int):
@@ -90,10 +91,15 @@ class ShardedFlow:
         futs = [self._pool.submit(fn, i, rep, lo, hi) for i, (rep, (lo, hi)) in enumerate(zip(self.replicas, bounds))]
         return [f.result() for f in futs]            # re-raises a worker's exception here
 
-    def log_prob(self, x_host: torch.Tensor, out_host: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """log p of the rows of `x_host` [rows, *event] (host memory) -> `out_host` [rows] (host memory)."""
+    def log_prob(self, x_host: torch.Tensor, out_host: Optional[torch.Tensor] = None, *, dequantize: Optional[str] = None,
+                 seed: Optional[int] = None) -> torch.Tensor:
+        """log p of the rows of `x_host` [rows, *event] (host memory) -> `out_host` [rows] (host memory).  With `dequantize`
+        (see Flow.log_prob), x_host is uint8; one seed serves all devices and every block keeps its global row numbers, so
+        the result does not depend on the number of devices."""
         if x_host.is_cuda:
             raise RuntimeError("usflows_b200.parallel: expects host rows (each device copies its own block)")
+        if dequantize is not None:
+            seed = ops.dequant_spec(x_host, dequantize, seed).seed
         self.sync_weights()
         ev = math.prod(self.flow._event_shape())
         x2 = x_host.reshape(-1, ev)
@@ -104,7 +110,10 @@ class ShardedFlow:
 
         def work(i, rep, lo, hi):
             if hi > lo:
-                rep.log_prob_host(x2[lo:hi], flat[lo:hi])
+                if dequantize is None:
+                    rep.log_prob_host(x2[lo:hi], flat[lo:hi])
+                else:
+                    rep.log_prob_host(x2[lo:hi], flat[lo:hi], dequantize=dequantize, seed=seed, row_offset=lo)
         self._map(work, rows)
         return out_host
 
@@ -163,9 +172,11 @@ def _sharded(flow, devices) -> ShardedFlow:
 
 
 def log_prob_sharded(flow, x_host: torch.Tensor, devices: Optional[Sequence] = None,
-                     out_host: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """`flow.log_prob` of host rows on `devices` (default: all visible GPUs), rows split into contiguous blocks."""
-    return _sharded(flow, devices).log_prob(x_host, out_host)
+                     out_host: Optional[torch.Tensor] = None, *, dequantize: Optional[str] = None,
+                     seed: Optional[int] = None) -> torch.Tensor:
+    """`flow.log_prob` of host rows on `devices` (default: all visible GPUs), rows split into contiguous blocks; uint8 rows
+    with `dequantize` as in ShardedFlow.log_prob."""
+    return _sharded(flow, devices).log_prob(x_host, out_host, dequantize=dequantize, seed=seed)
 
 
 def sample_sharded(flow, n: int, devices: Optional[Sequence] = None, out_host: Optional[torch.Tensor] = None) -> torch.Tensor:
