@@ -24,7 +24,7 @@ from __future__ import annotations
 
 import math
 from dataclasses import dataclass, field
-from typing import List, Optional
+from typing import List, Optional, Tuple
 
 import torch
 
@@ -57,6 +57,39 @@ def get_precision() -> str:
 def set_chunk_rows(rows: int) -> None:
     global _default_chunk_rows
     _default_chunk_rows = int(rows)
+
+
+def chunk_bounds(rows: int, cap: int) -> List[Tuple[int, int]]:
+    """(r0, r1) of each chunk of a `rows`-row batch: ceil(rows / cap) near-equal chunks, each rounded up to whole 256-row
+    tiles (the last chunk takes the rest)."""
+    if rows <= 0:
+        return []
+    n_chunks = (rows + cap - 1) // cap
+    chunk = min(rows, ((rows + n_chunks - 1) // n_chunks + 255) // 256 * 256)
+    return [(r0, min(rows, r0 + chunk)) for r0 in range(0, rows, chunk)]
+
+
+def run_chunks(bounds, device, guarded: bool, first, again, shared_flags=(), ladj_rows=None) -> None:
+    """first(i, r0, r1, flag) for every chunk (r0, r1) of `bounds`, in order.  `guarded`: the program runs on fp16 split
+    planes, so every chunk gets its own int32 range flag (else `flag` is None); after ONE device->host read, again(i, r0, r1)
+    recomputes each chunk whose flag is set, in order, with the tf32-split program (same accuracy class, no range limit).
+    Every chunk is recomputed when one of `shared_flags` (the flag of a captured graph replayed for several chunks) is set.
+    `ladj_rows[r0:r1]` (per-row log-determinants the abandoned pass has already added to) is zeroed before again(i, r0, r1)."""
+    if not guarded:
+        for i, (r0, r1) in enumerate(bounds):
+            first(i, r0, r1, None)
+        return
+    flags = torch.zeros(len(bounds), dtype=torch.int32, device=device)
+    for i, (r0, r1) in enumerate(bounds):
+        first(i, r0, r1, flags[i:i + 1])
+    redo = torch.nonzero(torch.cat([flags, *shared_flags]) if shared_flags else flags).reshape(-1).tolist()
+    if redo and redo[-1] >= len(bounds):
+        redo = range(len(bounds))
+    for i in redo:
+        r0, r1 = bounds[i]
+        if ladj_rows is not None:
+            ladj_rows[r0:r1].zero_()
+        again(i, r0, r1)
 
 
 # --------------------------------------------------------------------------------------------------
@@ -319,6 +352,7 @@ class Program:
         self.steps = self._emit(items, compress)
         if self._wflag is not None and int(self._wflag.item()) != 0:
             self.force_fallback = True                          # a weight does not fit fp16: always run 3xTF32
+        self.uses_range_flag = self.mode == "fp32"              # fp16 split planes: chunks carry a range flag
 
     # -- tiny event sizes: pack every layer into one weight blob + op list for the whole-flow kernel
     @staticmethod
@@ -538,10 +572,8 @@ class Program:
     def n_launches(self) -> int:
         return len(self.steps)
 
-    def run(self, x: torch.Tensor, mode: Optional[str] = None, chunk_rows: Optional[int] = None,
-            out: Optional[torch.Tensor] = None, sink=None,
-            flag_out: Optional[torch.Tensor] = None, ladj_rows: Optional[torch.Tensor] = None,
-            dq: Optional[ops.Dequant] = None) -> Optional[torch.Tensor]:
+    def run(self, x: torch.Tensor, *, out: Optional[torch.Tensor] = None, sink=None, chunk_rows: Optional[int] = None,
+            ladj_rows: Optional[torch.Tensor] = None, dq: Optional[ops.Dequant] = None) -> Optional[torch.Tensor]:
         """Evaluate the program on x [rows, d].  With `sink`, the final stream value of each chunk is handed
         to `sink(chunk_f32 [r, width], r0, r1)` from a reused workspace buffer instead of being stored.  With `dq`, x is
         uint8 and its first ingest dequantises it (ops.Dequant)."""
@@ -564,44 +596,25 @@ class Program:
                 return None
             return res
         if self.force_fallback:
-            return self._fallback().run(x, chunk_rows=chunk_rows, out=out, sink=sink, ladj_rows=ladj_rows, dq=dq)
-        cap = chunk_rows or _default_chunk_rows
-        n_chunks = (rows + cap - 1) // cap
-        chunk = min(rows, ((rows + n_chunks - 1) // n_chunks + 255) // 256 * 256)
-        starts = list(range(0, rows, chunk))
-        own_flags = self.mode == "fp32" and flag_out is None
-        flags = torch.zeros(len(starts), dtype=torch.int32, device=x.device) if own_flags else None
+            return self._fallback().run(x, out=out, sink=sink, chunk_rows=chunk_rows, ladj_rows=ladj_rows, dq=dq)
         if sink is None and out is None:
             out = torch.empty(rows, width, dtype=torch.float32, device=x.device)
-        for ci, r0 in enumerate(starts):
-            r1 = min(rows, r0 + chunk)
-            flag = flags[ci:ci + 1] if own_flags else flag_out
-            lr = None if ladj_rows is None else ladj_rows[r0:r1]
-            cdq = None if dq is None else dq.shifted(r0)
+
+        def chunk(prog, r0, r1, flag):
+            fin = out[r0:r1] if sink is None else self.final_buffer(x.device, "final", r1 - r0, x.shape[1])
+            prog._run_chunk(x[r0:r1], fin, flag, None if dq is None else dq.shifted(r0),
+                            ladj_rows=None if ladj_rows is None else ladj_rows[r0:r1])
             if sink is not None:
-                fin = _workspace.planes(x.device, "final", r1 - r0, width, "f32")
-                self._run_chunk(x[r0:r1], fin, flag, lr, cdq)
                 sink(fin, r0, r1)
-            else:
-                self._run_chunk(x[r0:r1], out[r0:r1], flag, lr, cdq)
-        if own_flags:
-            # one device->host read per call: chunks whose activations left the fp16 range are recomputed with the
-            # tf32-split engine (same accuracy class, no range limit)
-            for ci in torch.nonzero(flags).reshape(-1).tolist():
-                r0 = starts[ci]
-                r1 = min(rows, r0 + chunk)
-                fb = self._fallback()
-                lr = None if ladj_rows is None else ladj_rows[r0:r1]
-                if lr is not None:
-                    lr.zero_()                                  # the abandoned pass already added its log-scales
-                cdq = None if dq is None else dq.shifted(r0)
-                if sink is not None:
-                    fin = _workspace.planes(x.device, "final", r1 - r0, width, "f32")
-                    fb._run_chunk(x[r0:r1], fin, None, lr, cdq)
-                    sink(fin, r0, r1)
-                else:
-                    fb._run_chunk(x[r0:r1], out[r0:r1], None, lr, cdq)
+
+        run_chunks(chunk_bounds(rows, chunk_rows or _default_chunk_rows), x.device, self.uses_range_flag,
+                   lambda i, r0, r1, flag: chunk(self, r0, r1, flag),
+                   lambda i, r0, r1: chunk(self._fallback(), r0, r1, None), ladj_rows=ladj_rows)
         return None if sink is not None else out
+
+    def final_buffer(self, device, name: str, rows: int, d_in: int) -> torch.Tensor:
+        """The workspace buffer [rows, out_width(d_in)] a chunk's result is written to when it is handed on."""
+        return _workspace.planes(device, name, rows, self.out_width(d_in), "f32")
 
     def _stream_planes(self) -> set:
         return {"fp32": {"h16", "l16"}, "fp32_tf32": {"hi", "lo"}, "bf16": {"bf16", "f32"}}.get(self.mode, {"f32"})
@@ -610,7 +623,7 @@ class Program:
         return {"fp32": {"h16", "l16"}, "fp32_tf32": {"hi", "lo"}, "bf16": {"bf16"}}.get(self.mode, {"f32"})
 
     def _run_chunk(self, x: torch.Tensor, final_out: torch.Tensor, flag: Optional[torch.Tensor] = None,
-                   ladj_rows: Optional[torch.Tensor] = None, dq: Optional[ops.Dequant] = None) -> None:
+                   dq: Optional[ops.Dequant] = None, *, ladj_rows: Optional[torch.Tensor] = None) -> None:
         """One chunk x [rows, d]; with `dq`, x is uint8 and is dequantised by the first kernel that reads it."""
         dev, rows = x.device, x.shape[0]
         steps = self.steps
@@ -774,6 +787,7 @@ class Program:
         prog = cls.__new__(cls)
         prog.mode, prog.items, prog.compress, prog.steps, prog.small, prog.has_row_ladj = mode, [], None, steps, None, False
         prog.layers, prog.direction, prog._fallback_prog, prog._wflag, prog.force_fallback = [], "forward", None, None, False
+        prog.uses_range_flag = mode == "fp32"
         return prog
 
 

@@ -82,6 +82,16 @@ class _plain_stream_order:
         return False
 
 
+def _capture(dev, body) -> "torch.cuda.CUDAGraph":
+    """`body()` captured into a CUDA graph on `dev`, after one eager pass that sizes every workspace buffer it uses."""
+    body()
+    torch.cuda.synchronize(dev)
+    graph = torch.cuda.CUDAGraph()
+    with _plain_stream_order(), torch.cuda.graph(graph, stream=capture_stream(dev), capture_error_mode="thread_local"):
+        body()
+    return graph
+
+
 def _wave_aligned_chunk_rows(prog, device) -> int:
     """Rows per H2D copy / kernel batch of `log_prob_host`: the smallest multiple of 256-row tile rows >= HOST_CHUNK_ROWS / 2
     for which the widest layer's tile count is a whole number of waves of the persistent CTA-pair kernel (one tile per
@@ -89,7 +99,7 @@ def _wave_aligned_chunk_rows(prog, device) -> int:
     of chunk i); whole waves keep the tail of every launch full."""
     import ctypes
     from . import _lib
-    if getattr(prog, "small", None) is not None:                 # one launch per chunk: copy granularity only
+    if prog.small is not None:                                   # one launch per chunk: copy granularity only
         return max(HOST_CHUNK_ROWS, (32 << 20) // (4 * prog.small["d"]))
     widest = max([st.N for st in prog.steps if st.kind == "mm"] or [0])
     if widest < 32:
@@ -247,79 +257,57 @@ class Flow(torch.nn.Module):
         x2, batch_shape = engine._flatten_rows(x, len(self._event_shape()), torch.float32 if dq is None else torch.uint8)
         if dq is not None:
             x2 = x2.contiguous()
-        d = x2.shape[1]
-        rows = x2.shape[0]
-        if isinstance(prog, image_engine.ImageProgram):      # image-shaped event: the latent arrives channels-last
-            if x2.is_cuda and 0 < rows <= SMALL_BATCH_GRAPH_IMAGES and not prog.force_fallback \
-                    and not torch.cuda.is_current_stream_capturing():
-                lp = self._log_prob_small_batch(prog, ladj, x2 if dq is None else engine._dequantized(x2, dq))
-                if lp is not None:                                  # ~100 launches per step: one graph replay instead
-                    return lp.reshape(batch_shape)
-            out = torch.empty(rows, dtype=torch.float32, device=x2.device)
-            perm = self._channels_last_perm(x2.device)
-            with torch.no_grad():
-                prog.run(x2, sink=lambda z, r0, r1: base._density_into(ops.Act(r1 - r0, d, f32=z), -ladj, out[r0:r1],
-                                                                       perm=perm), dq=dq)
-            return out.reshape(batch_shape)
-        if x2.is_cuda and 0 < rows <= SMALL_BATCH_GRAPH_ROWS and getattr(prog, "small", None) is None \
+        rows, d = x2.shape
+        images = isinstance(prog, image_engine.ImageProgram)
+        perm = self._channels_last_perm(x2.device) if images else None      # image-shaped events: the latent is channels-last
+        if x2.is_cuda and 0 < rows <= (SMALL_BATCH_GRAPH_IMAGES if images else SMALL_BATCH_GRAPH_ROWS) and prog.small is None \
                 and not prog.force_fallback and not prog.has_row_ladj and not torch.cuda.is_current_stream_capturing():
-            lp = self._log_prob_small_batch(prog, ladj, x2 if dq is None else engine._dequantized(x2, dq))
+            lp = self._log_prob_small_batch(prog, ladj, x2 if dq is None else engine._dequantized(x2, dq), perm)
             if lp is not None:
                 return lp.reshape(batch_shape)
         if USE_C_PLAN and x2.is_cuda and rows > 0 and prog.plan_able() and getattr(base, "base_kind", -1) >= 0 \
                 and not torch.cuda.is_current_stream_capturing():
             return self._log_prob_plan(prog, base, ladj, x2, dq).reshape(batch_shape)
         out = torch.empty(rows, dtype=torch.float32, device=x2.device)
-
-        def sink(z_chunk, r0, r1):
-            base._density_into(ops.Act(r1 - r0, d, f32=z_chunk), -ladj, out[r0:r1])
-
+        # affine couplings: per-row log-determinants next to the model constant
+        row_ladj = torch.zeros(rows, dtype=torch.float32, device=x2.device) if prog.has_row_ladj else None
         with torch.no_grad():
-            if prog.has_row_ladj:          # affine couplings: per-row log-determinants next to the model constant
-                row_ladj = torch.zeros(rows, dtype=torch.float32, device=x2.device)
-                prog.run(x2, sink=sink, ladj_rows=row_ladj, dq=dq)
-                if rows:
-                    ops.sub_rows(out, row_ladj)
-            else:
-                prog.run(x2, sink=sink, dq=dq)
+            prog.run(x2, sink=lambda z, r0, r1: base._density_into(ops.Act(r1 - r0, d, f32=z), -ladj, out[r0:r1], perm=perm),
+                     ladj_rows=row_ladj, dq=dq)
+            if row_ladj is not None and rows:
+                ops.sub_rows(out, row_ladj)
         return out.reshape(batch_shape)
 
     @staticmethod
     def _plan_chunks(rows: int):
-        """(chunk rows, plan capacity) as `Program.run` would cut the batch; the capacity is rounded up so that a few plans
+        """(chunk bounds, plan capacity) as `Program.run` would cut the batch; the capacity is rounded up so that a few plans
         serve every batch size."""
         cap = engine._default_chunk_rows
-        n_chunks = (rows + cap - 1) // cap
-        chunk = min(rows, ((rows + n_chunks - 1) // n_chunks + 255) // 256 * 256)
+        bounds = engine.chunk_bounds(rows, cap)
+        chunk = bounds[0][1]
         size = 4096
         while size < chunk:
             size *= 2
-        return chunk, min(size, max(cap, chunk))
+        return bounds, min(size, max(cap, chunk))
 
     def _log_prob_plan(self, prog, base, ladj: float, x2: torch.Tensor, dq: Optional[ops.Dequant] = None) -> torch.Tensor:
         """`log_prob` through the whole-stack C entry: one `usf_flow_logprob` call per chunk (ingest, every contraction and
         the base density are launched by the library).  Same kernels, same order, same bits as the launch-by-launch route."""
         rows, d = x2.shape
         x2 = x2.contiguous()
-        chunk, capacity = self._plan_chunks(rows)
+        bounds, capacity = self._plan_chunks(rows)
+        shifted = lambda r0: None if dq is None else dq.shifted(r0)        # noqa: E731
         with torch.no_grad():
             plan = prog.c_plan(d, capacity, base, -ladj)
             out = torch.empty(rows, dtype=torch.float32, device=x2.device)
-            starts = list(range(0, rows, chunk))
-            flags = torch.zeros(len(starts), dtype=torch.int32, device=x2.device) if prog.mode == "fp32" else None
-            for ci, r0 in enumerate(starts):
-                r1 = min(rows, r0 + chunk)
-                plan.log_prob(x2[r0:r1], out[r0:r1], None if flags is None else flags[ci:ci + 1],
-                              None if dq is None else dq.shifted(r0))
-            if flags is not None:                       # chunks that left the fp16 range: tf32-split engine, launch by launch
-                for ci in torch.nonzero(flags).reshape(-1).tolist():
-                    r0 = starts[ci]
-                    r1 = min(rows, r0 + chunk)
-                    prog._fallback().run(x2[r0:r1], sink=lambda z, a, b, r0=r0: base._density_into(
-                        ops.Act(b - a, z.shape[1], f32=z), -ladj, out[r0 + a:r0 + b]), dq=None if dq is None else dq.shifted(r0))
+            engine.run_chunks(
+                bounds, x2.device, prog.uses_range_flag,
+                lambda i, r0, r1, flag: plan.log_prob(x2[r0:r1], out[r0:r1], flag, shifted(r0)),
+                lambda i, r0, r1: prog._fallback().run(x2[r0:r1], sink=lambda z, a, b: base._density_into(
+                    ops.Act(b - a, z.shape[1], f32=z), -ladj, out[r0 + a:r0 + b]), dq=shifted(r0)))
         return out
 
-    def _log_prob_small_batch(self, prog, ladj: float, x2: torch.Tensor):
+    def _log_prob_small_batch(self, prog, ladj: float, x2: torch.Tensor, perm: Optional[torch.Tensor]):
         """Small batches are bound by the host-side cost of ~23 kernel launches (~40 us each through ctypes + tensor-map
         encoding), not by the kernels: the launch program + base density of a given row count is captured ONCE into a CUDA
         graph over fixed staging buffers and replayed (input copied in, result cloned out).  Returns None when a value
@@ -336,28 +324,15 @@ class Flow(torch.nn.Module):
             base._prepared()                  # parameter-side work happens here, outside any graph capture
             xin = torch.empty(rows, d, dtype=torch.float32, device=dev)
             out = torch.empty(rows, dtype=torch.float32, device=dev)
-            flag = torch.zeros(1, dtype=torch.int32, device=dev) if getattr(prog, "uses_range_flag", prog.mode == "fp32") else None
-            width = prog.out_width(d)
-            if isinstance(prog, image_engine.ImageProgram):
-                fin = image_engine._dense(dev, "img_final_small", rows, d)
-                perm = self._channels_last_perm(dev)
+            flag = torch.zeros(1, dtype=torch.int32, device=dev) if prog.uses_range_flag else None
+            fin = prog.final_buffer(dev, "final_small", rows, d)
 
-                def body():
-                    prog._run_chunk(xin, fin, False, flag)
-                    base._density_into(ops.Act(rows, d, f32=fin), -ladj, out, perm=perm)
-            else:
-                fin = engine._workspace.planes(dev, "final_small", rows, width, "f32")
-
-                def body():
-                    prog._run_chunk(xin, fin, flag)
-                    base._density_into(ops.Act(rows, width, f32=fin), -ladj, out)
+            def body():
+                prog._run_chunk(xin, fin, flag)
+                base._density_into(ops.Act(rows, fin.shape[1], f32=fin), -ladj, out, perm=perm)
             with torch.no_grad():
                 xin.copy_(x2)
-                body()                                        # eager pass: sizes every workspace buffer before capture
-                torch.cuda.synchronize(dev)
-                graph = torch.cuda.CUDAGraph()
-                with _plain_stream_order(), torch.cuda.graph(graph, stream=capture_stream(dev), capture_error_mode="thread_local"):
-                    body()
+                graph = _capture(dev, body)
             if len(cache) >= 8:                               # a few row counts per weight version; drop the oldest
                 cache.pop(next(iter(cache)))
             ent = cache[key] = dict(graph=graph, x=xin, out=out, flag=flag, gen=engine._workspace.generation)
@@ -379,16 +354,11 @@ class Flow(torch.nn.Module):
         if ent is not None and ent["gen"] == engine._workspace.generation:
             return ent
         dev = buf.device
-        rows, width = buf.shape[0], prog.out_width(d)
-        flag = torch.zeros(1, dtype=torch.int32, device=dev) if prog.mode == "fp32" else None
-        fin = engine._workspace.planes(dev, f"final_host{slot}", rows, width, "f32")
+        flag = torch.zeros(1, dtype=torch.int32, device=dev) if prog.uses_range_flag else None
+        fin = prog.final_buffer(dev, f"final_host{slot}", buf.shape[0], d)
         params = None if dq_mode is None else torch.zeros(2, dtype=torch.int64, device=dev)
         dq = None if dq_mode is None else ops.Dequant(dq_mode, 0, 0, params)
-        prog._run_chunk(buf, fin, flag, None, dq)         # eager pass: sizes every workspace buffer before capture
-        torch.cuda.synchronize(dev)
-        graph = torch.cuda.CUDAGraph()
-        with _plain_stream_order(), torch.cuda.graph(graph, stream=capture_stream(dev), capture_error_mode="thread_local"):
-            prog._run_chunk(buf, fin, flag, None, dq)
+        graph = _capture(dev, lambda: prog._run_chunk(buf, fin, flag, dq))
         ent = dict(graph=graph, fin=fin, flag=flag, params=params, gen=engine._workspace.generation)
         for k in [k for k in cache if k[0] == slot and ((k[1] != key[1] and k[3] == dq_mode) or cache[k]["gen"] != ent["gen"])]:
             del cache[k]                                  # graphs of a replaced staging buffer / of stale workspaces
@@ -429,65 +399,35 @@ class Flow(torch.nn.Module):
         rows, d = x2.shape
         if out_host is None:
             out_host = torch.empty(rows, dtype=torch.float32, pin_memory=True)
-        if isinstance(prog, image_engine.ImageProgram):
-            # image-shaped events: two staging buffers in turn, the H2D copy of chunk i + 1 on the copy stream under the
-            # kernels of chunk i, one D2H copy of all log-probs at the end
-            step = max(1, chunk_rows or HOST_CHUNK_ROWS)
-            main = torch.cuda.current_stream(dev)
-            attr = "_img_stage" if dq is None else "_img_stage_u8"      # 8-bit rows are staged as they are
-            stage = getattr(self, attr, None)
-            if stage is None or stage.shape[1:] != (min(step, max(rows, 1)), d) or stage.device != dev:
-                stage = torch.empty(2, min(step, max(rows, 1)), d, dtype=torch.float32 if dq is None else torch.uint8, device=dev)
-                setattr(self, attr, stage)
-                self._copy_stream = torch.cuda.Stream(device=dev)
-            out_dev = torch.empty(rows, dtype=torch.float32, device=dev)
-            starts = list(range(0, rows, step))
-            copied = [torch.cuda.Event() for _ in range(2)]
-            consumed = [torch.cuda.Event() for _ in range(2)]
-            self._copy_stream.wait_stream(main)
-
-            def issue_copy(i):
-                r0 = starts[i]
-                n = min(step, rows - r0)
-                with torch.cuda.stream(self._copy_stream):
-                    if i >= 2:
-                        self._copy_stream.wait_event(consumed[i % 2])
-                    stage[i % 2, :n].copy_(x2[r0:r0 + n], non_blocking=True)
-                    copied[i % 2].record(self._copy_stream)
-
-            if starts:
-                issue_copy(0)
-            for i, r0 in enumerate(starts):
-                n = min(step, rows - r0)
-                if i + 1 < len(starts):
-                    issue_copy(i + 1)
-                main.wait_event(copied[i % 2])
-                out_dev[r0:r0 + n] = self._log_prob(stage[i % 2, :n].reshape(n, *self._event_shape()),
-                                                    None if dq is None else dq.shifted(r0))
-                consumed[i % 2].record(main)
-            out_host.reshape(-1)[:rows].copy_(out_dev, non_blocking=True)
-            main.synchronize()
-            return out_host
-        # Chunk schedule.  The H2D copy of chunk i+1 hides under the kernels of chunk i (a row copies faster than it
-        # computes), so only the FIRST copy is exposed: start with the smallest wave-aligned chunk and let the later
-        # ones grow (fewer kernel boundaries, fuller tails).  An explicit `chunk_rows` gives uniform chunks.
-        unit = min(chunk_rows or _wave_aligned_chunk_rows(prog, dev), max(rows, 1))
-        sizes, left = [], rows
-        while left > 0:
-            mult = 1 if chunk_rows else HOST_CHUNK_UNITS[min(len(sizes), len(HOST_CHUNK_UNITS) - 1)]
-            take = min(unit * mult, left)
-            if left - take < unit // 2:                  # do not leave a sliver for a last launch sequence
-                take = left
-            sizes.append(take)
-            left -= take
-        chunk = max(sizes) if sizes else unit
-        starts = [sum(sizes[:i]) for i in range(len(sizes))]
-        # staging: one device buffer per chunk (slices of one allocation holding the whole batch) when that fits -- the
-        # copies then run back to back on the copy stream, independent of the kernels --, else two buffers used in turn
         # 8-bit rows are staged as they are (a quarter of the bytes), in a buffer of their own: fp32 and uint8 calls in turn
         # keep their staging buffers and captured graphs
         sdt, attr = (torch.float32, "_host_stage") if dq is None else (torch.uint8, "_host_stage_u8")
-        whole = rows * d * sdt.itemsize <= HOST_STAGE_BYTES and len(sizes) <= HOST_MAX_STAGE_SLICES
+        images = len(self._event_shape()) == 3
+        if images:
+            # image-shaped events: uniform chunks in two staging buffers in turn, each through `_log_prob` (whose routes
+            # guard their own chunks); the H2D copy of chunk i + 1 is issued before chunk i is enqueued
+            step = max(1, chunk_rows or HOST_CHUNK_ROWS)
+            bounds = [(r0, min(rows, r0 + step)) for r0 in range(0, rows, step)]
+            whole, ahead = False, 1
+        else:
+            # Chunk schedule.  The H2D copy of chunk i+1 hides under the kernels of chunk i (a row copies faster than it
+            # computes), so only the FIRST copy is exposed: start with the smallest wave-aligned chunk and let the later
+            # ones grow (fewer kernel boundaries, fuller tails).  An explicit `chunk_rows` gives uniform chunks.
+            unit = min(chunk_rows or _wave_aligned_chunk_rows(prog, dev), max(rows, 1))
+            bounds, r0 = [], 0
+            while r0 < rows:
+                mult = 1 if chunk_rows else HOST_CHUNK_UNITS[min(len(bounds), len(HOST_CHUNK_UNITS) - 1)]
+                take = min(unit * mult, rows - r0)
+                if rows - r0 - take < unit // 2:         # do not leave a sliver for a last launch sequence
+                    take = rows - r0
+                bounds.append((r0, r0 + take))
+                r0 += take
+            # staging: one device buffer per chunk (slices of one allocation holding the whole batch) when that fits -- the
+            # copies then run back to back on the copy stream, independent of the kernels --, else two buffers used in turn
+            whole = rows * d * sdt.itemsize <= HOST_STAGE_BYTES and len(bounds) <= HOST_MAX_STAGE_SLICES
+            ahead = 0
+        sizes = [r1 - r0 for r0, r1 in bounds]
+        chunk = max(sizes, default=1)
         need = max(rows, 1) if whole else 2 * chunk
         stage = getattr(self, attr, None)
         if stage is None or stage.shape[0] < need or stage.shape[1] != d or stage.device != dev:
@@ -495,32 +435,70 @@ class Flow(torch.nn.Module):
             setattr(self, attr, stage)
             self._host_out = torch.empty(0, dtype=torch.float32, device=dev)
             self._copy_stream = torch.cuda.Stream(device=dev)
-        n_buf = max(1, len(sizes)) if whole else 2
         if whole:
-            bufs = [stage[starts[i]:starts[i] + sizes[i]] for i in range(len(sizes))] or [stage[:0]]
+            bufs = [stage[r0:r1] for r0, r1 in bounds] or [stage[:0]]
         else:
             bufs = [stage[:chunk], stage[chunk:2 * chunk]]
+        n_buf = len(bufs)
         if self._host_out.numel() < rows:
             self._host_out = torch.empty(rows, dtype=torch.float32, device=dev)
         out_dev = self._host_out[:rows]
         main = torch.cuda.current_stream(dev)
         copied = [torch.cuda.Event() for _ in range(n_buf)]
         consumed = [torch.cuda.Event() for _ in range(n_buf)]
-        guarded = prog.mode == "fp32" and not prog.force_fallback       # fp16-split engine: range flag per chunk
-        flags = torch.zeros(len(starts), dtype=torch.int32, device=dev) if guarded else None
-
-        def make_sink(r0):
-            def sink(z_chunk, a, b):
-                base._density_into(ops.Act(b - a, d, f32=z_chunk), -ladj, out_dev[r0 + a:r0 + b])
-            return sink
-
-        use_graphs = HOST_CUDA_GRAPHS and not prog.force_fallback and rows >= unit and getattr(prog, "small", None) is None \
-            and not prog.has_row_ladj
+        # chunks run `_run_chunk` under a range flag; the single-launch and the always-tf32-split programs have none
+        guarded = not images and prog.uses_range_flag and prog.small is None and not prog.force_fallback
         row_ladj = torch.zeros(rows, dtype=torch.float32, device=dev) if prog.has_row_ladj else None
+        lr = lambda r0, r1: None if row_ladj is None else row_ladj[r0:r1]     # noqa: E731
+        shifted = lambda r0: None if dq is None else dq.shifted(r0)           # noqa: E731
+
+        def sink_at(r0):
+            return lambda z, a, b: base._density_into(ops.Act(b - a, d, f32=z), -ladj, out_dev[r0 + a:r0 + b])
+
+        def issue_copy(i):
+            r0, r1 = bounds[i]
+            slot = i % n_buf
+            with torch.cuda.stream(self._copy_stream):
+                if i >= n_buf:
+                    self._copy_stream.wait_event(consumed[slot])
+                bufs[slot][:r1 - r0].copy_(x2[r0:r1], non_blocking=True)
+                copied[slot].record(self._copy_stream)
+
+        def first(i, r0, r1, flag):
+            if i + ahead < len(bounds):
+                issue_copy(i + ahead)
+            slot = i % n_buf
+            buf = bufs[slot][:r1 - r0]
+            g = graphs.get((slot, r1 - r0))
+            main.wait_event(copied[slot])
+            if images:
+                out_dev[r0:r1] = self._log_prob(buf.reshape(r1 - r0, *self._event_shape()), shifted(r0))
+            elif g is not None:
+                # one graph launch replaces the ~23 kernel launches of the chunk: the host-side launch cost
+                # (~40 us per launch through ctypes + tensor-map encoding) is what bounds small chunks otherwise
+                if g["params"] is not None:
+                    g["params"].copy_(params[i])
+                g["graph"].replay()
+                sink_at(r0)(g["fin"], 0, r1 - r0)
+            elif guarded:
+                fin = prog.final_buffer(dev, "final", r1 - r0, d)
+                prog._run_chunk(buf, fin, flag, shifted(r0), ladj_rows=lr(r0, r1))
+                sink_at(r0)(fin, 0, r1 - r0)
+            else:
+                prog.run(buf, chunk_rows=chunk, sink=sink_at(r0), ladj_rows=lr(r0, r1), dq=shifted(r0))
+            consumed[slot].record(main)
+
+        def again(i, r0, r1):
+            buf = bufs[i % n_buf][:r1 - r0]
+            if n_buf < len(bounds):                       # staging buffers in turn: the slot may hold another chunk's rows
+                buf.copy_(x2[r0:r1])
+            prog._fallback().run(buf, chunk_rows=chunk, sink=sink_at(r0), ladj_rows=lr(r0, r1), dq=shifted(r0))
+
         with torch.no_grad():
-            graphs = None
-            if use_graphs:                                # one graph per (staging buffer, chunk size), largest first so
-                graphs = {}                               # that the shared workspaces are sized once
+            graphs = {}
+            if not images and HOST_CUDA_GRAPHS and not prog.force_fallback and rows >= unit and prog.small is None \
+                    and not prog.has_row_ladj:
+                # one graph per (staging buffer, chunk size), largest first so that the shared workspaces are sized once
                 for _ in range(2):                        # a workspace that grew while capturing invalidates earlier graphs
                     for i in sorted(range(len(sizes)), key=lambda j: -sizes[j]):
                         if sizes[i] >= unit // 2:
@@ -532,45 +510,13 @@ class Flow(torch.nn.Module):
                     if g["flag"] is not None:
                         g["flag"].zero_()
             if graphs and dq is not None:                 # {seed, global row} of every chunk, read by the graphs' ingest
-                params = torch.tensor([[dq.seed, dq.row0 + r0] for r0 in starts], dtype=torch.int64).to(dev)
+                params = torch.tensor([[dq.seed, dq.row0 + r0] for r0, _ in bounds], dtype=torch.int64).to(dev)
             self._copy_stream.wait_stream(main)
-            for i, r0 in enumerate(starts):
-                r1 = r0 + sizes[i]
-                slot = i % n_buf
-                buf = bufs[slot][: r1 - r0]
-                with torch.cuda.stream(self._copy_stream):
-                    if i >= n_buf:
-                        self._copy_stream.wait_event(consumed[slot])
-                    buf.copy_(x2[r0:r1], non_blocking=True)
-                    copied[slot].record(self._copy_stream)
-                main.wait_event(copied[slot])
-                g = None if graphs is None else graphs.get((slot, sizes[i]))
-                if g is not None:
-                    # one graph launch replaces the ~23 kernel launches of the chunk: the host-side launch cost
-                    # (~40 us per launch through ctypes + tensor-map encoding) is what bounds small chunks otherwise
-                    if g["params"] is not None:
-                        g["params"].copy_(params[i])
-                    g["graph"].replay()
-                    make_sink(r0)(g["fin"], 0, sizes[i])
-                else:
-                    prog.run(buf, chunk_rows=chunk, sink=make_sink(r0),
-                             flag_out=flags[i:i + 1] if guarded else None,
-                             ladj_rows=None if row_ladj is None else row_ladj[r0:r1], dq=None if dq is None else dq.shifted(r0))
-                consumed[slot].record(main)
-            if guarded:                                   # one sync; out-of-range chunks go through the tf32 split
-                redo = set(torch.nonzero(flags).reshape(-1).tolist())
-                if graphs and any(int(g["flag"].item()) != 0 for g in graphs.values() if g["flag"] is not None):
-                    redo = set(range(len(starts)))        # a graph's flag is not per chunk: recompute all of them
-                for i in sorted(redo):
-                    r0 = starts[i]
-                    r1 = r0 + sizes[i]
-                    buf = bufs[i % n_buf][: r1 - r0]
-                    buf.copy_(x2[r0:r1])
-                    if row_ladj is not None:
-                        row_ladj[r0:r1].zero_()
-                    prog._fallback().run(buf, chunk_rows=chunk, sink=make_sink(r0),
-                                         ladj_rows=None if row_ladj is None else row_ladj[r0:r1],
-                                         dq=None if dq is None else dq.shifted(r0))
+            if ahead and bounds:
+                issue_copy(0)
+            # a graph's flag is not per chunk: when one is set, every chunk is recomputed
+            engine.run_chunks(bounds, dev, guarded, first, again, shared_flags=[g["flag"] for g in graphs.values()],
+                              ladj_rows=row_ladj)
             if row_ladj is not None and rows:
                 ops.sub_rows(out_dev, row_ladj)
             out_host.reshape(-1)[:rows].copy_(out_dev, non_blocking=True)
@@ -668,20 +614,12 @@ class Flow(torch.nn.Module):
     def _apply_plan(self, prog, x2: torch.Tensor) -> torch.Tensor:
         rows, d = x2.shape
         x2 = x2.contiguous()
-        chunk, capacity = self._plan_chunks(rows)
+        bounds, capacity = self._plan_chunks(rows)
         plan = prog.c_plan(d, capacity)
-        width = prog.out_width(d)
-        y = torch.empty(rows, width, dtype=torch.float32, device=x2.device)
-        starts = list(range(0, rows, chunk))
-        flags = torch.zeros(len(starts), dtype=torch.int32, device=x2.device) if prog.mode == "fp32" else None
-        for ci, r0 in enumerate(starts):
-            r1 = min(rows, r0 + chunk)
-            plan.apply(x2[r0:r1], y[r0:r1], None if flags is None else flags[ci:ci + 1])
-        if flags is not None:
-            for ci in torch.nonzero(flags).reshape(-1).tolist():
-                r0 = starts[ci]
-                r1 = min(rows, r0 + chunk)
-                prog._fallback().run(x2[r0:r1], out=y[r0:r1])
+        y = torch.empty(rows, prog.out_width(d), dtype=torch.float32, device=x2.device)
+        engine.run_chunks(bounds, x2.device, prog.uses_range_flag,
+                          lambda i, r0, r1, flag: plan.apply(x2[r0:r1], y[r0:r1], flag),
+                          lambda i, r0, r1: prog._fallback().run(x2[r0:r1], out=y[r0:r1]))
         return y
 
     def _run(self, direction: str, x: torch.Tensor, zero_ctx: bool = False) -> torch.Tensor:
@@ -690,8 +628,7 @@ class Flow(torch.nn.Module):
         x2, batch_shape = engine._flatten_rows(x, len(self._event_shape()))
         with torch.no_grad(), ops.on_device(x2):
             prog, _ = self._program(direction, zero_ctx)
-            if USE_C_PLAN and x2.is_cuda and x2.shape[0] > 0 and isinstance(prog, engine.Program) and prog.plan_able() \
-                    and not torch.cuda.is_current_stream_capturing():
+            if USE_C_PLAN and x2.is_cuda and x2.shape[0] > 0 and prog.plan_able() and not torch.cuda.is_current_stream_capturing():
                 y = self._apply_plan(prog, x2)
             else:
                 y = prog.run(x2)

@@ -310,9 +310,17 @@ class ImageProgram:
     def out_width(self, d_in: int) -> int:
         return d_in
 
+    def plan_able(self) -> bool:                             # the whole-stack C entry covers flat events only
+        return False
+
+    def final_buffer(self, device, name: str, rows: int, d_in: int) -> torch.Tensor:
+        """The workspace buffer [rows, d_in] a channels-last chunk result is written to when it is handed on."""
+        return _dense(device, "img_" + name, rows, d_in)
+
     # ----------------------------------------------------------------------------------------------
-    def _run_chunk(self, x: torch.Tensor, out: torch.Tensor, nchw_out: bool, flag, dq: Optional[ops.Dequant] = None) -> None:
-        """x [n, C*H*W] (NCHW, read-only) -> out [n, C*H*W]: NCHW when `nchw_out`, else channels-last ([n, H*W*C]).  With
+    def _run_chunk(self, x: torch.Tensor, out: torch.Tensor, flag, dq: Optional[ops.Dequant] = None, *,
+                   nchw_out: bool = False) -> None:
+        """x [n, C*H*W] (NCHW, read-only) -> out [n, C*H*W]: channels-last ([n, H*W*C]), or NCHW when `nchw_out`.  With
         `dq`, x is uint8 and the NCHW -> channels-last conversion dequantises it."""
         dev, n = x.device, x.shape[0]
         rows, C, HW = n * self.HW, self.C, self.HW
@@ -359,40 +367,36 @@ class ImageProgram:
             ops.layout_transpose(cur, n, HW, C, tmp, scale=xs[0], scale_mode=xs[1], scale_on_input=False)
             ops.layout_transpose(tmp, n, C, HW, out)
 
-    def run(self, x: torch.Tensor, nchw_out: bool = True, sink=None, chunk_rows: Optional[int] = None,
-            dq: Optional[ops.Dequant] = None) -> Optional[torch.Tensor]:
+    def run(self, x: torch.Tensor, *, out: Optional[torch.Tensor] = None, sink=None, chunk_rows: Optional[int] = None,
+            ladj_rows: Optional[torch.Tensor] = None, dq: Optional[ops.Dequant] = None) -> Optional[torch.Tensor]:
         """x [N, C*H*W] -> [N, C*H*W] (NCHW order), or per chunk `sink(channels_last_chunk [n, H*W*C], r0, r1)`; with `dq`, x
-        is uint8 (see _run_chunk)."""
+        is uint8 (see _run_chunk).  `ladj_rows` is never written: no image step has per-row log-determinants."""
         ops.require_cuda(x, "input", torch.float32 if dq is None else torch.uint8)
         x = x.contiguous()
         N, d = x.shape
         if d != self.C * self.HW:
             raise RuntimeError("usflows_b200: event shape mismatch")
-        out = None if sink is not None else torch.empty(N, d, dtype=torch.float32, device=x.device)
+        if sink is None and out is None:
+            out = torch.empty(N, d, dtype=torch.float32, device=x.device)
         if N == 0:
             return out
         if self.force_fallback:
-            return self._fallback().run(x, nchw_out, sink, chunk_rows, dq)
+            return self._fallback().run(x, out=out, sink=sink, chunk_rows=chunk_rows, dq=dq)
         all_pix = all(op[0] != "coupling" or op[1].pix is not None for op in self.ops)
         per = max(1, (chunk_rows or (IMAGE_CHUNK_ROWS_PIX if all_pix else IMAGE_CHUNK_ROWS)) // self.HW)
-        starts = list(range(0, N, per))
-        flags = torch.zeros(len(starts), dtype=torch.int32, device=x.device) if self.uses_range_flag else None
 
-        def one(prog, i, r0, flag):
-            r1 = min(N, r0 + per)
+        def chunk(prog, r0, r1, flag):
             cdq = None if dq is None else dq.shifted(r0)
             if sink is not None:
-                fin = _dense(x.device, "img_final", r1 - r0, d)
-                prog._run_chunk(x[r0:r1], fin, False, flag, cdq)
+                fin = self.final_buffer(x.device, "final", r1 - r0, d)
+                prog._run_chunk(x[r0:r1], fin, flag, cdq)
                 sink(fin, r0, r1)
             else:
-                prog._run_chunk(x[r0:r1], out[r0:r1], nchw_out, flag, cdq)
+                prog._run_chunk(x[r0:r1], out[r0:r1], flag, cdq, nchw_out=True)
 
-        for i, r0 in enumerate(starts):
-            one(self, i, r0, None if flags is None else flags[i:i + 1])
-        if flags is not None:                                # chunks that left the fp16 range: tf32-split engine
-            for i in torch.nonzero(flags).reshape(-1).tolist():
-                one(self._fallback(), i, starts[i], None)
+        engine.run_chunks([(r0, min(N, r0 + per)) for r0 in range(0, N, per)], x.device, self.uses_range_flag,
+                          lambda i, r0, r1, flag: chunk(self, r0, r1, flag),
+                          lambda i, r0, r1: chunk(self._fallback(), r0, r1, None))
         return out
 
 

@@ -26,7 +26,7 @@ import torch
 
 from . import engine, ops
 
-_UNCOPIED = ("_programs", "_host_stage", "_host_stage_u8", "_host_out", "_img_stage", "_img_stage_u8", "_copy_stream", "_cl_perm",
+_UNCOPIED = ("_programs", "_host_stage", "_host_stage_u8", "_host_out", "_copy_stream", "_cl_perm",
              "_cl_perm_key", "_sharded")
 
 
