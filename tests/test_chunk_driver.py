@@ -161,6 +161,21 @@ def test_only_the_flagged_image_chunk_is_rerun(fake_ops, monkeypatch, what):
     _check_rerun(got, want16, want_tf, [(4, 8)])
 
 
+def test_only_the_flagged_chunk_of_a_network_run_alone_is_rerun(fake_ops, monkeypatch):
+    """nn.DenseNN / nn.ConvNet called on their own (engine.run_mlp / run_conditioner): chunk 1 leaves the fp16 range and is
+    recomputed with the network's own tf32-split launches."""
+    from usflows_b200 import engine, nn
+    monkeypatch.setattr(engine, "_default_chunk_rows", 256)
+    torch.manual_seed(0)
+    x, big = _rows(600, [64], [(256, 512)], 3e5)
+    for run, net in ((engine.run_mlp, nn.DenseNN(64, [64, 64], [64])), (engine.run_conditioner, nn.ConvNet([64], [64, 64]))):
+        want16, want_tf = run(net, x, "fp32"), run(net, big, "fp32_tf32")
+        fake_backend.CALLS.clear()
+        got = run(net, big, "fp32")
+        assert {c[2] for c in _tf32_split_calls()} == {256}
+        _check_rerun(got, want16, want_tf, [(256, 512)])
+
+
 # ---- B200 ------------------------------------------------------------------------------------------------------------
 @pytest.mark.gpu
 @pytest.mark.parametrize("what", ["log_prob", "backward"])

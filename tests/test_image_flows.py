@@ -122,6 +122,21 @@ def test_image_flow_api_shapes(fake_ops):
     assert rel_err(per_layer, arr["ladj32"]) <= 2e-6                   # BlockAffine: inner x H*W (transforms.py:964-980)
 
 
+def test_image_program_rejects_a_wrong_event_width(fake_ops):
+    """The event width is checked before any kernel reads the rows, also where no output is allocated: `log_prob` hands
+    each chunk to a sink, `run(out=...)` writes into the caller's buffer."""
+    spec, params, arr = load_case("img_mnist_16x7x7")
+    flow = build_flow(spec, params, device="cpu")
+    x = arr["x"][:20, :, :, :6].contiguous()                          # [20, 16, 7, 6]: one column short
+    fake_ops.CALLS.clear()
+    with pytest.raises(RuntimeError, match="event shape mismatch"):
+        flow.log_prob(x)
+    prog, _ = flow._program("backward")
+    with pytest.raises(RuntimeError, match="event shape mismatch"):
+        prog.run(x.reshape(20, -1), out=torch.empty(20, 16 * 7 * 7))
+    assert fake_ops.CALLS == []
+
+
 def test_convnet2d_module_matches_oracle(fake_ops):
     import usflows_b200 as U
     spec, params, _ = load_case("img_mnist_16x7x7")

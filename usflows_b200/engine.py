@@ -101,6 +101,11 @@ def _engine_for(mode: str, N: int, K: int) -> int:
     return {"fp32": ENGINE_TC_3XF16, "fp32_tf32": ENGINE_TC_3XTF32, "tf32": ENGINE_TC_TF32, "bf16": ENGINE_TC_BF16}[mode]
 
 
+def _planes(mode: str) -> tuple:
+    """The operand planes of a mode: those of the engine its contractions of tensor-core width run on."""
+    return ops.ENGINE_PLANES[_engine_for(mode, TC_MIN_DIM, TC_MIN_DIM)]
+
+
 @dataclass
 class Prim:
     """One primitive op of the lowered layer stack (direction already applied)."""
@@ -224,33 +229,24 @@ class Step:
 
 
 def _operand(w64_or_32: torch.Tensor, mode: str, engine: int, overflow_flag: Optional[torch.Tensor] = None):
-    """fp32/fp64 weight [N, K] -> operand planes of the engine, pitch padded to a 16-byte multiple."""
+    """fp32/fp64 weight [N, K] -> operand planes of the engine (ops.ENGINE_PLANES), zero-filled, pitch padded to a 16-byte
+    multiple: (plane, None), or (hi, lo) of a split format, two planes of ONE allocation with hi first."""
     w = w64_or_32.to(torch.float32)
     rows, cols = w.shape
     ld = pad4(cols)
+    src = torch.zeros(rows, ld, dtype=torch.float32, device=w.device)[:, :cols]
+    src.copy_(w)
+    if ops.ENGINE_PLANES[engine] == ("f32",):
+        return src, None
+    dtype = {ENGINE_TC_3XF16: torch.float16, ENGINE_TC_3XTF32: torch.float32, ENGINE_TC_BF16: torch.bfloat16}[engine]
+    buf = torch.zeros(len(ops.ENGINE_PLANES[engine]), rows, ld, dtype=dtype, device=w.device)[:, :, :cols]
     if engine == ENGINE_TC_3XF16:
-        src = torch.zeros(rows, ld, dtype=torch.float32, device=w.device)[:, :cols]
-        src.copy_(w)
-        buf = torch.zeros(2, rows, ld, dtype=torch.float16, device=w.device)
-        hi, lo = buf[0, :, :cols], buf[1, :, :cols]
-        ops.split_f16(src, hi, lo, overflow_flag)
-        return hi, lo
-    if engine == ENGINE_TC_3XTF32:
-        buf = torch.zeros(2, rows, ld, dtype=torch.float32, device=w.device)
-        hi, lo = buf[0, :, :cols], buf[1, :, :cols]
-        src = torch.zeros(rows, ld, dtype=torch.float32, device=w.device)[:, :cols]
-        src.copy_(w)
-        ops.split_tf32(src, hi, lo)
-        return hi, lo
-    if engine == ENGINE_TC_BF16:
-        src = torch.zeros(rows, ld, dtype=torch.float32, device=w.device)[:, :cols]
-        src.copy_(w)
-        b = torch.zeros(rows, ld, dtype=torch.bfloat16, device=w.device)[:, :cols]
-        ops.to_bf16(src, b)
-        return b, None
-    b = torch.zeros(rows, ld, dtype=torch.float32, device=w.device)[:, :cols]
-    b.copy_(w)
-    return b, None
+        ops.split_f16(src, buf[0], buf[1], overflow_flag)
+    elif engine == ENGINE_TC_3XTF32:
+        ops.split_tf32(src, buf[0], buf[1])
+    else:
+        ops.to_bf16(src, buf[0])
+    return buf[0], buf[1] if len(buf) == 2 else None
 
 
 def convnet_steps(mode: str, desc: dict, first_w, first_b, last_w, last_b, wflag=None, *, in_seg=None, out_seg=None,
@@ -290,19 +286,88 @@ def convnet_steps(mode: str, desc: dict, first_w, first_b, last_w, last_b, wflag
     return steps
 
 
-class Program:
-    """Launch program of one direction of a layer stack for one precision mode and weight version."""
+class ProgramCore:
+    """What the launch programs of flat (Program) and image-shaped (image_engine.ImageProgram) events share: the lowering of
+    the layer stack, the fp16-range policy for weights, the tf32-split fallback and the chunked `run`.  A subclass supplies
+      _build(prims)          its launches from the lowered stack, and `uses_range_flag`
+      _in_mode(mode)         the same program in another precision mode (the tf32-split fallback)
+      _chunk_bounds(rows, chunk_rows) -> [(r0, r1), ...]
+      _chunk(x, out, flag, dq, ladj_rows, to_caller)   one chunk into `out`: the caller's output when `to_caller`, else
+                             the `final_buffer` handed to a sink
+      out_width(d_in)"""
 
-    def __init__(self, layers, direction: str, mode: Optional[str] = None):
+    fp16_weight_modes = ("fp32",)      # the modes whose weight preparation writes fp16 split planes
+
+    def __init__(self, layers, direction: str, mode: Optional[str]):
         self.mode = mode or _default_precision
         self.layers, self.direction = list(layers), direction
-        self._fallback_prog: Optional["Program"] = None
+        self._fallback_prog: Optional["ProgramCore"] = None
         self._wflag: Optional[torch.Tensor] = None          # set by weight preparation if a weight leaves fp16 range
-        self.force_fallback = False
-        seq = list(layers) if direction == "forward" else list(reversed(list(layers)))
         prims: List[Prim] = []
-        for layer in seq:
+        for layer in (self.layers if direction == "forward" else self.layers[::-1]):
             _lower_layer(layer, direction, prims)
+        self._build(prims)
+        # a weight does not fit fp16: always run the tf32-split program
+        self.force_fallback = self._wflag is not None and int(self._wflag.item()) != 0
+
+    def _weight_flag(self, device) -> Optional[torch.Tensor]:
+        """The device flag weight preparation sets when a weight leaves the fp16 range (None in modes without fp16 weights)."""
+        if self.mode not in self.fp16_weight_modes:
+            return None
+        if self._wflag is None:
+            self._wflag = torch.zeros(1, dtype=torch.int32, device=device)
+        return self._wflag
+
+    def _fallback(self) -> "ProgramCore":
+        """The same program in "fp32_tf32" mode: the same accuracy class without the fp16 range limit."""
+        if self._fallback_prog is None:
+            self._fallback_prog = self._in_mode("fp32_tf32")
+        return self._fallback_prog
+
+    def run(self, x: torch.Tensor, *, out: Optional[torch.Tensor] = None, sink=None, chunk_rows: Optional[int] = None,
+            ladj_rows: Optional[torch.Tensor] = None, dq: Optional[ops.Dequant] = None) -> Optional[torch.Tensor]:
+        """Evaluate the program on x [rows, d] chunk by chunk into `out` (allocated when None).  With `sink`, the result of
+        each chunk is handed to `sink(chunk_f32 [r, width], r0, r1)` from a reused workspace buffer (`final_buffer`)
+        instead.  With `dq`, x is uint8 and its first ingest dequantises it (ops.Dequant).  `ladj_rows` [rows]: per-row
+        log-determinants the affine couplings add to."""
+        ops.require_cuda(x, "input", torch.float32 if dq is None else torch.uint8)
+        if x.dim() != 2:
+            raise RuntimeError("usflows_b200: expected a [rows, d] input")
+        x = x.contiguous()
+        rows, width = x.shape[0], self.out_width(x.shape[1])         # out_width also rejects a wrong event width
+        if sink is None and out is None:
+            out = torch.empty(rows, width, dtype=torch.float32, device=x.device)
+        if rows == 0:                       # empty batch: nothing to launch
+            return None if sink is not None else out
+        if self.force_fallback:
+            return self._fallback().run(x, out=out, sink=sink, chunk_rows=chunk_rows, ladj_rows=ladj_rows, dq=dq)
+
+        def chunk(prog, r0, r1, flag):
+            fin = out[r0:r1] if sink is None else self.final_buffer(x.device, "final", r1 - r0, x.shape[1])
+            prog._chunk(x[r0:r1], fin, flag, None if dq is None else dq.shifted(r0),
+                        None if ladj_rows is None else ladj_rows[r0:r1], sink is None)
+            if sink is not None:
+                sink(fin, r0, r1)
+
+        run_chunks(self._chunk_bounds(rows, chunk_rows), x.device, self.uses_range_flag,
+                   lambda i, r0, r1, flag: chunk(self, r0, r1, flag),
+                   lambda i, r0, r1: chunk(self._fallback(), r0, r1, None), ladj_rows=ladj_rows)
+        return None if sink is not None else out
+
+
+class Program(ProgramCore):
+    """Launch program of one direction of a layer stack for one precision mode and weight version."""
+
+    def __init__(self, layers, direction: str, mode: Optional[str] = None, build=None):
+        """`build(mode)` -> the launch steps of a program that evaluates one conditioner network alone (`layers` is then
+        empty)."""
+        self.build = build
+        super().__init__(layers, direction, mode)
+
+    def _in_mode(self, mode: str) -> "Program":
+        return Program(self.layers, self.direction, mode, self.build)
+
+    def _build(self, prims: List[Prim]) -> None:
         # 1. compose maximal runs of affine-like maps that contain at least one dense matrix
         items: List[Prim] = []
         run: List[Prim] = []
@@ -349,9 +414,7 @@ class Program:
             self.mode = "fp32_simt"
             compress = self._compression_plan(items)
         self.compress = compress
-        self.steps = self._emit(items, compress)
-        if self._wflag is not None and int(self._wflag.item()) != 0:
-            self.force_fallback = True                          # a weight does not fit fp16: always run 3xTF32
+        self.steps = self._emit(items, compress) if self.build is None else self.build(self.mode)
         self.uses_range_flag = self.mode == "fp32"              # fp16 split planes: chunks carry a range flag
 
     # -- tiny event sizes: pack every layer into one weight blob + op list for the whole-flow kernel
@@ -425,18 +488,6 @@ class Program:
         return dict(prog=torch.tensor(prog, dtype=torch.int32, device=dev), blob=torch.cat(blocks).contiguous(),
                     n_ops=len(items), D=D, H=H, d=d)
 
-    def _flag_for_weights(self, device) -> Optional[torch.Tensor]:
-        if self.mode != "fp32":
-            return None
-        if self._wflag is None:
-            self._wflag = torch.zeros(1, dtype=torch.int32, device=device)
-        return self._wflag
-
-    def _fallback(self) -> "Program":
-        if self._fallback_prog is None:
-            self._fallback_prog = Program(self.layers, self.direction, "fp32_tf32")
-        return self._fallback_prog
-
     # -- mask compression: run the couplings in a feature order that makes "conditioner inputs" and "updated
     #    features" two contiguous column segments, so the first / last conditioner GEMMs shrink to half size
     def _compression_plan(self, items):
@@ -466,6 +517,28 @@ class Program:
             return None
         return dict(part=part, idx1=idx1, idx0=idx0, order=torch.cat([idx1, idx0]), h1=h1, h0=h0)
 
+    @staticmethod
+    def _coupling_io(mask, compress, ws, bs, affine: bool = False):
+        """(in_seg, out_seg) of a coupling's conditioner, whose Linear weights / biases `ws` / `bs` (first to last) are
+        adapted in place.  With mask compression the conditioner reads the column segment in_seg and updates out_seg, and
+        its first / last Linear keep only those columns / rows; else both segments are None and the mask is folded into
+        the first / last Linear.  `affine`: the last Linear's rows are [log-scale | shift], both halves are re-indexed."""
+        if compress is None:
+            m = mask.reshape(-1).to(torch.float32)
+            g = torch.cat([1 - m, 1 - m]) if affine else 1 - m
+            ws[0] = ws[0] * m[None, :]
+            ws[-1], bs[-1] = ws[-1] * g[:, None], bs[-1] * g
+            return None, None
+        first = torch.equal(mask, compress["part"])                 # the conditioner reads the idx1 features
+        idx_in = compress["idx1"] if first else compress["idx0"]
+        idx_out = compress["idx0"] if first else compress["idx1"]
+        if affine:                                                  # rows [0, d): log-scale, [d, 2d): shift
+            idx_out = torch.cat([idx_out, mask.numel() + idx_out])
+        ws[0] = ws[0][:, idx_in]
+        ws[-1], bs[-1] = ws[-1][idx_out], bs[-1][idx_out]
+        h1, h0 = compress["h1"], compress["h0"]
+        return ((0, h1), (h1, h0)) if first else ((h1, h0), (0, h1))
+
     def _emit(self, items, compress) -> List[Step]:
         mode = self.mode
         steps: List[Step] = []
@@ -481,60 +554,25 @@ class Program:
                         c = None if c is None else c[compress["order"]]
                 N, K = W.shape
                 eng = _engine_for(mode, N, K)
-                w, w_lo = _operand(W, mode, eng, self._flag_for_weights(W.device))
+                w, w_lo = _operand(W, mode, eng, self._weight_flag(W.device))
                 bias = None if c is None else c.to(torch.float32).contiguous()
                 steps.append(Step("mm", w=w, w_lo=w_lo, N=N, K=K, engine=eng, bias=bias))
             elif p.kind == "coupling" and p.prep.get("net") == "convnet":
-                desc, mask = p.prep["desc"], p.prep["mask"]
-                first_w, first_b = desc["first"]
-                last_w, last_b = desc["last"]
-                in_seg = out_seg = None
-                if compress is not None:
-                    first = torch.equal(mask, compress["part"])
-                    idx_in = compress["idx1"] if first else compress["idx0"]
-                    idx_out = compress["idx0"] if first else compress["idx1"]
-                    h1, h0 = compress["h1"], compress["h0"]
-                    in_seg = (0, h1) if first else (h1, h0)
-                    out_seg = (h1, h0) if first else (0, h1)
-                    first_w, last_w, last_b = first_w[:, idx_in], last_w[idx_out], last_b[idx_out]
-                else:                                                   # fold the mask into the first / last Linear
-                    m = mask.reshape(-1).to(torch.float32)
-                    first_w, last_w, last_b = first_w * m[None, :], last_w * (1 - m)[:, None], last_b * (1 - m)
-                steps += convnet_steps(mode, desc, first_w, first_b, last_w, last_b, self._flag_for_weights(first_w.device),
+                desc = p.prep["desc"]
+                ws, bs = [desc["first"][0], desc["last"][0]], [desc["first"][1], desc["last"][1]]
+                in_seg, out_seg = self._coupling_io(p.prep["mask"], compress, ws, bs)
+                steps += convnet_steps(mode, desc, ws[0], bs[0], ws[1], bs[1], self._weight_flag(ws[0].device),
                                        in_seg=in_seg, out_seg=out_seg, resid=True, sign=p.sign)
             elif p.kind == "coupling":
-                ws, bs, mask = p.prep["weights"], p.prep["biases"], p.prep["mask"]
+                ws, bs = list(p.prep["weights"]), list(p.prep["biases"])
                 nl = len(ws)
                 affine = bool(p.prep.get("affine"))
-                dfull = mask.numel()
-                in_seg = out_seg = None
-                ws = list(ws)
-                bs = list(bs)
-                if compress is not None:
-                    first = torch.equal(mask, compress["part"])       # conditioner reads the idx1 features
-                    idx_in = compress["idx1"] if first else compress["idx0"]
-                    idx_out = compress["idx0"] if first else compress["idx1"]
-                    h1, h0 = compress["h1"], compress["h0"]
-                    in_seg = (0, h1) if first else (h1, h0)
-                    out_seg = (h1, h0) if first else (0, h1)
-                    ws[0] = ws[0][:, idx_in]
-                    if affine:                                          # rows [0,d): log-scale, [d,2d): shift
-                        ws[-1] = torch.cat([ws[-1][idx_out], ws[-1][dfull + idx_out]])
-                        bs[-1] = torch.cat([bs[-1][idx_out], bs[-1][dfull + idx_out]])
-                    else:
-                        ws[-1] = ws[-1][idx_out]
-                        bs[-1] = bs[-1][idx_out]
-                else:                                                   # fold the mask into the first / last Linear
-                    m = mask.reshape(-1).to(torch.float32)
-                    ws[0] = ws[0] * m[None, :]
-                    g = torch.cat([1 - m, 1 - m]) if affine else 1 - m
-                    ws[-1] = ws[-1] * g[:, None]
-                    bs[-1] = bs[-1] * g
+                in_seg, out_seg = self._coupling_io(p.prep["mask"], compress, ws, bs, affine)
                 for j in range(nl):
                     last = j == nl - 1
                     N, K = ws[j].shape
                     eng = _engine_for(mode, N, K)
-                    w, w_lo = _operand(ws[j], mode, eng, self._flag_for_weights(ws[j].device))
+                    w, w_lo = _operand(ws[j], mode, eng, self._weight_flag(ws[j].device))
                     if last and affine:
                         steps.append(Step("mm", src="x" if j == 0 else "h", dst="st", w=w, w_lo=w_lo, N=N, K=K, engine=eng,
                                           bias=bs[j].to(torch.float32).contiguous(), in_seg=in_seg if j == 0 else None))
@@ -574,59 +612,35 @@ class Program:
 
     def run(self, x: torch.Tensor, *, out: Optional[torch.Tensor] = None, sink=None, chunk_rows: Optional[int] = None,
             ladj_rows: Optional[torch.Tensor] = None, dq: Optional[ops.Dequant] = None) -> Optional[torch.Tensor]:
-        """Evaluate the program on x [rows, d].  With `sink`, the final stream value of each chunk is handed
-        to `sink(chunk_f32 [r, width], r0, r1)` from a reused workspace buffer instead of being stored.  With `dq`, x is
-        uint8 and its first ingest dequantises it (ops.Dequant)."""
-        ops.require_cuda(x, "input", torch.float32 if dq is None else torch.uint8)
-        if x.dim() != 2:
-            raise RuntimeError("usflows_b200: expected a [rows, d] input")
-        x = x.contiguous()
-        rows = x.shape[0]
-        width = self.out_width(x.shape[1])
-        if rows == 0:                       # empty batch: nothing to launch
-            return None if sink is not None else torch.empty(0, width, dtype=torch.float32, device=x.device)
-        if dq is not None and self.small is not None and x.shape[1] == self.small["d"]:
-            x, dq = _dequantized(x, dq), None                   # one launch for the whole stack: it reads fp32
-        if self.small is not None and x.shape[1] == self.small["d"]:
-            sm = self.small
-            res = out if (out is not None and sink is None) else torch.empty(rows, sm["d"], dtype=torch.float32, device=x.device)
+        sm = self.small
+        if sm is not None and x.dim() == 2 and x.shape[0] and x.shape[1] == sm["d"]:    # one launch for the whole stack
+            ops.require_cuda(x, "input", torch.float32 if dq is None else torch.uint8)
+            x = x.contiguous() if dq is None else _dequantized(x.contiguous(), dq)        # it reads fp32
+            res = out if (out is not None and sink is None) else torch.empty(x.shape, dtype=torch.float32, device=x.device)
             ops.flow_small(x, sm["prog"], sm["blob"], sm["n_ops"], sm["D"], sm["H"], res)
             if sink is not None:
-                sink(res, 0, rows)
+                sink(res, 0, x.shape[0])
                 return None
             return res
-        if self.force_fallback:
-            return self._fallback().run(x, out=out, sink=sink, chunk_rows=chunk_rows, ladj_rows=ladj_rows, dq=dq)
-        if sink is None and out is None:
-            out = torch.empty(rows, width, dtype=torch.float32, device=x.device)
+        return super().run(x, out=out, sink=sink, chunk_rows=chunk_rows, ladj_rows=ladj_rows, dq=dq)
 
-        def chunk(prog, r0, r1, flag):
-            fin = out[r0:r1] if sink is None else self.final_buffer(x.device, "final", r1 - r0, x.shape[1])
-            prog._run_chunk(x[r0:r1], fin, flag, None if dq is None else dq.shifted(r0),
-                            ladj_rows=None if ladj_rows is None else ladj_rows[r0:r1])
-            if sink is not None:
-                sink(fin, r0, r1)
+    def _chunk_bounds(self, rows: int, chunk_rows: Optional[int]):
+        return chunk_bounds(rows, chunk_rows or _default_chunk_rows)
 
-        run_chunks(chunk_bounds(rows, chunk_rows or _default_chunk_rows), x.device, self.uses_range_flag,
-                   lambda i, r0, r1, flag: chunk(self, r0, r1, flag),
-                   lambda i, r0, r1: chunk(self._fallback(), r0, r1, None), ladj_rows=ladj_rows)
-        return None if sink is not None else out
+    def _chunk(self, x, out, flag, dq, ladj_rows, to_caller: bool) -> None:
+        self._run_chunk(x, out, flag, dq, ladj_rows=ladj_rows)
 
     def final_buffer(self, device, name: str, rows: int, d_in: int) -> torch.Tensor:
         """The workspace buffer [rows, out_width(d_in)] a chunk's result is written to when it is handed on."""
         return _workspace.planes(device, name, rows, self.out_width(d_in), "f32")
-
-    def _stream_planes(self) -> set:
-        return {"fp32": {"h16", "l16"}, "fp32_tf32": {"hi", "lo"}, "bf16": {"bf16", "f32"}}.get(self.mode, {"f32"})
-
-    def _hidden_planes(self) -> set:
-        return {"fp32": {"h16", "l16"}, "fp32_tf32": {"hi", "lo"}, "bf16": {"bf16"}}.get(self.mode, {"f32"})
 
     def _run_chunk(self, x: torch.Tensor, final_out: torch.Tensor, flag: Optional[torch.Tensor] = None,
                    dq: Optional[ops.Dequant] = None, *, ladj_rows: Optional[torch.Tensor] = None) -> None:
         """One chunk x [rows, d]; with `dq`, x is uint8 and is dequantised by the first kernel that reads it."""
         dev, rows = x.device, x.shape[0]
         steps = self.steps
+        hidden = _planes(self.mode)                                       # conditioner hidden and contraction operands
+        stream = hidden + ("f32",) if self.mode == "bf16" else hidden      # bf16: the residual stream stays fp32 too
         flip = {"x": 0, "h": 0}
         cur: Optional[Act] = None               # stream
         hid: Optional[Act] = None               # conditioner hidden
@@ -634,7 +648,7 @@ class Program:
         res_buf: Optional[torch.Tensor] = None  # ConvNet conditioner: fp32 residual stream of the gated blocks
         st_buf: Optional[torch.Tensor] = None   # fp32 scratch: affine coupling [log-scale | shift], ConvNet [val | gate]
 
-        def new_act(slot: str, width: int, planes: set) -> Act:
+        def new_act(slot: str, width: int, planes: tuple) -> Act:
             flip[slot] ^= 1
             a = Act(rows, width)
             for pl in planes:
@@ -662,14 +676,14 @@ class Program:
         src_f32 = Act(rows, x.shape[1], f32=x if dq is None else None)
         cur = src_f32
         if dq is not None and steps and steps[0].kind in ("leaky", "permute"):    # kernels that read fp32 only
-            cur = new_act("x", x.shape[1], {"f32"})
+            cur = new_act("x", x.shape[1], ("f32",))
             ingest(src_f32, cur)
         for i, st in enumerate(steps):
             nxt = steps[i + 1] if i + 1 < len(steps) else None
             if st.kind == "mm":
                 if st.src == "x":
                     in_coupling = st.dst in ("h", "st") or st.resid
-                    need = self._stream_planes() if in_coupling else self._operand_planes()
+                    need = stream if in_coupling else hidden
                     direct_ok = st.engine == ENGINE_SIMT or (x.data_ptr() % 16 == 0 and x.stride(0) % 4 == 0)
                     if not all(getattr(cur, pl) is not None for pl in need) or (cur is src_f32 and not direct_ok):
                         if cur.f32 is None and not (cur is src_f32 and dq is not None):
@@ -684,7 +698,7 @@ class Program:
                     out = Act(rows, st.N, f32=_workspace.planes(dev, st.dst, rows, st.N, "f32"))
                     resid = None
                 elif st.dst == "h":
-                    out = new_act("h", st.N, self._hidden_planes())
+                    out = new_act("h", st.N, hidden)
                     resid = None
                 elif st.resid:                                         # coupling output
                     if st.out_seg is not None:                         # in place on the updated column segment
@@ -693,7 +707,7 @@ class Program:
                         full_out = cur
                     else:
                         resid = cur
-                        out = new_act("x", st.N, self._stream_planes())
+                        out = new_act("x", st.N, stream)
                         full_out = out
                     if st.final:
                         if st.out_seg is not None:
@@ -707,10 +721,8 @@ class Program:
                     if st.final:
                         out = Act(rows, st.N, f32=final_out)
                     else:
-                        planes = set(self._stream_planes())
-                        if nxt is not None and nxt.kind in ("leaky", "permute", "vec"):
-                            planes = {"f32"}
-                        out = new_act("x", st.N, planes)
+                        elementwise_next = nxt is not None and nxt.kind in ("leaky", "permute", "vec")
+                        out = new_act("x", st.N, ("f32",) if elementwise_next else stream)
                     full_out = out
                 ops.linear(st.engine, a, st.w, st.w_lo, st.N, st.K, bias=st.bias, relu=st.relu, resid=resid,
                            resid_sign=st.sign, out=out, overflow_flag=flag)
@@ -723,11 +735,11 @@ class Program:
                 else:
                     cur = full_out
             elif st.kind == "gate":                                    # ConvNet conditioner glue between two contractions
-                act = new_act("h", st.N, self._hidden_planes())
+                act = new_act("h", st.N, hidden)
                 raw = None
                 if st.want_raw:
                     raw = Act(rows, st.N)
-                    for pl in self._hidden_planes():
+                    for pl in hidden:
                         setattr(raw, pl, _workspace.planes(dev, "hr", rows, st.N, pl))
                 y = None
                 if st.keep_f32:                                        # gated: in place on the residual stream
@@ -740,7 +752,7 @@ class Program:
                     res_buf = y
             elif st.kind == "affine":                                  # x_seg <- x_seg * exp(s) + t  (or the inverse), in place
                 if cur is src_f32:                                     # never update the caller's tensor
-                    b = new_act("x", cur.width, self._stream_planes())
+                    b = new_act("x", cur.width, stream)
                     ingest(cur, b, overflow_flag=flag)
                     cur = b
                 target = seg_view(cur, st.out_seg)
@@ -750,7 +762,7 @@ class Program:
             else:                                                      # elementwise kernels on the fp32 plane
                 if cur.f32 is None and not (st.kind == "vec" and cur is src_f32 and dq is not None):
                     raise RuntimeError("internal: elementwise step needs an fp32 stream plane")
-                out = Act(rows, cur.width, f32=final_out) if st.final else new_act("x", cur.width, {"f32"})
+                out = Act(rows, cur.width, f32=final_out) if st.final else new_act("x", cur.width, ("f32",))
                 if st.kind == "vec":
                     ingest(cur, out, div=st.vec_div, mul=st.vec_mul)
                 elif st.kind == "leaky":
@@ -778,18 +790,6 @@ class Program:
                 cache.pop(next(iter(cache))).close()
             cache[key] = CPlan(self, d_in, max_rows, base, add_const)
         return cache[key]
-
-    def _operand_planes(self) -> set:
-        return {"fp32": {"h16", "l16"}, "fp32_tf32": {"hi", "lo"}, "bf16": {"bf16"}}.get(self.mode, {"f32"})
-
-    @classmethod
-    def from_steps(cls, steps: List[Step], mode: str) -> "Program":
-        prog = cls.__new__(cls)
-        prog.mode, prog.items, prog.compress, prog.steps, prog.small, prog.has_row_ladj = mode, [], None, steps, None, False
-        prog.layers, prog.direction, prog._fallback_prog, prog._wflag, prog.force_fallback = [], "forward", None, None, False
-        prog.uses_range_flag = mode == "fp32"
-        return prog
-
 
 class CPlan:
     """Owner of one `usf_plan` (include/usflows_b200.h, "Whole-stack evaluation"): keeps the Program (whose operand planes
@@ -957,27 +957,31 @@ def run_layers(layers, direction: str, x: torch.Tensor, mode: Optional[str] = No
 
 def run_mlp(net, x: torch.Tensor, mode: Optional[str] = None) -> torch.Tensor:
     """Plain evaluation of a DenseNN (no mask, no residual) through the contraction kernels."""
-    with ops.on_device(x):
-        return _run_mlp(net, x, mode)
-
-
-def _run_mlp(net, x, mode):
-    x2, batch_shape = _flatten_rows(x)
-    mode = mode or _default_precision
     lin = list(net.layers)                   # DenseNN, or an _MLPView of a ConditionalDenseNN without its context layer
-    if min(min(l.weight.shape) for l in lin) < TC_MIN_DIM:
-        mode = "fp32_simt"
-    steps = []
-    for j, l in enumerate(lin):
-        last = j == len(lin) - 1
-        N, K = l.weight.shape
-        eng = _engine_for(mode, N, K)
-        w, w_lo = _operand(l.weight.detach(), mode, eng)
-        steps.append(Step("mm", src="x" if j == 0 else "h", dst="x" if last else "h", w=w, w_lo=w_lo, N=N, K=K,
-                          engine=eng, bias=l.bias.detach().contiguous(), relu=not last, final=last))
-    prog = Program.from_steps(steps, mode)
-    with torch.no_grad(), ops.on_device(x2):
-        y = prog.run(x2)
+
+    def build(mode):
+        steps = []
+        for j, l in enumerate(lin):
+            last = j == len(lin) - 1
+            N, K = l.weight.shape
+            eng = _engine_for(mode, N, K)
+            w, w_lo = _operand(l.weight.detach(), mode, eng)
+            steps.append(Step("mm", src="x" if j == 0 else "h", dst="x" if last else "h", w=w, w_lo=w_lo, N=N, K=K,
+                              engine=eng, bias=l.bias.detach().contiguous(), relu=not last, final=last))
+        return steps
+    return _run_net(x, mode, [l.weight for l in lin], build)
+
+
+def _run_net(x: torch.Tensor, mode: Optional[str], weights, build) -> torch.Tensor:
+    """x [..., d] through a network with weight matrices `weights` whose launch steps are `build(mode)`; the whole network
+    runs on the SIMT engine when one of its contractions is narrower than TC_MIN_DIM."""
+    with ops.on_device(x):
+        x2, batch_shape = _flatten_rows(x)
+        mode = mode or _default_precision
+        if min(min(w.shape) for w in weights) < TC_MIN_DIM:
+            mode = "fp32_simt"
+        with torch.no_grad():
+            y = Program([], "forward", mode, build).run(x2)
     return y.reshape(*batch_shape, y.shape[-1]) if x.dim() != 2 else y
 
 
@@ -1124,19 +1128,10 @@ def _convnet_weights(desc: dict) -> list:
 
 def run_conditioner(net, x: torch.Tensor, mode: Optional[str] = None) -> torch.Tensor:
     """Plain evaluation of a `nn.ConvNet` (no mask, no residual) through the same kernels a coupling uses."""
-    with ops.on_device(x):
-        return _run_conditioner(net, x, mode)
-
-
-def _run_conditioner(net, x, mode):
-    x2, batch_shape = _flatten_rows(x)
-    mode = mode or _default_precision
     desc = _convnet_desc(net)
-    if min(min(w.shape) for w in _convnet_weights(desc)) < TC_MIN_DIM:
-        mode = "fp32_simt"
-    steps = convnet_steps(mode, desc, *desc["first"], *desc["last"])
-    steps[-1].final = True
-    prog = Program.from_steps(steps, mode)
-    with torch.no_grad(), ops.on_device(x2):
-        y = prog.run(x2)
-    return y.reshape(*batch_shape, y.shape[-1]) if x.dim() != 2 else y
+
+    def build(mode):
+        steps = convnet_steps(mode, desc, *desc["first"], *desc["last"])
+        steps[-1].final = True
+        return steps
+    return _run_net(x, mode, _convnet_weights(desc), build)

@@ -22,11 +22,8 @@ from typing import List, Optional
 import torch
 
 from . import engine, ops
-from .engine import Prim, _engine_for, _lower_layer, _operand, _workspace
-from .ops import Act, ENGINE_SIMT, ENGINE_TC_3XF16, ENGINE_TC_3XTF32, ENGINE_TC_BF16, ENGINE_TC_TF32
-
-_PLANES = {ENGINE_SIMT: ("f32",), ENGINE_TC_TF32: ("f32",), ENGINE_TC_3XF16: ("h16", "l16"), ENGINE_TC_3XTF32: ("hi", "lo"),
-           ENGINE_TC_BF16: ("bf16",)}
+from .engine import Prim, _engine_for, _operand, _workspace
+from .ops import Act, ENGINE_TC_3XF16, ENGINE_TC_3XTF32
 IMPLICIT_CONV = True                # k x k convolutions as implicit GEMMs (usf_conv2d_rows) where the shape allows it
 PIX_CONV = True                     # ... and the whole ConvNet2D on pixel planes (usf_conv2d_pix) where its widths allow it
 PIX_CH = 32                         # channels of a pixel-plane row
@@ -40,7 +37,7 @@ IMAGE_CHUNK_ROWS_PIX = 1 << 21      # ... when every conditioner runs on pixel p
 
 def _act(dev, name: str, rows: int, width: int, eng: int) -> Act:
     a = Act(rows, width)
-    for pl in _PLANES[eng]:
+    for pl in ops.ENGINE_PLANES[eng]:
         setattr(a, pl, _workspace.planes(dev, name, rows, width, pl))
     return a
 
@@ -242,24 +239,22 @@ class _ConvNet2DPlan:
         return t.f32[:, :self.last.n_true]
 
 
-class ImageProgram:
+class ImageProgram(engine.ProgramCore):
     """Launch program of one direction of a layer stack over image-shaped events, for one mode and weight version."""
 
     small = None
     has_row_ladj = False
+    fp16_weight_modes = PIX_MODES      # the pixel-plane conditioners take fp16 split weights in these modes
 
-    def __init__(self, layers, direction: str, mode: str, in_dims):
-        self.mode = mode or engine.get_precision()
-        self.layers, self.direction = list(layers), direction
+    def __init__(self, layers, direction: str, mode: Optional[str], in_dims):
         self.C, self.H, self.W = (int(v) for v in in_dims)
         self.HW = self.H * self.W
-        self.force_fallback = False
-        self._fallback_prog: Optional["ImageProgram"] = None
-        self._wflag: Optional[torch.Tensor] = None
-        seq = list(layers) if direction == "forward" else list(reversed(list(layers)))
-        prims: List[Prim] = []
-        for layer in seq:
-            _lower_layer(layer, direction, prims)
+        super().__init__(layers, direction, mode)
+
+    def _in_mode(self, mode: str) -> "ImageProgram":
+        return ImageProgram(self.layers, self.direction, mode, (self.C, self.H, self.W))
+
+    def _build(self, prims: List[Prim]) -> None:
         self.entry_scale = self.exit_scale = None            # (vector in NCHW order, mode 1 = multiply / 2 = divide)
         if prims and prims[0].kind in ("mul", "div"):
             self.entry_scale = (prims[0].v.contiguous(), 1 if prims[0].kind == "mul" else 2)
@@ -279,35 +274,23 @@ class ImageProgram:
         for p in prims:
             if p.kind == "aff":                              # 1x1 convolution with the C x C matrix (transforms.py:904-962)
                 dev = p.W.device
-                self.ops.append(("aff", _Gemm(self.mode, p.W, p.c, self._flag(dev))))
+                self.ops.append(("aff", _Gemm(self.mode, p.W, p.c, self._weight_flag(dev))))
             elif p.kind == "coupling" and p.prep.get("net") == "convnet2d":
                 dev = p.prep["mask"].device
                 m = p.prep["mask"].reshape(self.C, self.HW).t().contiguous()          # channels-last order
-                plan = _ConvNet2DPlan(p.prep["module"], self.mode, self._flag(dev), self.H, self.W)
+                plan = _ConvNet2DPlan(p.prep["module"], self.mode, self._weight_flag(dev), self.H, self.W)
                 self.ops.append(("coupling", plan, m.reshape(-1), (1 - m).reshape(-1).contiguous(), p.sign))
             else:
                 raise NotImplementedError(f"usflows_b200: no image-shaped kernel path for a '{p.kind}' step here "
                                           "(ScaleTransform is supported at either end of the stack)")
-        if self._wflag is not None and int(self._wflag.item()) != 0:
-            self.force_fallback = True
         # fp16 split planes are in play (fp32 mode everywhere; tf32 / bf16 modes inside pixel-plane conditioners): chunks carry
         # a device flag and are re-run on the tf32-split program when a value leaves the fp16 range
         self.uses_range_flag = self.mode == "fp32" or (self.mode in PIX_MODES and any(
             op[0] == "coupling" and op[1].pix is not None for op in self.ops))
 
-    def _flag(self, dev):
-        if self.mode not in PIX_MODES:
-            return None
-        if self._wflag is None:
-            self._wflag = torch.zeros(1, dtype=torch.int32, device=dev)
-        return self._wflag
-
-    def _fallback(self) -> "ImageProgram":
-        if self._fallback_prog is None:
-            self._fallback_prog = ImageProgram(self.layers, self.direction, "fp32_tf32", (self.C, self.H, self.W))
-        return self._fallback_prog
-
     def out_width(self, d_in: int) -> int:
+        if d_in != self.C * self.HW:
+            raise RuntimeError("usflows_b200: event shape mismatch")
         return d_in
 
     def plan_able(self) -> bool:                             # the whole-stack C entry covers flat events only
@@ -337,7 +320,7 @@ class ImageProgram:
             if op[0] == "aff":
                 g = op[1]
                 a = Act(rows, C, f32=cur)
-                if _PLANES[g.engine] != ("f32",):            # tensor-core engine: re-encode the fp32 stream into its planes
+                if ops.ENGINE_PLANES[g.engine] != ("f32",):      # tensor-core engine: re-encode the fp32 stream into its planes
                     a = _act(dev, "img_a", rows, C, g.engine)
                     ops.ingest(cur, a, overflow_flag=flag)
                 if direct and idx == len(self.ops) - 1:
@@ -367,37 +350,14 @@ class ImageProgram:
             ops.layout_transpose(cur, n, HW, C, tmp, scale=xs[0], scale_mode=xs[1], scale_on_input=False)
             ops.layout_transpose(tmp, n, C, HW, out)
 
-    def run(self, x: torch.Tensor, *, out: Optional[torch.Tensor] = None, sink=None, chunk_rows: Optional[int] = None,
-            ladj_rows: Optional[torch.Tensor] = None, dq: Optional[ops.Dequant] = None) -> Optional[torch.Tensor]:
-        """x [N, C*H*W] -> [N, C*H*W] (NCHW order), or per chunk `sink(channels_last_chunk [n, H*W*C], r0, r1)`; with `dq`, x
-        is uint8 (see _run_chunk).  `ladj_rows` is never written: no image step has per-row log-determinants."""
-        ops.require_cuda(x, "input", torch.float32 if dq is None else torch.uint8)
-        x = x.contiguous()
-        N, d = x.shape
-        if d != self.C * self.HW:
-            raise RuntimeError("usflows_b200: event shape mismatch")
-        if sink is None and out is None:
-            out = torch.empty(N, d, dtype=torch.float32, device=x.device)
-        if N == 0:
-            return out
-        if self.force_fallback:
-            return self._fallback().run(x, out=out, sink=sink, chunk_rows=chunk_rows, dq=dq)
+    def _chunk_bounds(self, rows: int, chunk_rows: Optional[int]):
+        """Whole images, IMAGE_CHUNK_ROWS* channels-last rows per chunk."""
         all_pix = all(op[0] != "coupling" or op[1].pix is not None for op in self.ops)
         per = max(1, (chunk_rows or (IMAGE_CHUNK_ROWS_PIX if all_pix else IMAGE_CHUNK_ROWS)) // self.HW)
+        return [(r0, min(rows, r0 + per)) for r0 in range(0, rows, per)]
 
-        def chunk(prog, r0, r1, flag):
-            cdq = None if dq is None else dq.shifted(r0)
-            if sink is not None:
-                fin = self.final_buffer(x.device, "final", r1 - r0, d)
-                prog._run_chunk(x[r0:r1], fin, flag, cdq)
-                sink(fin, r0, r1)
-            else:
-                prog._run_chunk(x[r0:r1], out[r0:r1], flag, cdq, nchw_out=True)
-
-        engine.run_chunks([(r0, min(N, r0 + per)) for r0 in range(0, N, per)], x.device, self.uses_range_flag,
-                          lambda i, r0, r1, flag: chunk(self, r0, r1, flag),
-                          lambda i, r0, r1: chunk(self._fallback(), r0, r1, None))
-        return out
+    def _chunk(self, x, out, flag, dq, ladj_rows, to_caller: bool) -> None:
+        self._run_chunk(x, out, flag, dq, nchw_out=to_caller)      # the caller's output is NCHW, a sink's channels-last
 
 
 def channels_last_index(C: int, HW: int, device) -> torch.Tensor:

@@ -91,6 +91,11 @@ class Act:
         raise RuntimeError("activation has no fp32-accurate plane to use as a residual")
 
 
+# the planes of an Act each contraction engine's operands are prepared in (what `linear` reads as A)
+ENGINE_PLANES = {ENGINE_SIMT: ("f32",), ENGINE_TC_TF32: ("f32",), ENGINE_TC_3XF16: ("h16", "l16"),
+                 ENGINE_TC_3XTF32: ("hi", "lo"), ENGINE_TC_BF16: ("bf16",)}
+
+
 def linear(engine: int, a: Act, w, w_lo, N: int, K: int, *, bias=None, relu=False, resid: Optional[Act] = None,
            resid_sign: float = 1.0, colscale=None, postsub=None, out: Act, trans_w: bool = False,
            overflow_flag: Optional[torch.Tensor] = None) -> None:
