@@ -108,13 +108,10 @@ def base_logprob(z, loc, scale, kind, add_const, out):
 
 
 def base_sample(out, loc, scale, kind, seed, offset):
-    g = torch.Generator().manual_seed((seed + offset) % (2 ** 63))
-    if kind == real_ops.BASE_LAPLACE:
-        u = torch.rand(out.rows, out.width, generator=g) * 2 - 1
-        e = -u.sign() * torch.log1p(-u.abs())
-    else:
-        e = torch.randn(out.rows, out.width, generator=g)
-    _store(out, loc + scale * e)
+    """The device's draws: the fp64 restatement of base_sample_kernel, rounded to fp32."""
+    from philox_ref import ref_base_sample
+    v = ref_base_sample(out.rows, out.width, loc.double().numpy(), scale.double().numpy(), kind, seed, offset)
+    _store(out, torch.from_numpy(v).to(torch.float32))
 
 
 def flow_small(x, prog_i32, blob, n_ops, D, H, out):

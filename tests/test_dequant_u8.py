@@ -12,21 +12,7 @@ import torch
 
 import fake_backend
 from helpers import build_flow, load_case, rel_err
-
-MASK = np.uint64(0xFFFFFFFF)
-
-
-def np_philox4x32_10(ctr, key):
-    """Philox4x32-10 on uint64 arrays holding 32-bit words: ctr = 4 arrays, key = 2 arrays (or scalars)."""
-    c0, c1, c2, c3 = (np.asarray(c, dtype=np.uint64) & MASK for c in ctr)
-    k0, k1 = (np.asarray(k, dtype=np.uint64) & MASK for k in key)
-    for _ in range(10):
-        p0 = np.uint64(0xD2511F53) * c0
-        p1 = np.uint64(0xCD9E8D57) * c2
-        c0, c1, c2, c3 = (p1 >> np.uint64(32)) ^ c1 ^ k0, p1 & MASK, (p0 >> np.uint64(32)) ^ c3 ^ k1, p0 & MASK
-        k0 = (k0 + np.uint64(0x9E3779B9)) & MASK
-        k1 = (k1 + np.uint64(0xBB67AE85)) & MASK
-    return c0, c1, c2, c3
+from philox_ref import MASK, np_philox4x32_10
 
 
 def np_dequant(x, mode, seed, row0=0):
