@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define USF_ABI_VERSION 8
+#define USF_ABI_VERSION 9   /* ABI 9: the test hooks that chose the single-CTA GEMM and the 3-D operand loads are gone */
 
 #define USF_OK 0
 #define USF_ERR_INVALID (-1)     /* bad argument (shape, alignment, null pointer) */
@@ -143,14 +143,9 @@ int usf_set_accum_chunk(int k_slabs);
 int usf_set_accum_lead(int chains);
 /* test hook: force the tcgen05 tile width BLOCK_N (0 = automatic) */
 int usf_debug_set_block_n(int block_n);
-/* test hook: 2 = CTA-pair (cta_group::2) tcgen05 kernel (default), 1 = single-CTA tcgen05 kernel */
-int usf_debug_set_impl(int impl);
 /* test hook: 1 (default) = the kernels of an evaluation are chained with programmatic dependent launch, 0 = plain
  * stream order */
 int usf_debug_set_pdl(int on);
-/* test hook: 1 = the hi / lo operand planes of a tile travel in ONE 3-D TMA operation (planes as the third tensor
- * dimension, plane stride = distance of the two pointers), 0 (default) = one 2-D operation per plane; same bits, same speed */
-int usf_debug_set_planes3d(int on);
 /* profiling hook for the CTA-pair tcgen05 kernel: `device_buf` (512 x 8 uint64, or NULL to switch off) receives
  * clock64() stamps of the first 512 accumulation chains of cluster 0 (0 = accumulator free seen by the MMA issuer,
  * 1 = operands landed, 2 = chain issued, 3 = accumulator full seen by epilogue warp 4, 4 = drained, 5 = tile stored);

@@ -24,7 +24,7 @@ def test_header_symbols_are_exported_and_bound():
     for name in declared:
         assert hasattr(lib, name), f"{name} declared in the header but not exported"
         assert name in _lib.SIGNATURES, f"{name} has no ctypes signature in _lib.py"
-    assert lib.usf_abi_version() == 8
+    assert lib.usf_abi_version() == 9
 
 
 def test_planes_struct_layout_matches_header():

@@ -31,7 +31,8 @@ ENGINES = [("simt", 0, "f32", 3e-6), ("3xtf32", 1, "split", 3e-6), ("tf32", 2, "
 
 @pytest.mark.parametrize("eng_name,eng,fmt,tol", ENGINES)
 @pytest.mark.parametrize("M,N,K", [(1, 40, 40), (128, 128, 32), (300, 784, 1024), (1000, 1024, 784), (257, 3072, 520),
-                                   (513, 100, 50), (64, 33, 47)])
+                                   (513, 100, 50), (64, 33, 47), (300, 784, 784), (1000, 1024, 392), (515, 392, 1024),
+                                   (257, 208, 72), (64, 48, 40)])
 def test_linear_all_engines_full_epilogue(eng_name, eng, fmt, tol, M, N, K):
     from usflows_b200 import ops
     from usflows_b200.ops import Act
@@ -212,7 +213,8 @@ def _f16_planes(t):
 
 
 @pytest.mark.parametrize("M,N,K", [(1, 40, 40), (300, 784, 1024), (1000, 392, 784), (777, 1024, 392), (257, 3072, 520),
-                                   (513, 100, 56), (2048, 224, 72), (640, 432, 1000)])
+                                   (513, 100, 56), (2048, 224, 72), (640, 432, 1000), (300, 784, 784), (1000, 1024, 392),
+                                   (515, 392, 1024), (257, 208, 72), (64, 48, 40)])
 def test_fp16_split_engine_full_epilogue(M, N, K):
     """3 x fp16 tensor-core products with the fp16-split residual and output planes (the default fp32 mode)."""
     from usflows_b200 import ops
@@ -505,44 +507,6 @@ def test_tma_store_path_for_bf16_and_fp32_planes(eng_name, eng, fmt, planes, M, 
         t = getattr(p, name)
         if t is not None and ops.pad4(N) != N and "f32" not in planes:
             assert float(t._base[:, N:].abs().float().max()) == 0.0
-
-
-@pytest.mark.parametrize("eng_name,eng,fmt", [("3xtf32", 1, "split"), ("3xf16", 4, "f16")])
-@pytest.mark.parametrize("M,N,K", [(300, 784, 784), (1000, 1024, 392), (515, 392, 1024), (257, 208, 72), (64, 48, 40)])
-def test_both_operand_planes_in_one_tma_operation(eng_name, eng, fmt, M, N, K):
-    """Split engines: hi and lo planes of a tile fetched by ONE 3-D TMA operation (planes = third tensor dimension, possible
-    when lo - hi is a positive multiple of 16 bytes; a measured-neutral option) == one 2-D operation per plane (default); also
-    when the planes do not allow the 3-D form."""
-    from usflows_b200 import _lib, ops
-    from usflows_b200.ops import Act
-    g = torch.Generator().manual_seed(M + N + K)
-    a = torch.randn(M, K, generator=g)
-    w = torch.randn(N, K, generator=g) / K ** 0.5
-    bias = torch.randn(N, generator=g).cuda()
-    act, a_used = _f16_planes(a) if fmt == "f16" else _planes(a, fmt)
-    wact, w_used = _f16_planes(w) if fmt == "f16" else _planes(w, fmt)
-    hi, lo = (act.h16, act.l16) if fmt == "f16" else (act.hi, act.lo)
-    w_hi, w_lo = (wact.h16, wact.l16) if fmt == "f16" else (wact.hi, wact.lo)
-    assert lo.data_ptr() > hi.data_ptr()
-    # the same activation with the planes the other way round in memory: the 3-D form is impossible, the kernel must notice
-    rev = torch.zeros(2, M, ops.pad4(K), dtype=hi.dtype, device="cuda")
-    rev[1, :, :K].copy_(hi)
-    rev[0, :, :K].copy_(lo)
-    act_rev = Act(M, K, h16=rev[1, :, :K], l16=rev[0, :, :K]) if fmt == "f16" else Act(M, K, hi=rev[1, :, :K], lo=rev[0, :, :K])
-    lib = _lib.load()
-    outs = []
-    for on, A in ((1, act), (0, act), (1, act_rev)):
-        out = torch.zeros(M, ops.pad4(N, 4), device="cuda")[:, :N]
-        lib.usf_debug_set_planes3d(on)
-        try:
-            ops.linear(eng, A, w_hi, w_lo, N, K, bias=bias, relu=True, out=Act(M, N, f32=out))
-            torch.cuda.synchronize()
-        finally:
-            lib.usf_debug_set_planes3d(0)
-        outs.append(out)
-    assert torch.equal(outs[0], outs[1]) and torch.equal(outs[0], outs[2])
-    ref = torch.relu(a_used.double() @ w_used.double().T + bias.double().cpu())
-    assert rel_err(outs[0], ref) <= 3e-6
 
 
 @pytest.mark.parametrize("M,N,K", [(1, 1, 1), (5, 3, 7), (64, 64, 16), (130, 70, 33), (784, 784, 784), (100, 784, 50),

@@ -1,7 +1,7 @@
 """GEMM micro-benchmark / checker for the tcgen05 contraction kernels (run on the B200 box).
 
     python tools/gemm_bench.py [--engines 3xtf32,tf32,bf16] [--shapes 16384x784x784,...] [--chunk 2]
-                               [--bn 0] [--check] [--iters 20] [--planes split|f32] [--impl 1|2]
+                               [--bn 0] [--check] [--iters 20]
 
 Prints one JSON line per (engine, shape): time, MMA-level TFLOP/s (counting every tensor-core pass), and the
 error against an fp64 product when --check is given.

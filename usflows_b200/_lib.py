@@ -181,9 +181,7 @@ SIGNATURES = {
     "usf_debug_set_block_n": (C.c_int, [C.c_int]),
     "usf_set_accum_chunk": (C.c_int, [C.c_int]),
     "usf_set_accum_lead": (C.c_int, [C.c_int]),
-    "usf_debug_set_impl": (C.c_int, [C.c_int]),
     "usf_debug_set_pdl": (C.c_int, [C.c_int]),
-    "usf_debug_set_planes3d": (C.c_int, [C.c_int]),
     "usf_debug_gemm_timeline": (C.c_int, [_P, C.c_int]),
 }
 
@@ -210,7 +208,7 @@ def load():
         fn = getattr(lib, name)  # AttributeError if the ABI and this table disagree
         fn.restype = res
         fn.argtypes = args
-    if lib.usf_abi_version() != 8:
+    if lib.usf_abi_version() != 9:
         raise RuntimeError("usflows_b200: ABI version mismatch between _lib.py and the shared library")
     _lib = lib
     return lib

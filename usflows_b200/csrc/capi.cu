@@ -28,13 +28,11 @@ int g_force_block_n = 0;
 int g_chunk_slabs = 2;
 int g_conv_chunk_slabs = 3;
 int g_lead_chains = 2;
-int g_tc_impl = 2;
 unsigned long long* g_dbg_buf = nullptr;
 int g_dbg_flags = 0;
 int g_no_fast_store = 0;
 int g_use_pdl = 1;
 int g_no_async_store = 0;
-int g_planes3d = 0;
 
 int num_sms() {
   static int cached[64] = {0};
@@ -159,22 +157,11 @@ int usf_debug_set_block_n(int bn) {  // test hook: force the tcgen05 tile width 
   return USF_OK;
 }
 
-int usf_debug_set_impl(int impl) {  // test hook: 2 = CTA-pair tcgen05 kernel (default), 1 = single-CTA kernel
-  USF_REQUIRE(impl == 1 || impl == 2, "impl must be 1 or 2");
-  g_tc_impl = impl;
-  return USF_OK;
-}
-
 int usf_debug_gemm_timeline(unsigned long long* device_buf, int flags) {
   g_dbg_buf = device_buf;
   g_dbg_flags = flags & ~(4 | 32);
   g_no_fast_store = (flags & 4) ? 1 : 0;
   g_no_async_store = (flags & 32) ? 1 : 0;
-  return USF_OK;
-}
-
-int usf_debug_set_planes3d(int on) {  // test hook: hi / lo operand planes in one 3-D TMA operation (default on)
-  g_planes3d = on ? 1 : 0;
   return USF_OK;
 }
 

@@ -10,7 +10,8 @@
 // core reads -- while the whole weight (k*k*C x N in two tf32 planes, 74 KB at C = N = 32, k = 3) stays resident in shared
 // memory for the lifetime of the persistent CTA (loaded once by TMA).  fp32-accurate 3-term tf32 split
 // (A_hi.W_hi + A_lo.W_hi + A_hi.W_lo), accumulation chains closed every `chunk_slabs` K-slabs and summed in fp32 registers
-// by the epilogue warps, exactly as gemm_tc.cuh's 3xTF32 engine; the fused epilogue (bias, ReLU, output planes) is shared.
+// by the epilogue warps, exactly as the 3xTF32 engine of the contraction (gemm_tc2.cuh); the fused epilogue (bias, ReLU,
+// output planes) is shared.
 //
 // Warp roles (N <= 32: 768 threads): warp 0 weight loader (TMA, once), warp 1 MMA issuer + TMEM owner, warps 4-7
 // epilogue, warps 8-23 gather (4 threads per tile row).  3 A stages of 32 KB (hi + lo) + the resident weight.

@@ -1,23 +1,19 @@
-// tcgen05 / TMEM / TMA contraction for sm_100a:  out = epilogue( sum_terms A_t[M,K] . W_t[N,K]^T )
+// Shared tcgen05 / TMEM / TMA primitives for sm_100a, and the single-CTA pieces of the implicit-GEMM convolution
+// (conv_tc.cuh).  The contraction itself is the CTA-pair kernel of gemm_tc2.cuh.
 //
-//   * operands K-major in shared memory, 128-byte swizzle, one 128 B K-slab per pipeline stage
-//     (32 tf32/fp32 elements or 64 bf16 elements), filled by TMA (cp.async.bulk.tensor.2d) with
-//     hardware zero fill for the M / N / K tails
-//   * one elected thread issues tcgen05.mma (cta_group::1, M=128, N=BLOCK_N, K=32 B per instruction),
-//     fp32 accumulators live in TMEM, double buffered so the epilogue of tile i overlaps the MMAs of
-//     tile i+1
-//   * NTERMS = 3 is the fp32-accurate mode: A = A_hi + A_lo, W = W_hi + W_lo with every plane exactly
-//     representable in tf32; D = A_hi.W_hi + A_lo.W_hi + A_hi.W_lo accumulated in fp32 (error ~2^-21)
-//   * the tensor core adds into its fp32 accumulator with truncation, so a long K chain carries a
-//     systematic toward-zero bias (~0.2 ulp per MMA step, measured: 5e-6 relative at K=1024 x 3 terms,
-//     coherent across layers).  The fp32 mode therefore closes the TMEM accumulator every
-//     `chunk_slabs` K-slabs and the epilogue warps add the partial tile into fp32 registers with
-//     round-to-nearest (two TMEM accumulators ping-pong between the MMA issuer and the epilogue)
-//   * persistent CTAs (grid = min(tiles, SMs)), warp-specialised: warp 0 TMA producer, warp 1 MMA
-//     issuer + TMEM owner, warps 4..11 epilogue (tcgen05.ld 32x32b -> registers -> fused epilogue ->
-//     global stores; warp w owns TMEM lane quarter w % 4 and one half of the tile's columns); the
-//     epilogue warpgroups take the register file with setmaxnreg (232 regs: up to 128 fp32 partial sums
-//     per thread stay in registers)
+//   * mbarrier, elect, fence, TMA load, tcgen05.mma / commit and tcgen05.ld helpers used by every tcgen05 kernel
+//     (gemm_tc2.cuh, conv_tc.cuh, conv_pix.cuh)
+//   * operands K-major in shared memory, 128-byte swizzle, one 128 B K-slab per pipeline stage (32 tf32/fp32 elements
+//     or 64 bf16/fp16 elements): make_operand_map builds the TMA map (hardware zero fill for the M / N / K tails),
+//     make_smem_desc the matching shared-memory descriptor
+//   * warp roles of the warp-specialised kernels: warp 0 TMA producer, warp 1 MMA issuer + TMEM owner, warps 4..11
+//     epilogue (warp w owns TMEM lane quarter w % 4 and one half of the tile's columns); the epilogue warpgroups take
+//     the register file with setmaxnreg
+//   * tc::Config + epilogue_loop: the single-CTA (cta_group::1, M = 128) tile and its epilogue warps.  The tensor core
+//     adds into its fp32 accumulator with truncation, so a long K chain carries a systematic toward-zero bias (~0.2 ulp
+//     per MMA step, measured: 5e-6 relative at K=1024 x 3 terms, coherent across layers); the fp32-accurate mode
+//     therefore closes the TMEM accumulator every `chunk_slabs` K-slabs and the epilogue warps add the partial tile into
+//     fp32 registers with round-to-nearest (two TMEM accumulators ping-pong between the MMA issuer and the epilogue)
 #pragma once
 #include "common.cuh"
 
@@ -175,24 +171,14 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
+// single-CTA (cta_group::1, M = 128) tile: TMEM accumulator layout, epilogue column halves, instruction descriptor
 template <int BLOCK_N, int NTERMS, bool BF16>
 struct Config {
   static_assert(BLOCK_N % 16 == 0 && BLOCK_N >= 16 && BLOCK_N <= 256, "UMMA N for M=128");
   static_assert(NTERMS == 1 || NTERMS == 3, "1 = single pass, 3 = tf32 split");
   static constexpr int kBlockN = BLOCK_N;
-  static constexpr int NPLANES = NTERMS == 3 ? 2 : 1;
-  static constexpr int A_TILE = BLOCK_M * SLAB_BYTES;
-  static constexpr int B_TILE = BLOCK_N * SLAB_BYTES;
-  static constexpr int B_TILE_PAD = (B_TILE + 1023) / 1024 * 1024;  // keep every tile 1024 B aligned
-  static constexpr int STAGE_BYTES = NPLANES * (A_TILE + B_TILE_PAD);
-  static constexpr int TX_BYTES = NPLANES * (A_TILE + B_TILE);
-  static constexpr int STAGES_RAW = (220 * 1024) / STAGE_BYTES;
-  static constexpr int STAGES = STAGES_RAW > 8 ? 8 : STAGES_RAW;
-  static_assert(STAGES >= 2, "need at least a double-buffered pipeline");
   static constexpr int ACC_STRIDE = BLOCK_N <= 32 ? 32 : BLOCK_N <= 64 ? 64 : BLOCK_N <= 128 ? 128 : 256;
   static constexpr int TMEM_COLS = 2 * ACC_STRIDE;  // power of two >= 64
-  static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*align slack*/ + 256 /*barriers*/;
-  static constexpr int ELEMS_PER_SLAB = SLAB_BYTES / (BF16 ? 2 : 4);
   static constexpr int HALF0 = ((BLOCK_N / 16 + 1) / 2) * 16;  // columns owned by epilogue warps 4..7
   static constexpr int HALF1 = BLOCK_N - HALF0;                // ... and by warps 8..11 (may be 0)
   // instruction descriptor: D=f32, A/B = tf32 (2) or bf16 (1), both K-major, N>>3, M>>4
@@ -257,136 +243,6 @@ __device__ __forceinline__ void epilogue_loop(int col0, int quarter, int lane, u
   }
 }
 
-template <int BLOCK_N, int NTERMS, bool BF16>
-__global__ void __launch_bounds__(NUM_THREADS, 1)
-gemm_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_a_lo,
-               const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_w_lo,
-               long long M, int N, int K, int chunk_slabs, Epilogue ep) {
-  using C = Config<BLOCK_N, NTERMS, BF16>;
-  extern __shared__ uint8_t smem_raw[];
-  const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
-  const uint32_t bar_base = smem_base + C::STAGES * C::STAGE_BYTES;
-  // barrier block: full[STAGES], empty[STAGES], tmem_full[2], tmem_empty[2], tmem base pointer
-  auto full_bar = [&](int s) { return bar_base + 8u * s; };
-  auto empty_bar = [&](int s) { return bar_base + 8u * (C::STAGES + s); };
-  auto tfull_bar = [&](int s) { return bar_base + 8u * (2 * C::STAGES + s); };
-  auto tempty_bar = [&](int s) { return bar_base + 8u * (2 * C::STAGES + 2 + s); };
-  const uint32_t tmem_slot = bar_base + 8u * (2 * C::STAGES + 4);
-  uint32_t* tmem_slot_ptr = reinterpret_cast<uint32_t*>(smem_raw + (tmem_slot - smem_u32(smem_raw)));
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int n_blocks = (N + BLOCK_N - 1) / BLOCK_N;
-  const long long m_blocks = (M + BLOCK_M - 1) / BLOCK_M;
-  const long long n_tiles = m_blocks * n_blocks;
-  const int k_slabs = (K + C::ELEMS_PER_SLAB - 1) / C::ELEMS_PER_SLAB;
-  if (chunk_slabs <= 0 || chunk_slabs > k_slabs) chunk_slabs = k_slabs;  // slabs per TMEM accumulation chain
-
-  if (warp == 0 && lane == 0) {
-    prefetch_tmap(&tm_a);
-    prefetch_tmap(&tm_w);
-    if (NTERMS == 3) { prefetch_tmap(&tm_a_lo); prefetch_tmap(&tm_w_lo); }
-  }
-  if (warp == 1) {
-    if (lane == 0) {
-      for (int s = 0; s < C::STAGES; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
-      for (int s = 0; s < 2; ++s) { mbar_init(tfull_bar(s), 1); mbar_init(tempty_bar(s), NUM_EPI_WARPS); }
-      fence_barrier_init();
-    }
-    __syncwarp();
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "n"(C::TMEM_COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tcgen05_fence_before();
-  __syncthreads();
-  tcgen05_fence_after();
-  const uint32_t tmem_base = *tmem_slot_ptr;
-
-  if (warp < FIRST_EPI_WARP) {
-  asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(REGS_NON_EPI));
-  if (warp == 0) {
-    // ===================== TMA producer =====================
-    if (lane == 0) {
-      int stage = 0;
-      uint32_t phase = 0;
-      for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-        const int m_idx = (int)(tile / n_blocks) * BLOCK_M;
-        const int n_idx = (int)(tile % n_blocks) * BLOCK_N;
-        for (int ks = 0; ks < k_slabs; ++ks) {
-          mbar_wait(empty_bar(stage), phase ^ 1);
-          const uint32_t sa = smem_base + stage * C::STAGE_BYTES;
-          const uint32_t sb = sa + C::NPLANES * C::A_TILE;
-          const int k_idx = ks * C::ELEMS_PER_SLAB;
-          mbar_expect_tx(full_bar(stage), C::TX_BYTES);
-          tma_load_2d(sa, &tm_a, full_bar(stage), k_idx, m_idx);
-          tma_load_2d(sb, &tm_w, full_bar(stage), k_idx, n_idx);
-          if (NTERMS == 3) {
-            tma_load_2d(sa + C::A_TILE, &tm_a_lo, full_bar(stage), k_idx, m_idx);
-            tma_load_2d(sb + C::B_TILE_PAD, &tm_w_lo, full_bar(stage), k_idx, n_idx);
-          }
-          if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ===================== MMA issuer =====================
-    int stage = 0;
-    uint32_t phase = 0;
-    int acc = 0;
-    uint32_t acc_phase = 0;
-    for (long long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-      for (int ks0 = 0; ks0 < k_slabs; ks0 += chunk_slabs) {
-        const int ks1 = ks0 + chunk_slabs < k_slabs ? ks0 + chunk_slabs : k_slabs;
-        mbar_wait(tempty_bar(acc), acc_phase ^ 1);  // epilogue has drained this accumulator
-        tcgen05_fence_after();
-        const uint32_t tmem_d = tmem_base + acc * C::ACC_STRIDE;
-        for (int ks = ks0; ks < ks1; ++ks) {
-          mbar_wait(full_bar(stage), phase);
-          tcgen05_fence_after();
-          if (lane == 0) {
-            const uint32_t sa = smem_base + stage * C::STAGE_BYTES;
-            const uint32_t sb = sa + C::NPLANES * C::A_TILE;
-            const uint64_t da_hi = make_smem_desc(sa), db_hi = make_smem_desc(sb);
-            if (NTERMS == 3) {  // small terms first: they meet the accumulator while it is smallest
-              const uint64_t da_lo = make_smem_desc(sa + C::A_TILE), db_lo = make_smem_desc(sb + C::B_TILE_PAD);
-#pragma unroll
-              for (int k = 0; k < SLAB_BYTES / UMMA_K_BYTES; ++k) {
-                const uint64_t koff = (uint64_t)((k * UMMA_K_BYTES) >> 4);
-                umma<BF16>(da_lo + koff, db_hi + koff, tmem_d, C::IDESC, (ks > ks0 || k > 0) ? 1u : 0u);
-                umma<BF16>(da_hi + koff, db_lo + koff, tmem_d, C::IDESC, 1u);
-              }
-            }
-#pragma unroll
-            for (int k = 0; k < SLAB_BYTES / UMMA_K_BYTES; ++k) {
-              const uint64_t koff = (uint64_t)((k * UMMA_K_BYTES) >> 4);
-              umma<BF16>(da_hi + koff, db_hi + koff, tmem_d, C::IDESC, (NTERMS == 3 || ks > ks0 || k > 0) ? 1u : 0u);
-            }
-            umma_commit(empty_bar(stage));                  // smem slot free once these MMAs retire
-            if (ks == ks1 - 1) umma_commit(tfull_bar(acc));  // this accumulation chain is complete
-          }
-          __syncwarp();
-          if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
-        }
-        if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-      }
-    }
-  }
-  } else {
-    // ===================== epilogue warps (TMEM lane quarter = warp % 4; column half = (warp-4)/4) ======
-    asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(REGS_EPI));
-    if (warp < FIRST_EPI_WARP + 4) epilogue_loop<C, C::HALF0>(0, warp & 3, lane, tmem_base, tfull_bar(0), tempty_bar(0), n_tiles, n_blocks,
-                                             k_slabs, chunk_slabs, M, N, ep);
-    else          epilogue_loop<C, C::HALF1>(C::HALF0, warp & 3, lane, tmem_base, tfull_bar(0), tempty_bar(0), n_tiles,
-                                             n_blocks, k_slabs, chunk_slabs, M, N, ep);
-  }
-
-  tcgen05_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    tcgen05_fence_after();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(C::TMEM_COLS) : "memory");
-  }
-}
-
 }  // namespace tc
 
 // host side ---------------------------------------------------------------------------------------
@@ -399,17 +255,17 @@ PFN_encodeTiled get_encode_tiled();
 // 2-D row-major [rows, cols] operand, box = 128 B of K x box_rows rows, 128B swizzle, zero OOB fill
 // dtype: 0 = fp32 / tf32, 1 = bf16, 2 = fp16
 inline int make_operand_map(CUtensorMap* map, const void* ptr, long long rows, long long cols, long long ld,
-                            int box_rows, int dtype, int slab_bytes = tc::SLAB_BYTES) {
+                            int box_rows, int dtype) {
   PFN_encodeTiled enc = get_encode_tiled();
   if (!enc) return fail(USF_ERR_CUDA, "cuTensorMapEncodeTiled entry point not available%s%s");
   const int esz = dtype ? 2 : 4;
   cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
   cuuint64_t strides[1] = {(cuuint64_t)ld * esz};
-  cuuint32_t box[2] = {(cuuint32_t)(slab_bytes / esz), (cuuint32_t)box_rows};
+  cuuint32_t box[2] = {(cuuint32_t)(tc::SLAB_BYTES / esz), (cuuint32_t)box_rows};
   cuuint32_t estr[2] = {1, 1};
   CUresult r = enc(map, dtype == 1 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : dtype == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2,
                    const_cast<void*>(ptr), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   slab_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                   CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
     snprintf(g_err, sizeof(g_err), "cuTensorMapEncodeTiled failed with CUresult %d (rows=%lld cols=%lld ld=%lld)",
@@ -418,67 +274,5 @@ inline int make_operand_map(CUtensorMap* map, const void* ptr, long long rows, l
   }
   return USF_OK;
 }
-
-template <int BLOCK_N, int NTERMS, bool BF16>
-int launch_gemm_tc_cfg(const usf_linear_args* a, const Epilogue& ep, cudaStream_t st) {
-  using C = tc::Config<BLOCK_N, NTERMS, BF16>;
-  static bool attr_set_dev[MAX_DEVICES] = {false};
-  bool& attr_set = attr_set_dev[current_device_slot()];
-  auto kern = tc::gemm_tc_kernel<BLOCK_N, NTERMS, BF16>;
-  if (!attr_set) {
-    USF_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
-    attr_set = true;
-  }
-  CUtensorMap ma, mal, mw, mwl;
-  int rc;
-  if ((rc = make_operand_map(&ma, a->a, a->M, a->K, a->lda, tc::BLOCK_M, BF16 ? 1 : 0))) return rc;
-  if ((rc = make_operand_map(&mw, a->w, a->N, a->K, a->ldw, BLOCK_N, BF16 ? 1 : 0))) return rc;
-  if (NTERMS == 3) {
-    if ((rc = make_operand_map(&mal, a->a_lo, a->M, a->K, a->lda, tc::BLOCK_M, BF16 ? 1 : 0))) return rc;
-    if ((rc = make_operand_map(&mwl, a->w_lo, a->N, a->K, a->ldw, BLOCK_N, BF16 ? 1 : 0))) return rc;
-  } else {
-    mal = ma;
-    mwl = mw;
-  }
-  const long long tiles = ((a->M + tc::BLOCK_M - 1) / tc::BLOCK_M) * ((a->N + BLOCK_N - 1) / BLOCK_N);
-  const int grid = (int)(tiles < num_sms() ? tiles : num_sms());
-  kern<<<grid, tc::NUM_THREADS, C::SMEM_BYTES, st>>>(ma, mal, mw, mwl, a->M, a->N, a->K,
-                                                       NTERMS == 3 ? g_chunk_slabs : 0, ep);
-  USF_CUDA_OK(cudaGetLastError());
-  return USF_OK;
-}
-
-// BLOCK_N choice: the widest tile that wastes the least of N (wide tiles halve the shared-memory
-// operand traffic per MMA cycle: 64 + 8192/N bytes per cycle for tf32)
-inline int pick_block_n(int N) {
-  static const int cands[] = {256, 208, 128, 64, 32};
-  int best = 256;
-  double best_cost = 1e30;
-  for (int bn : cands) {
-    int nb = (N + bn - 1) / bn;
-    double waste = (double)nb * bn / N;               // padded / useful MMA work
-    double smem = (64.0 + 8192.0 / bn) / 128.0;       // fraction of smem bandwidth needed (tf32, 1 CTA)
-    double cost = waste * (smem > 1.0 ? smem : 1.0) * (1.0 + 0.02 * nb);
-    if (cost < best_cost) { best_cost = cost; best = bn; }
-  }
-  return best;
-}
-
-template <int NTERMS, bool BF16>
-int launch_gemm_tc_terms(const usf_linear_args* a, const Epilogue& ep, cudaStream_t st, int bn) {
-  switch (bn) {
-    case 256: return launch_gemm_tc_cfg<256, NTERMS, BF16>(a, ep, st);
-    case 208: return launch_gemm_tc_cfg<208, NTERMS, BF16>(a, ep, st);
-    case 128: return launch_gemm_tc_cfg<128, NTERMS, BF16>(a, ep, st);
-    case 64: return launch_gemm_tc_cfg<64, NTERMS, BF16>(a, ep, st);
-    case 32: return launch_gemm_tc_cfg<32, NTERMS, BF16>(a, ep, st);
-  }
-  return fail(USF_ERR_INVALID, "unsupported BLOCK_N (built: 256, 208, 128, 64, 32)%s%s");
-}
-
-// one translation unit per engine (gemm_tc_inst_*.cu) so the variants compile in parallel
-int launch_gemm_tc_3xtf32(const usf_linear_args* a, const Epilogue& ep, cudaStream_t st, int bn);
-int launch_gemm_tc_tf32(const usf_linear_args* a, const Epilogue& ep, cudaStream_t st, int bn);
-int launch_gemm_tc_bf16(const usf_linear_args* a, const Epilogue& ep, cudaStream_t st, int bn);
 
 }  // namespace usf

@@ -2,7 +2,7 @@
 //
 // Two CTAs of a cluster (one TPC) share every MMA: UMMA M = 256 (128 rows of A per CTA), N = BLOCK_N with
 // each CTA staging only HALF of the W tile, so the shared-memory fill traffic per MMA cycle drops by a third
-// against the single-CTA kernel (gemm_tc.cuh) -- the single-CTA kernel is bound by the L2 -> SM fill rate
+// against a single-CTA (M = 128) tile -- a single-CTA contraction is bound by the L2 -> SM fill rate
 // (~40 B/cycle/SM measured), not by the tensor pipe.
 //
 //   * per CTA and K-slab (128 B of K): A tile 128 rows + W half tile BLOCK_N/2 rows, per operand plane,
@@ -12,7 +12,8 @@
 //     "accumulator ready" arrivals to both CTAs; each CTA's epilogue drains its own 128 TMEM lanes and
 //     releases the accumulator on the leader's barrier (remote mbarrier.arrive)
 //   * fp32 mode (NTERMS = 3): the accumulation chain is closed every `chunk_slabs` K-slabs and promoted into
-//     fp32 registers with round-to-nearest (see gemm_tc.cuh); two TMEM accumulators ping-pong
+//     fp32 registers with round-to-nearest (the tensor core accumulates with truncation, see gemm_tc.cuh); two TMEM
+//     accumulators ping-pong
 //   * epilogue: registers -> per-warp padded smem patch (16 columns at a time) -> coalesced 64 B row segments
 //     with the fused bias / ReLU / residual / column scale / post-subtract / hi-lo or bf16 re-encoding
 #pragma once
@@ -62,14 +63,6 @@ __device__ __forceinline__ void tma_load_2d_pair(uint32_t dst, const CUtensorMap
   asm volatile(
       "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
       ::"r"(dst), "l"(map), "r"(leader_bar), "r"(c0), "r"(c1)
-      : "memory");
-}
-// both operand planes (hi, lo) of a tile in ONE TMA operation: the planes are the third dimension of the tensor map (any two
-// plane pointers are "a tensor with two planes" whose plane stride is their difference) and land back to back in shared memory
-__device__ __forceinline__ void tma_load_3d_pair(uint32_t dst, const CUtensorMap* map, uint32_t leader_bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.3d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-      ::"r"(dst), "l"(map), "r"(leader_bar), "r"(c0), "r"(c1), "r"(0)
       : "memory");
 }
 constexpr int STAGE_EPI_BYTES = 4096;          // per epilogue warp: one 32-row x (128 B | 2 x 64 B) staging box
@@ -149,27 +142,11 @@ __device__ __forceinline__ void umma_commit_pair(uint32_t bar) {
       : "memory");
 }
 
-// K-major operand tile with rows of SLAB bytes (128: SWIZZLE_128B, 64: SWIZZLE_64B), 8-row groups 8 * SLAB bytes apart
-template <int SLAB>
-__device__ __forceinline__ uint64_t make_smem_desc_s(uint32_t smem_addr) {
-  uint64_t d = 0;
-  d |= (uint64_t)((smem_addr & 0x3ffff) >> 4);  // start address, bits [0,14)
-  d |= (uint64_t)1 << 16;                        // leading byte offset (unused for swizzled K-major)
-  d |= (uint64_t)((8 * SLAB) >> 4) << 32;        // stride byte offset = 8 rows * SLAB B
-  d |= (uint64_t)1 << 46;                        // descriptor version (Blackwell)
-  d |= (uint64_t)(SLAB == 128 ? 2 : 4) << 61;    // SWIZZLE_128B = 2, SWIZZLE_64B = 4
-  return d;
-}
-
-// SLAB = bytes of K per pipeline stage and operand row (128: three stages; the kernel is written for either).  Measured
-// (tools/gemm_timeline.py --slab, B200): the MMA issuer waits ~1 050 of ~1 980 cycles per 64-element chain for operands with
-// three 128-byte stages; SIX half-size stages (64-byte rows, 64B swizzle: 5 of 6 stages in flight instead of 2 of 3) are
-// SLOWER -- chain period 2 506 vs 1 979 cycles, 784 x 784 over 65 536 rows 274 vs 246 us, 1024 x 1024 366 vs 331 us: twice
-// the TMA operations per K, each fetching 64-byte rows, cost more than the deeper pipeline gives.  So SLAB = 128 it is; the
-// 64-byte instantiation is not built.
-template <int BLOCK_N, int NTERMS, int KIND, int SLAB = 128>
+// One pipeline stage holds one 128-byte K-slab per operand row (tc::SLAB_BYTES).  Six half-size stages (64-byte rows, 64B
+// swizzle) were measured slower on a B200 (784 x 784 over 65 536 rows: 274 vs 246 us; DESIGN.md section 4.2): twice the TMA
+// operations per K cost more than the deeper pipeline gives.
+template <int BLOCK_N, int NTERMS, int KIND>
 struct Config {
-  static constexpr int SLAB_BYTES = SLAB;       // (shadows tc::SLAB_BYTES inside this configuration)
   static_assert(BLOCK_N % 16 == 0 && BLOCK_N >= 32 && BLOCK_N <= 256, "UMMA N for M=256 (cta_group::2)");
   static_assert(NTERMS == 1 || NTERMS == 3, "1 = single pass, 3 = tf32 split");
   static constexpr int kBlockN = BLOCK_N;
@@ -238,8 +215,7 @@ __device__ __forceinline__ void red_add128(void* p, uint4 v) {
 }
 template <int RB>
 __device__ __forceinline__ void stage_copy_out(uint32_t stage, int lane, uint8_t* plane, long long ld_bytes,
-                                               long long row0, long long M, int col_bytes0, int n_bytes, int dbg_flags = 0,
-                                               bool atomic = false) {
+                                               long long row0, long long M, int col_bytes0, int n_bytes, bool atomic = false) {
   // plane + row * ld_bytes + col_bytes0 is the first byte of the box in global memory; n_bytes = row length in bytes
   constexpr int CPR = RB / 16, ROWS_PER_IT = 32 / CPR;
   const int chunk = lane % CPR, rsub = lane / CPR;
@@ -250,7 +226,7 @@ __device__ __forceinline__ void stage_copy_out(uint32_t stage, int lane, uint8_t
   for (int it = 0; it < CPR; ++it) t[it] = lds128(stage + stage_off<RB>(it * ROWS_PER_IT + rsub, chunk));
 #pragma unroll
   for (int it = 0; it < CPR; ++it)
-    if (row0 + it * ROWS_PER_IT + rsub < M && !(dbg_flags & 8)) {
+    if (row0 + it * ROWS_PER_IT + rsub < M) {
       if (atomic) red_add128(g + (long long)it * ROWS_PER_IT * ld_bytes, t[it]);
       else stg128(g + (long long)it * ROWS_PER_IT * ld_bytes, t[it]);
     }
@@ -385,6 +361,8 @@ __device__ __forceinline__ void store_chunk(const Epilogue& ep, const EpiRegs& e
   if (f & EF_OUT16) {      // fp16 split planes: x = hi + lo' 2^-11
     constexpr int RB = W * 2;
     const uint32_t stage_lo = stage + 32 * RB;
+    // debug flag 16: register-direct stores.  Unused, but deleting it shifts ptxas' register allocation and slowed the
+    // BLOCK_N = 256 3xTF32 instantiation by 2% (1024 x 1024 over 65 536 rows, B200)
     const bool direct = (dbg_flags & 16) != 0;
     uint4* gh = reinterpret_cast<uint4*>(er.oh + m * er.ld16 + n0);
     uint4* gl = reinterpret_cast<uint4*>(er.ol + m * er.ld16 + n0);
@@ -419,8 +397,8 @@ __device__ __forceinline__ void store_chunk(const Epilogue& ep, const EpiRegs& e
     if (dbg_slot) t2 = clock64();
     if (!direct) {
       __syncwarp();
-      stage_copy_out<RB>(stage, lane, reinterpret_cast<uint8_t*>(er.oh), (long long)er.ld16 * 2, row0, M, n0 * 2, N * 2, dbg_flags);
-      stage_copy_out<RB>(stage_lo, lane, reinterpret_cast<uint8_t*>(er.ol), (long long)er.ld16 * 2, row0, M, n0 * 2, N * 2, dbg_flags);
+      stage_copy_out<RB>(stage, lane, reinterpret_cast<uint8_t*>(er.oh), (long long)er.ld16 * 2, row0, M, n0 * 2, N * 2);
+      stage_copy_out<RB>(stage_lo, lane, reinterpret_cast<uint8_t*>(er.ol), (long long)er.ld16 * 2, row0, M, n0 * 2, N * 2);
       __syncwarp();
     }
     if (dbg_slot) {
@@ -436,7 +414,7 @@ __device__ __forceinline__ void store_chunk(const Epilogue& ep, const EpiRegs& e
       sts128(stage + stage_off<RB>(lane, q), __float_as_uint(v[4 * q]), __float_as_uint(v[4 * q + 1]), __float_as_uint(v[4 * q + 2]),
              __float_as_uint(v[4 * q + 3]));
     __syncwarp();
-    stage_copy_out<RB>(stage, lane, reinterpret_cast<uint8_t*>(er.of32), (long long)er.ldf32 * 4, row0, M, n0 * 4, N * 4, 0,
+    stage_copy_out<RB>(stage, lane, reinterpret_cast<uint8_t*>(er.of32), (long long)er.ldf32 * 4, row0, M, n0 * 4, N * 4,
                        (f & EF_ATOMIC) != 0);
     __syncwarp();
   }
@@ -900,15 +878,14 @@ __device__ __forceinline__ void epilogue_loop(int col0, int quarter, int lane, u
   __syncwarp();
 }
 
-template <int BLOCK_N, int NTERMS, int KIND, bool SPLITK = false, int SLAB = 128>
+template <int BLOCK_N, int NTERMS, int KIND, bool SPLITK = false>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
 gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_a_lo,
                 const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_w_lo,
-                long long M, int N, int K, int chunk_slabs, int lead_chains, int split_k, int split_per, int planes3d,
+                long long M, int N, int K, int chunk_slabs, int lead_chains, int split_k, int split_per,
                 const __grid_constant__ Epilogue ep, const __grid_constant__ StoreMaps smaps, unsigned long long* dbg_buf,
                 int dbg_flags) {
-  using C = Config<BLOCK_N, NTERMS, KIND, SLAB>;
-  constexpr int SLAB_BYTES = C::SLAB_BYTES;
+  using C = Config<BLOCK_N, NTERMS, KIND>;
   extern __shared__ uint8_t smem_raw[];
   uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;   // same offset in both CTAs of the pair
   asm volatile("" : "+r"(smem_base));   // opaque: otherwise every use re-derives it (S2UR SR_CgaCtaId + arithmetic)
@@ -931,8 +908,8 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
   if (!SPLITK || split_k < 1) split_k = 1;
   const long long n_tiles = m_blocks * n_blocks * split_k;
   if (chunk_slabs <= 0 || chunk_slabs > k_slabs) chunk_slabs = k_slabs;
-  if (KIND == KIND_F16 && NTERMS == 3) chunk_slabs = 128 / SLAB_BYTES;   // 64 K-elements per accumulation chain (the 2^-11
-                                                                         // rescale happens once per chain)
+  if (KIND == KIND_F16 && NTERMS == 3) chunk_slabs = 1;   // one K-slab = 64 K-elements per accumulation chain (the 2^-11
+                                                         // rescale happens once per chain)
   // the last tile of a tile row is only as wide as N needs (UMMA N is a run-time field of the instruction descriptor;
   // multiples of 16 for M = 256), and the last K-slab only issues the 32-byte K steps that hold data
   auto tile_width = [&](int n_idx) {
@@ -989,16 +966,11 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
             const int k_idx = (tc.ks_begin + ks) * C::ELEMS_PER_SLAB;
             const uint32_t fb = mapa(full_bar(stage), 0);
             if (rank == 0) mbar_expect_tx(full_bar(stage), 2 * C::STAGE_BYTES);
-            if (NTERMS == 3 && planes3d) {          // hi + lo planes of A (and of W) in one operation each
-              tma_load_3d_pair(sa, &tm_a, fb, k_idx, m_idx);
-              tma_load_3d_pair(sb, &tm_w, fb, k_idx, n_idx);
-            } else {
-              tma_load_2d_pair(sa, &tm_a, fb, k_idx, m_idx);
-              tma_load_2d_pair(sb, &tm_w, fb, k_idx, n_idx);
-              if (NTERMS == 3) {
-                tma_load_2d_pair(sa + C::A_TILE, &tm_a_lo, fb, k_idx, m_idx);
-                tma_load_2d_pair(sb + C::B_TILE, &tm_w_lo, fb, k_idx, n_idx);
-              }
+            tma_load_2d_pair(sa, &tm_a, fb, k_idx, m_idx);
+            tma_load_2d_pair(sb, &tm_w, fb, k_idx, n_idx);
+            if (NTERMS == 3) {
+              tma_load_2d_pair(sa + C::A_TILE, &tm_a_lo, fb, k_idx, m_idx);
+              tma_load_2d_pair(sb + C::B_TILE, &tm_w_lo, fb, k_idx, n_idx);
             }
             if (++stage == C::STAGES) { stage = 0; phase ^= 1; }
           }
@@ -1038,8 +1010,8 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
               {
                 const uint32_t sa = smem_base + st * C::STAGE_BYTES;
                 const uint32_t sb = sa + C::NPLANES * C::A_TILE;
-                const uint64_t da_hi = make_smem_desc_s<SLAB_BYTES>(sa), db_hi = make_smem_desc_s<SLAB_BYTES>(sb);
-                const uint64_t da_lo = make_smem_desc_s<SLAB_BYTES>(sa + C::A_TILE), db_lo = make_smem_desc_s<SLAB_BYTES>(sb + C::B_TILE);
+                const uint64_t da_hi = make_smem_desc(sa), db_hi = make_smem_desc(sb);
+                const uint64_t da_lo = make_smem_desc(sa + C::A_TILE), db_lo = make_smem_desc(sb + C::B_TILE);
                 const int nk = ks == ks_last ? last_ksteps : KSTEPS;
 #pragma unroll
                 for (int k = 0; k < KSTEPS; ++k) {
@@ -1057,7 +1029,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
               {
                 const uint32_t sa = smem_base + stage * C::STAGE_BYTES;
                 const uint32_t sb = sa + C::NPLANES * C::A_TILE;
-                const uint64_t da_hi = make_smem_desc_s<SLAB_BYTES>(sa), db_hi = make_smem_desc_s<SLAB_BYTES>(sb);
+                const uint64_t da_hi = make_smem_desc(sa), db_hi = make_smem_desc(sb);
                 const int nk = ks == ks_last ? last_ksteps : KSTEPS;
                 if (ks == ks0) umma_pair_f16_scale11(da_hi, db_hi, tmem_d, idesc);
 #pragma unroll
@@ -1080,10 +1052,10 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
               {
                 const uint32_t sa = smem_base + stage * C::STAGE_BYTES;
                 const uint32_t sb = sa + C::NPLANES * C::A_TILE;
-                const uint64_t da_hi = make_smem_desc_s<SLAB_BYTES>(sa), db_hi = make_smem_desc_s<SLAB_BYTES>(sb);
+                const uint64_t da_hi = make_smem_desc(sa), db_hi = make_smem_desc(sb);
                 const int nk = ks == ks_last ? last_ksteps : KSTEPS;
                 if (NTERMS == 3) {  // small terms first: they meet the accumulator while it is smallest
-                  const uint64_t da_lo = make_smem_desc_s<SLAB_BYTES>(sa + C::A_TILE), db_lo = make_smem_desc_s<SLAB_BYTES>(sb + C::B_TILE);
+                  const uint64_t da_lo = make_smem_desc(sa + C::A_TILE), db_lo = make_smem_desc(sb + C::B_TILE);
 #pragma unroll
                   for (int k = 0; k < KSTEPS; ++k) {
                     if (k < nk) {
@@ -1189,36 +1161,16 @@ inline int make_store_map32(CUtensorMap* map, const void* ptr, long long rows, l
   return USF_OK;
 }
 
-extern int g_planes3d;                  // 1: hi / lo operand planes travel in one 3-D TMA operation where possible (usf_debug_set_planes3d;
-                                        // measured neutral: 246.5 vs 247.3 us on 784 x 784, so the default stays one 2-D operation per plane)
-
-// [2 planes, rows, cols] operand map over two plane pointers (plane stride = their distance); false if they do not allow it
-inline bool make_operand_map3(CUtensorMap* map, const void* hi, const void* lo, long long rows, long long cols, long long ld,
-                              int box_rows, int dtype) {
-  PFN_encodeTiled enc = get_encode_tiled();
-  const long long diff = (const char*)lo - (const char*)hi;
-  if (!enc || diff <= 0 || diff % 16 != 0 || diff >= (1LL << 40)) return false;
-  const int esz = dtype ? 2 : 4;
-  cuuint64_t dims[3] = {(cuuint64_t)cols, (cuuint64_t)rows, 2};
-  cuuint64_t strides[2] = {(cuuint64_t)ld * esz, (cuuint64_t)diff};
-  cuuint32_t box[3] = {(cuuint32_t)(tc::SLAB_BYTES / esz), (cuuint32_t)box_rows, 2};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = enc(map, dtype == 1 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : dtype == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3,
-                   const_cast<void*>(hi), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  return r == CUDA_SUCCESS;
-}
-
-template <int BLOCK_N, int NTERMS, int KIND, bool SPLITK = false, int SLAB = 128>
+template <int BLOCK_N, int NTERMS, int KIND, bool SPLITK = false>
 int launch_gemm_tc2_cfg(const usf_linear_args* a, const Epilogue& ep_in, cudaStream_t st) {
-  using C = tc2::Config<BLOCK_N, NTERMS, KIND, SLAB>;
+  using C = tc2::Config<BLOCK_N, NTERMS, KIND>;
   constexpr bool F16S = NTERMS == 3 && KIND == tc2::KIND_F16;
   // split-K exists for the fp16-split engine (the training pass); every other engine runs the plain kernel
   if (!SPLITK && F16S && a->split_k > 1)
-    return launch_gemm_tc2_cfg<BLOCK_N, NTERMS, KIND, F16S, SLAB>(a, ep_in, st);
+    return launch_gemm_tc2_cfg<BLOCK_N, NTERMS, KIND, F16S>(a, ep_in, st);
   static bool attr_set_dev[MAX_DEVICES] = {false};
   bool& attr_set = attr_set_dev[current_device_slot()];
-  auto kern = tc2::gemm_tc2_kernel<BLOCK_N, NTERMS, KIND, SPLITK, SLAB>;
+  auto kern = tc2::gemm_tc2_kernel<BLOCK_N, NTERMS, KIND, SPLITK>;
   const int dt = KIND == tc2::KIND_TF32 ? 0 : KIND == tc2::KIND_BF16 ? 1 : 2;
   if (!attr_set) {
     USF_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
@@ -1226,23 +1178,11 @@ int launch_gemm_tc2_cfg(const usf_linear_args* a, const Epilogue& ep_in, cudaStr
   }
   CUtensorMap ma, mal, mw, mwl;
   int rc;
-  int planes3d = 0;
-  if (NTERMS == 3 && SLAB == 128 && g_planes3d) {
-    CUtensorMap ta, tw;
-    if (make_operand_map3(&ta, a->a, a->a_lo, a->M, a->K, a->lda, tc::BLOCK_M, dt) &&
-        make_operand_map3(&tw, a->w, a->w_lo, a->N, a->K, a->ldw, C::HALF_N, dt)) {
-      ma = ta; mw = tw; mal = ta; mwl = tw;
-      planes3d = 1;
-    }
-  }
-  if (planes3d) {
-  } else if ((rc = make_operand_map(&ma, a->a, a->M, a->K, a->lda, tc::BLOCK_M, dt, SLAB))) {
-    return rc;
-  } else if ((rc = make_operand_map(&mw, a->w, a->N, a->K, a->ldw, C::HALF_N, dt, SLAB))) {
-    return rc;
-  } else if (NTERMS == 3) {
-    if ((rc = make_operand_map(&mal, a->a_lo, a->M, a->K, a->lda, tc::BLOCK_M, dt, SLAB))) return rc;
-    if ((rc = make_operand_map(&mwl, a->w_lo, a->N, a->K, a->ldw, C::HALF_N, dt, SLAB))) return rc;
+  if ((rc = make_operand_map(&ma, a->a, a->M, a->K, a->lda, tc::BLOCK_M, dt))) return rc;
+  if ((rc = make_operand_map(&mw, a->w, a->N, a->K, a->ldw, C::HALF_N, dt))) return rc;
+  if (NTERMS == 3) {
+    if ((rc = make_operand_map(&mal, a->a_lo, a->M, a->K, a->lda, tc::BLOCK_M, dt))) return rc;
+    if ((rc = make_operand_map(&mwl, a->w_lo, a->N, a->K, a->ldw, C::HALF_N, dt))) return rc;
   } else {
     mal = ma;
     mwl = mw;
@@ -1276,9 +1216,7 @@ int launch_gemm_tc2_cfg(const usf_linear_args* a, const Epilogue& ep_in, cudaStr
   int split_k = 1, split_per = 0;
   if (SPLITK && a->split_k > 1) {
     const int k_slabs = (int)((a->K + C::ELEMS_PER_SLAB - 1) / C::ELEMS_PER_SLAB);
-    constexpr int CH = F16S ? 128 / SLAB : 1;               // a piece is a whole number of accumulation chains
-    int per = (k_slabs + a->split_k - 1) / a->split_k;
-    per = (per + CH - 1) / CH * CH;
+    const int per = (k_slabs + a->split_k - 1) / a->split_k;   // (an accumulation chain of this engine is one slab)
     split_k = (k_slabs + per - 1) / per;                    // every work item gets at least one slab
     split_per = per;
     USF_REQUIRE(ep.fast_store && ep.out_f32 && !ep.out_h16 && !ep.out_hi && !ep.out_bf16 && !ep.bias && !ep.relu &&
@@ -1291,7 +1229,7 @@ int launch_gemm_tc2_cfg(const usf_linear_args* a, const Epilogue& ep_in, cudaStr
   const int grid = 2 * (int)(tiles < pairs ? tiles : pairs);
   USF_CUDA_OK(launch_chain(kern, dim3(grid), dim3(tc::NUM_THREADS), (size_t)C::SMEM_BYTES, st, ma, mal, mw, mwl, (long long)a->M,
                            (int)a->N, (int)a->K, NTERMS == 3 ? g_chunk_slabs : 0,
-                           (NTERMS == 3 && KIND == tc2::KIND_F16) ? g_lead_chains : 0, split_k, split_per, planes3d, ep, sm, g_dbg_buf,
+                           (NTERMS == 3 && KIND == tc2::KIND_F16) ? g_lead_chains : 0, split_k, split_per, ep, sm, g_dbg_buf,
                            g_dbg_flags));
   return USF_OK;
 }
@@ -1327,7 +1265,6 @@ int launch_gemm_tc2_tf32(const usf_linear_args* a, const Epilogue& ep, cudaStrea
 int launch_gemm_tc2_bf16(const usf_linear_args* a, const Epilogue& ep, cudaStream_t st, int bn);
 int launch_gemm_tc2_3xf16(const usf_linear_args* a, const Epilogue& ep, cudaStream_t st, int bn);
 
-extern int g_tc_impl;         // 2 = CTA-pair kernel (default), 1 = single-CTA kernel (usf_debug_set_impl)
 extern int g_force_block_n;   // test hook (usf_debug_set_block_n)
 
 inline int launch_gemm_tc(const usf_linear_args* a, const Epilogue& ep, cudaStream_t st) {
@@ -1341,20 +1278,11 @@ inline int launch_gemm_tc(const usf_linear_args* a, const Epilogue& ep, cudaStre
   USF_REQUIRE(!a->trans_w, "trans_w is a SIMT-engine option");
   if (a->engine == USF_ENGINE_TC_3XTF32 || a->engine == USF_ENGINE_TC_3XF16)
     USF_REQUIRE(a->a_lo && a->w_lo && aligned16(a->a_lo) && aligned16(a->w_lo), "split engines need a_lo and w_lo planes");
-  if (a->engine == USF_ENGINE_TC_3XF16) {
-    const int bn = g_force_block_n > 0 ? g_force_block_n : pick_block_n2(a->N);
-    return launch_gemm_tc2_3xf16(a, ep, st, bn);
-  }
-  if (g_tc_impl == 2) {
-    const int bn = g_force_block_n > 0 ? g_force_block_n : pick_block_n2(a->N);
-    if (a->engine == USF_ENGINE_TC_3XTF32) return launch_gemm_tc2_3xtf32(a, ep, st, bn);
-    if (a->engine == USF_ENGINE_TC_TF32) return launch_gemm_tc2_tf32(a, ep, st, bn);
-    return launch_gemm_tc2_bf16(a, ep, st, bn);
-  }
-  const int bn = g_force_block_n > 0 ? g_force_block_n : pick_block_n(a->N);
-  if (a->engine == USF_ENGINE_TC_3XTF32) return launch_gemm_tc_3xtf32(a, ep, st, bn);
-  if (a->engine == USF_ENGINE_TC_TF32) return launch_gemm_tc_tf32(a, ep, st, bn);
-  return launch_gemm_tc_bf16(a, ep, st, bn);
+  const int bn = g_force_block_n > 0 ? g_force_block_n : pick_block_n2(a->N);
+  if (a->engine == USF_ENGINE_TC_3XF16) return launch_gemm_tc2_3xf16(a, ep, st, bn);
+  if (a->engine == USF_ENGINE_TC_3XTF32) return launch_gemm_tc2_3xtf32(a, ep, st, bn);
+  if (a->engine == USF_ENGINE_TC_TF32) return launch_gemm_tc2_tf32(a, ep, st, bn);
+  return launch_gemm_tc2_bf16(a, ep, st, bn);
 }
 
 }  // namespace usf

@@ -1,10 +1,7 @@
-// Instantiations of the tcgen05 contractions for the 3xtf32 engine (own translation unit: parallel build).
+// Instantiations of the CTA-pair tcgen05 contraction for the 3xtf32 engine (own translation unit: parallel build).
 #include "gemm_tc2.cuh"
 
 namespace usf {
-int launch_gemm_tc_3xtf32(const usf_linear_args* a, const Epilogue& ep, cudaStream_t st, int bn) {
-  return launch_gemm_tc_terms<3, false>(a, ep, st, bn);
-}
 int launch_gemm_tc2_3xtf32(const usf_linear_args* a, const Epilogue& ep, cudaStream_t st, int bn) {
   return launch_gemm_tc2_terms<3, tc2::KIND_TF32>(a, ep, st, bn);
 }
