@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define USF_ABI_VERSION 9   /* ABI 9: the test hooks that chose the single-CTA GEMM and the 3-D operand loads are gone */
+#define USF_ABI_VERSION 10  /* ABI 10: the accumulation / pixel-plane tuning setters and the GEMM timeline hook are gone; usf_debug_set_store_path */
 
 #define USF_OK 0
 #define USF_ERR_INVALID (-1)     /* bad argument (shape, alignment, null pointer) */
@@ -132,29 +132,17 @@ typedef struct usf_linear_args {
 
 int usf_linear(const usf_linear_args* args, void* stream);
 
-/* TC_3XTF32 accuracy knob: number of 32-element K-slabs accumulated in TMEM before the partial tile is
- * added into fp32 registers with round-to-nearest (the tensor core truncates when it accumulates; long
- * chains carry a systematic toward-zero bias).  0 = accumulate the whole K in TMEM.  Default 2. */
-int usf_set_accum_chunk(int k_slabs);
-/* fp16-split engine (TC_3XF16), CTA-pair kernel: the first `chains` (0, 1 or 2; default 2) accumulation chains of every output tile
- * span twice the usual number of K-slabs, so the tensor core keeps running on the next tile while the epilogue warps
- * still store the previous one (two TMEM accumulators = two chains of run-ahead).  Not applied to TC_3XTF32: its
- * chains already hold 48 MMA steps and the toward-zero accumulation bias of longer chains shows in the gradients. */
-int usf_set_accum_lead(int chains);
 /* test hook: force the tcgen05 tile width BLOCK_N (0 = automatic) */
 int usf_debug_set_block_n(int block_n);
 /* test hook: 1 (default) = the kernels of an evaluation are chained with programmatic dependent launch, 0 = plain
  * stream order */
 int usf_debug_set_pdl(int on);
-/* profiling hook for the CTA-pair tcgen05 kernel: `device_buf` (512 x 8 uint64, or NULL to switch off) receives
- * clock64() stamps of the first 512 accumulation chains of cluster 0 (0 = accumulator free seen by the MMA issuer,
- * 1 = operands landed, 2 = chain issued, 3 = accumulator full seen by epilogue warp 4, 4 = drained, 5 = tile stored);
- * `flags`: 1 = epilogue skips the TMEM drain, 2 = epilogue skips the store phase (timing experiments only:
- * results are wrong with either flag set); 256 = the coupling residual is read lane-per-row instead of coalesced through the
- * epilogue warp's in-box (same bits, slower); 4 = outputs leave through the generic register/patch store path instead of
- * the staged coalesced one; 32 = the epilogue warps copy their staged boxes out themselves instead of issuing
- * TMA stores (results identical with 4 and 32; tests cover the paths). */
-int usf_debug_gemm_timeline(unsigned long long* device_buf, int flags);
+/* test hook for the CTA-pair tcgen05 kernel: force the store / residual paths that automatic choice takes only on other
+ * shapes or configurations (0 = automatic; results are bit-identical on every path).  `flags` combines 4 = outputs leave
+ * through the generic register/patch store path instead of the staged coalesced one, 32 = the epilogue warps copy their
+ * staged boxes out themselves instead of issuing TMA stores, 256 = the coupling residual is read lane-per-row instead of
+ * coalesced through the epilogue warp's in-box.  Any other bit: USF_ERR_INVALID. */
+int usf_debug_set_store_path(int flags);
 
 /* ------------------------------------------------------------------------------------------------
  * whole layer stack in one launch for tiny event sizes (d <= 8, conditioner width <= 64): replaces the per-layer loop
@@ -324,8 +312,6 @@ typedef struct usf_conv_pix_args {
  * last convolution, MaskedCoupling's update.  USF_ERR_UNSUPPORTED when w > 256 or the k*k*4 KB weight leaves no room for two
  * 32 KB pipeline stages in 227 KB of shared memory. */
 int usf_conv2d_pix(const usf_conv_pix_args* a, void* stream);
-int usf_set_pix_gate_at(int32_t chains);     /* gated block: chains of the next tile issued in front of a tile's 1 x 1 contraction (default 1); tools only */
-int usf_set_pix_chain_taps(int32_t taps);   /* taps per TMEM accumulation chain (0 = default: 3 = 96 K-elements in the gated block, 2 in a plain convolution); tools only */
 
 /* x[r, c] += sign * g[(r mod hw)*c_dim + c] * t[r, c]: MaskedCoupling.forward/backward with a mask over [C, H, W]
  * (transforms.py:284-290, 301-306; g = 1 - mask in channels-last order). */

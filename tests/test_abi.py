@@ -16,7 +16,7 @@ def _declared_symbols():
     return sorted(set(re.findall(r"\b(usf_[a-z0-9_]+)\s*\(", text)))
 
 
-def test_header_symbols_are_exported_and_bound():
+def test_header_symbols_are_exported_bound_and_versioned():
     from usflows_b200 import _lib
     lib = _lib.load()
     declared = _declared_symbols()
@@ -24,7 +24,7 @@ def test_header_symbols_are_exported_and_bound():
     for name in declared:
         assert hasattr(lib, name), f"{name} declared in the header but not exported"
         assert name in _lib.SIGNATURES, f"{name} has no ctypes signature in _lib.py"
-    assert lib.usf_abi_version() == 9
+    assert lib.usf_abi_version() == 10
 
 
 def test_planes_struct_layout_matches_header():
@@ -121,11 +121,13 @@ def test_conv_pix_args_layout_matches_header():
     assert ctypes.sizeof(_lib.ConvPixArgs) == 2 * 8 + 4 * 4 + 2 * 8 + 4 * 4 + 4 * 8 + 2 * 4 + 3 * 8 + 2 * 4 + 4 * 8
 
 
-def test_conv_pix_entry_points_reject_bad_input_without_gpu():
+def test_pix_and_store_path_entry_points_reject_bad_input_without_gpu():
     from usflows_b200 import _lib
     lib = _lib.load()
     assert lib.usf_conv2d_pix(None, None) == -1 and b"null args" in lib.usf_last_error()
     a = _lib.ConvPixArgs()
     assert lib.usf_conv2d_pix(ctypes.byref(a), None) == -1                  # null operands
     assert lib.usf_pix_encode(None, 0, 0, 16, 49, None, 0, None, None, None) == -1
-    assert lib.usf_set_pix_chain_taps(0) == 0 and lib.usf_set_pix_gate_at(0) == 0
+    assert lib.usf_debug_set_store_path(16) == -1 and b"store path flags" in lib.usf_last_error()
+    assert lib.usf_debug_set_store_path(1 << 30) == -1
+    assert lib.usf_debug_set_store_path(4 | 32 | 256) == 0 and lib.usf_debug_set_store_path(0) == 0

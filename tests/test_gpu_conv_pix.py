@@ -147,47 +147,25 @@ def test_gated_block_in_one_launch(n, H, W, ln, relu_planes):
     assert int(flag.item()) == 0
 
 
-def test_overflow_flag_and_chain_length():
-    from usflows_b200 import _lib, ops
+def test_overflow_flag_and_multi_tile_gated_block():
+    from usflows_b200 import ops
     n, H, W = 9, 7, 7
     a16, _, _, _ = _encode_input(n, 32, H, W, seed=1, mask=False)
     w, b, w16, b32 = _weight(32, 32, 3, seed=2)
     rows = n * H * W
-    outs = []
-    for taps in (1, 2, 3, 9):
-        _lib.check(_lib.load().usf_set_pix_chain_taps(taps))
-        o = torch.empty(rows, 32, device="cuda")
-        ops.conv2d_pix(a16, n, H, W, 3, 1, w16, b32, 32, out_f32=o)
-        outs.append(o.cpu())
-    _lib.check(_lib.load().usf_set_pix_chain_taps(0))
-    for o in outs[1:]:
-        assert rel_err(o, outs[0]) <= 2e-6
     # the gated block with several tiles per CTA (the gate contraction of tile i is issued among the chains of tile i + 1)
+    # against fp64 torch on the decoded inputs, as test_gated_block_in_one_launch
     n2 = 4000
+    rows2 = n2 * H * W
     a2, _, _, _ = _encode_input(n2, 32, H, W, seed=4, mask=False, relu=True)
     w2_, b2_, w16_2, b32_2 = _weight(64, 32, 1, seed=6)
-    y0 = torch.randn(n2 * H * W, 32, generator=torch.Generator().manual_seed(8)).cuda()
-    ys = []
-    for taps in (1, 2, 3, 9):
-        _lib.check(_lib.load().usf_set_pix_chain_taps(taps))
-        yy = y0.clone()
-        ops.conv2d_pix(a2, n2, H, W, 3, 1, w16, b32, 32, gated=True, post_relu=True, w2=w16_2, bias2=b32_2, out_f32=yy)
-        ys.append(yy.cpu())
-    _lib.check(_lib.load().usf_set_pix_chain_taps(0))
-    for yy in ys[1:]:
-        assert rel_err(yy, ys[0]) <= 2e-6
-    # ... and wherever the gate contraction of a tile is issued among the chains of the next one: the same bits
-    for taps in (1, 3):
-        _lib.check(_lib.load().usf_set_pix_chain_taps(taps))
-        base = None
-        for gate_at in (0, 1, 2, 3, 7):
-            _lib.check(_lib.load().usf_set_pix_gate_at(gate_at))
-            yy = y0.clone()
-            ops.conv2d_pix(a2, n2, H, W, 3, 1, w16, b32, 32, gated=True, post_relu=True, w2=w16_2, bias2=b32_2, out_f32=yy)
-            base = yy if base is None else base
-            assert torch.equal(yy, base)
-    _lib.check(_lib.load().usf_set_pix_gate_at(1))
-    _lib.check(_lib.load().usf_set_pix_chain_taps(0))
+    y0 = torch.randn(rows2, 32, generator=torch.Generator().manual_seed(8))
+    u = torch.relu(F.conv2d(_as_image(_decode(a2).cpu(), n2, H, W), _decoded_weight(w16, 32, 32, 3), b.double(), padding="same"))
+    vg = F.conv2d(u, _decoded_weight(w16_2, 64, 32, 1), b2_.double()).permute(0, 2, 3, 1).reshape(rows2, 64)
+    want = torch.relu(y0.double() + vg[:, :32] * torch.sigmoid(vg[:, 32:]))
+    y = y0.cuda()
+    ops.conv2d_pix(a2, n2, H, W, 3, 1, w16, b32, 32, gated=True, post_relu=True, w2=w16_2, bias2=b32_2, out_f32=y)
+    assert float((y.cpu().double() - want).abs().max()) <= 1e-5 * max(1.0, float(want.abs().max()))
     flag = torch.zeros(1, dtype=torch.int32, device="cuda")
     p16 = torch.empty(rows, 64, dtype=torch.float16, device="cuda")
     ops.conv2d_pix(a16, n, H, W, 3, 1, w16, (b32 + 1e5).contiguous(), 32, out16=p16, overflow_flag=flag)

@@ -87,26 +87,24 @@ def test_narrow_rows_kernel_full_epilogue(M, N, K):
 
 
 @pytest.mark.parametrize("bn", [32, 64, 128, 208, 256])
-@pytest.mark.parametrize("chunk", [0, 1, 3])
-def test_tile_widths_and_accumulation_chunks(bn, chunk):
+def test_tile_widths(bn):
+    """Every tcgen05 tile width on the 3xTF32 engine (several accumulation chains per tile) against fp64."""
     from usflows_b200 import _lib, ops
     from usflows_b200.ops import Act
     M, N, K = 400, 600, 500
-    g = torch.Generator().manual_seed(bn + chunk)
+    g = torch.Generator().manual_seed(bn)
     a, w = torch.randn(M, K, generator=g), torch.randn(N, K, generator=g) / K ** 0.5
     act, a_used = _planes(a, "split")
     wact, w_used = _planes(w, "split")
     out = Act(M, N, f32=torch.zeros(M, ops.pad4(N), device="cuda")[:, :N])
     lib = _lib.load()
     lib.usf_debug_set_block_n(bn)
-    lib.usf_set_accum_chunk(chunk)
     try:
         ops.linear(1, act, wact.hi, wact.lo, N, K, out=out)
         torch.cuda.synchronize()
     finally:
         lib.usf_debug_set_block_n(0)
-        lib.usf_set_accum_chunk(2)
-    assert rel_err(out.f32, a_used.double() @ w_used.double().T) <= (3e-6 if chunk else 2e-5)
+    assert rel_err(out.f32, a_used.double() @ w_used.double().T) <= 3e-6
 
 
 def test_simt_transposed_weight_and_unaligned():
@@ -241,7 +239,7 @@ def test_fp16_split_engine_full_epilogue(M, N, K):
 
 @pytest.mark.parametrize("eng_name,eng,fmt", [("3xtf32", 1, "split"), ("tf32", 2, "f32"), ("bf16", 3, "bf16"), ("3xf16", 4, "f16")])
 @pytest.mark.parametrize("M,N,K", [(300, 784, 392), (515, 392, 1024), (130, 600, 72), (64, 48, 40), (513, 100, 56)])
-def test_staged_store_path_equals_register_store_path(eng_name, eng, fmt, M, N, K):
+def test_forced_store_paths_equal_the_staged_store(eng_name, eng, fmt, M, N, K):
     """The staged coalesced-store epilogue and the generic register/patch epilogue produce identical bits."""
     from usflows_b200 import _lib, ops
     from usflows_b200.ops import Act
@@ -260,12 +258,12 @@ def test_staged_store_path_equals_register_store_path(eng_name, eng, fmt, M, N, 
                   hi=torch.zeros(M, ops.pad4(N), device="cuda")[:, :N], lo=torch.zeros(M, ops.pad4(N), device="cuda")[:, :N],
                   bf16=torch.zeros(M, ops.pad4(N), device="cuda", dtype=torch.bfloat16)[:, :N])
         out.h16, out.l16 = torch.zeros(2, M, ops.pad4(N), dtype=torch.float16, device="cuda")[:, :, :N]
-        lib.usf_debug_gemm_timeline(None, flags)
+        lib.usf_debug_set_store_path(flags)
         try:
             ops.linear(eng, act, w_hi, w_lo, N, K, bias=bias, relu=True, out=out)
             torch.cuda.synchronize()
         finally:
-            lib.usf_debug_gemm_timeline(None, 0)
+            lib.usf_debug_set_store_path(0)
         results.append(out)
     p = results[0]
     for q in results[1:]:
@@ -278,7 +276,7 @@ def test_staged_store_path_equals_register_store_path(eng_name, eng, fmt, M, N, 
 
 @pytest.mark.parametrize("M,N,K", [(300, 784, 392), (70000, 1024, 128), (515, 400, 1024), (130, 608, 72), (64, 48, 40),
                                    (1000, 392, 1024), (257, 112, 64)])
-def test_tma_store_path_equals_inline_store(M, N, K):
+def test_forced_residual_and_store_paths_equal_the_tma_store(M, N, K):
     """fp16-split planes only (the hot configuration): boxes stored by TMA == stored by the epilogue warps themselves,
     including the in-place coupling form (residual read from the planes that are written)."""
     from usflows_b200 import _lib, ops
@@ -294,13 +292,13 @@ def test_tma_store_path_equals_inline_store(M, N, K):
     outs = []
     for flags in (0, 256, 32, 4):                         # 256: residual read lane-per-row instead of through the in-box
         stream, _ = _f16_planes(x0)                       # fresh copy of the stream for the in-place update
-        lib.usf_debug_gemm_timeline(None, flags)
+        lib.usf_debug_set_store_path(flags)
         try:
             ops.linear(ops.ENGINE_TC_3XF16, act, wact.h16, wact.l16, N, K, bias=bias, resid=stream, resid_sign=-1.0,
                        out=Act(M, N, h16=stream.h16, l16=stream.l16))
             torch.cuda.synchronize()
         finally:
-            lib.usf_debug_gemm_timeline(None, 0)
+            lib.usf_debug_set_store_path(0)
         outs.append(stream)
     for q in outs[1:]:
         assert torch.equal(outs[0].h16, q.h16) and torch.equal(outs[0].l16, q.l16)
@@ -461,7 +459,7 @@ def test_mat_prep_and_tri_mask():
 @pytest.mark.parametrize("eng_name,eng,fmt", [("tf32", 2, "f32"), ("bf16", 3, "bf16"), ("3xf16", 4, "f16")])
 @pytest.mark.parametrize("planes", ["bf16", "bf16+f32+resid", "f32", "f32+resid"])
 @pytest.mark.parametrize("M,N,K", [(300, 784, 392), (70000, 1024, 64), (515, 392, 1024), (130, 600, 72), (64, 48, 40), (257, 112, 64)])
-def test_tma_store_path_for_bf16_and_fp32_planes(eng_name, eng, fmt, planes, M, N, K):
+def test_forced_store_paths_equal_the_tma_store_of_bf16_and_fp32_planes(eng_name, eng, fmt, planes, M, N, K):
     """Mode 2 of the asynchronous store path (bf16 plane and / or fp32 plane leave through TMA tensor stores: the bf16 and
     tf32 precision modes, and every fp32 result of the fp16-split engine) == the epilogue warps storing themselves (flag 32)
     == the generic register path (flag 4), including the in-place coupling form with an fp32 residual stream."""
@@ -486,12 +484,12 @@ def test_tma_store_path_for_bf16_and_fp32_planes(eng_name, eng, fmt, planes, M, 
         if "bf16" in planes:
             out.bf16 = torch.zeros(M, ops.pad4(N), device="cuda", dtype=torch.bfloat16)[:, :N]
         resid = Act(M, N, f32=out.f32) if "resid" in planes else None           # in place on the fp32 stream
-        lib.usf_debug_gemm_timeline(None, flags)
+        lib.usf_debug_set_store_path(flags)
         try:
             ops.linear(eng, act, w_hi, w_lo, N, K, bias=bias, relu="resid" not in planes, resid=resid, resid_sign=-1.0, out=out)
             torch.cuda.synchronize()
         finally:
-            lib.usf_debug_gemm_timeline(None, 0)
+            lib.usf_debug_set_store_path(0)
         results.append(out)
     p = results[0]
     for q in results[1:]:

@@ -1,7 +1,7 @@
 """GEMM micro-benchmark / checker for the tcgen05 contraction kernels (run on the B200 box).
 
-    python tools/gemm_bench.py [--engines 3xtf32,tf32,bf16] [--shapes 16384x784x784,...] [--chunk 2]
-                               [--bn 0] [--check] [--iters 20]
+    python tools/gemm_bench.py [--engines 3xtf32,tf32,bf16] [--shapes 16384x784x784,...] [--bn 0] [--check]
+                               [--iters 20] [--flags 0]
 
 Prints one JSON line per (engine, shape): time, MMA-level TFLOP/s (counting every tensor-core pass), and the
 error against an fp64 product when --check is given.
@@ -65,21 +65,17 @@ def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--engines", default="3xf16,3xtf32,tf32,bf16")
     ap.add_argument("--shapes", default="16384x784x784,16384x1024x784,16384x1024x1024,16384x784x1024,16384x3072x3072")
-    ap.add_argument("--chunk", type=int, default=-1)
     ap.add_argument("--bn", type=int, default=0)
     ap.add_argument("--iters", type=int, default=20)
     ap.add_argument("--check", action="store_true")
     ap.add_argument("--epi", action="store_true", help="bias + relu epilogue")
-    ap.add_argument("--lead", type=int, default=-1)
     ap.add_argument("--resid", action="store_true", help="3xf16: in-place coupling residual (out = out - (a.w^T + bias))")
-    ap.add_argument("--flags", type=int, default=0, help="usf_debug_gemm_timeline flags (256 = residual without the in-box)")
+    ap.add_argument("--flags", type=int, default=0,
+                    help="usf_debug_set_store_path flags (4 = register/patch store, 32 = no TMA stores, 256 = residual without the in-box)")
     args = ap.parse_args()
     lib = _lib.load()
-    if args.chunk >= 0:
-        lib.usf_set_accum_chunk(args.chunk)
     lib.usf_debug_set_block_n(args.bn)
-    if args.lead >= 0:
-        lib.usf_set_accum_lead(args.lead)
+    _lib.check(lib.usf_debug_set_store_path(args.flags))
     print(torch.cuda.get_device_name(0), flush=True)
     for eng in args.engines.split(","):
         for shp in args.shapes.split(","):
@@ -91,8 +87,7 @@ def main():
                     ops.linear(ENG[eng], act, wt, wl, N, K, bias=bias, resid=out, resid_sign=-1.0, out=out)
                 else:
                     ops.linear(ENG[eng], act, wt, wl, N, K, bias=bias, relu=args.epi, out=out)
-            lib.usf_debug_gemm_timeline(None, args.flags)
-            rec = dict(engine=eng, M=M, N=N, K=K, bn=args.bn, chunk=args.chunk)
+            rec = dict(engine=eng, M=M, N=N, K=K, bn=args.bn, flags=args.flags)
             try:
                 for _ in range(3):
                     run()

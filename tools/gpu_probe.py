@@ -128,11 +128,10 @@ def flow_case(name, mode):
                 y_vs_ref32=rel_err(y, arr["y32"]), y_vs_f64=rel_err(y, arr["y64"]), yref_vs_f64=rel_err(arr["y32"], arr["y64"]))
 
 
-def time_gemm(engine, M, N, K, bn, chunk, iters=10):
+def time_gemm(engine, M, N, K, bn, iters=10):
     dev = "cuda"
     lib = _lib.load()
     lib.usf_debug_set_block_n(bn)
-    lib.usf_set_accum_chunk(chunk)
     ld = ops.pad4(K)
     if engine == ops.ENGINE_TC_BF16:
         a = Act(M, K, bf16=torch.randn(M, ld, device=dev).to(torch.bfloat16)[:, :K])
@@ -158,7 +157,6 @@ def time_gemm(engine, M, N, K, bn, chunk, iters=10):
     e1.record()
     torch.cuda.synchronize()
     lib.usf_debug_set_block_n(0)
-    lib.usf_set_accum_chunk(2)
     ms = e0.elapsed_time(e1) / iters
     return round(2.0 * M * N * K / (ms * 1e-3) / 1e12, 1)
 
@@ -170,22 +168,11 @@ if "--perf" in sys.argv:
             out = {}
             for (M, N, K) in [(16384, 1024, 1024), (16384, 784, 784), (16384, 1024, 784), (16384, 784, 1024), (16384, 3072, 3072), (65536, 1024, 1024)]:
                 if eng == ops.ENGINE_SIMT:
-                    out[f"{M}x{N}x{K}"] = time_gemm(eng, M, N, K, 0, 0, iters=3)
+                    out[f"{M}x{N}x{K}"] = time_gemm(eng, M, N, K, 0, iters=3)
                     continue
                 for bn in ([256, 208, 128] if N != 1024 and N != 3072 else [256, 128]):
-                    for chunk in ([0, 1, 2, 4] if eng == ops.ENGINE_TC_3XTF32 else [0]):
-                        out[f"{M}x{N}x{K}_bn{bn}_c{chunk}"] = time_gemm(eng, M, N, K, bn, chunk)
+                    out[f"{M}x{N}x{K}_bn{bn}"] = time_gemm(eng, M, N, K, bn)
             return out
-
-if "--chunks" in sys.argv:
-    for chunk in [0, 1, 2, 4, 8]:
-        for name in ["c2_d784", "c4_d3072_b2", "d100_h50_hh"]:
-            def run(name=name, chunk=chunk):
-                _lib.load().usf_set_accum_chunk(chunk)
-                r = flow_case(name, "fp32")
-                _lib.load().usf_set_accum_chunk(2)
-                return {k: r[k] for k in ("lp_vs_ref32", "z_vs_ref32", "y_vs_ref32", "lp_vs_f64", "z_vs_f64")}
-            section(f"chunk{chunk}_{name}")(run)
 
 modes = ["fp32"] if "--fp32-only" in sys.argv else ["fp32_simt", "fp32", "tf32", "bf16"]
 for mode in modes:

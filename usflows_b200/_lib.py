@@ -143,8 +143,6 @@ SIGNATURES = {
     "usf_masked_add": (C.c_int, [_P, _I64, _P, _I64, _I64, _I32, _I32, _P, _F, _P]),
     "usf_pix_encode": (C.c_int, [_P, _I64, _I64, _I32, _I32, _P, _I32, _P, _P, _P]),
     "usf_conv2d_pix": (C.c_int, [C.POINTER(ConvPixArgs), _P]),
-    "usf_set_pix_chain_taps": (C.c_int, [_I32]),
-    "usf_set_pix_gate_at": (C.c_int, [_I32]),
     "usf_gate_norm": (C.c_int, [_P, _I64, _P, _I64, _I64, _I32, _I32, _I32, _P, _P, _F, _P, _I64, C.POINTER(Planes), _I32,
                                 C.POINTER(Planes), _P, _P]),
     "usf_leaky_relu": (C.c_int, [_P, _I64, _I64, _I32, _F, _P, _I64, _P, _P]),
@@ -179,10 +177,8 @@ SIGNATURES = {
     "usf_tri_mask": (C.c_int, [_P, _I64, _I32, _I32, _F, _P, _I64, _F, _P, _I64, _P]),
     "usf_tri_inverse_batched": (C.c_int, [_P, _P, _P, _I32, _I64, _I64, _I32, C.c_uint32, _P]),
     "usf_debug_set_block_n": (C.c_int, [C.c_int]),
-    "usf_set_accum_chunk": (C.c_int, [C.c_int]),
-    "usf_set_accum_lead": (C.c_int, [C.c_int]),
     "usf_debug_set_pdl": (C.c_int, [C.c_int]),
-    "usf_debug_gemm_timeline": (C.c_int, [_P, C.c_int]),
+    "usf_debug_set_store_path": (C.c_int, [C.c_int]),
 }
 
 
@@ -208,7 +204,7 @@ def load():
         fn = getattr(lib, name)  # AttributeError if the ABI and this table disagree
         fn.restype = res
         fn.argtypes = args
-    if lib.usf_abi_version() != 9:
+    if lib.usf_abi_version() != 10:
         raise RuntimeError("usflows_b200: ABI version mismatch between _lib.py and the shared library")
     _lib = lib
     return lib

@@ -14,8 +14,6 @@
 
 namespace usf {
 // csrc/conv_pix.cuh (compiled in conv_pix_inst.cu only: the kernel is not a template)
-extern int g_pix_chain_taps;
-extern int g_pix_gate_at;
 int launch_conv_pix(const usf_conv_pix_args* a, cudaStream_t st);
 int launch_pix_encode(const float* x, long long ldx, long long rows, int c, int hw, const float* mask, int relu, void* out16,
                       int* overflow_flag, cudaStream_t st);
@@ -25,14 +23,8 @@ namespace usf {
 
 thread_local char g_err[512] = "";
 int g_force_block_n = 0;
-int g_chunk_slabs = 2;
-int g_conv_chunk_slabs = 3;
-int g_lead_chains = 2;
-unsigned long long* g_dbg_buf = nullptr;
-int g_dbg_flags = 0;
-int g_no_fast_store = 0;
+int g_store_path = 0;
 int g_use_pdl = 1;
-int g_no_async_store = 0;
 
 int num_sms() {
   static int cached[64] = {0};
@@ -157,29 +149,14 @@ int usf_debug_set_block_n(int bn) {  // test hook: force the tcgen05 tile width 
   return USF_OK;
 }
 
-int usf_debug_gemm_timeline(unsigned long long* device_buf, int flags) {
-  g_dbg_buf = device_buf;
-  g_dbg_flags = flags & ~(4 | 32);
-  g_no_fast_store = (flags & 4) ? 1 : 0;
-  g_no_async_store = (flags & 32) ? 1 : 0;
+int usf_debug_set_store_path(int flags) {  // test hook: force the contraction's other store / residual paths (0 = automatic)
+  USF_REQUIRE((flags & ~(4 | 32 | 256)) == 0, "store path flags: 4, 32, 256 or a combination");
+  g_store_path = flags;
   return USF_OK;
 }
 
 int usf_debug_set_pdl(int on) {  // test hook: programmatic dependent launch of the kernel chain (default on)
   g_use_pdl = on ? 1 : 0;
-  return USF_OK;
-}
-
-int usf_set_accum_lead(int chains) {  // leading double-length accumulation chains per tile (MMA run-ahead); 0 = none
-  USF_REQUIRE(chains >= 0 && chains <= 2, "lead chains must be 0, 1 or 2 (two TMEM accumulators)");
-  g_lead_chains = chains;
-  return USF_OK;
-}
-
-int usf_set_accum_chunk(int k_slabs) {  // 3xTF32 mode: K-slabs (32 elements each) per accumulation chain; 0 = whole K
-  USF_REQUIRE(k_slabs >= 0, "negative chunk");
-  g_chunk_slabs = k_slabs;
-  g_conv_chunk_slabs = k_slabs;           // (defaults differ: 2 for the contractions, 3 for usf_conv2d_rows)
   return USF_OK;
 }
 
@@ -463,18 +440,6 @@ int usf_conv2d_pix(const usf_conv_pix_args* a, void* stream) {
   USF_REQUIRE(!a->out16 || aligned16(a->out16), "unaligned pixel planes");
   if (a->n_images == 0) return USF_OK;
   return launch_conv_pix(a, S(stream));
-}
-
-int usf_set_pix_chain_taps(int32_t taps) {
-  USF_REQUIRE(taps >= 0, "taps per chain (0 = default)");
-  g_pix_chain_taps = taps;
-  return USF_OK;
-}
-
-int usf_set_pix_gate_at(int32_t chains) {
-  USF_REQUIRE(chains >= 0, "negative");
-  g_pix_gate_at = chains;
-  return USF_OK;
 }
 
 int usf_masked_add(float* x, int64_t ldx, const float* t, int64_t ldt, int64_t rows, int32_t c, int32_t hw, const float* g,

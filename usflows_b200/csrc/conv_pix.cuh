@@ -52,7 +52,6 @@ struct PixArgs {
   const float* bias2;                   // gated: [64]
   int post_relu;
   int* overflow_flag;
-  int dbg;                              // tools/conv_probe.py: 64 = no activation loads, 128 = no MMAs, 256 = no global loads / stores in the epilogue
 };
 
 namespace convpix {
@@ -149,7 +148,7 @@ __device__ __forceinline__ Tile decode_tile(const PixArgs& p, long long tile) {
 // layout of the tensor core, so the same block is the warp's part of the gate's operand tile): the epilogue thread of
 // row `lane` writes / reads its 128 bytes there, and the warp moves the block to / from global memory with 512
 // contiguous bytes per instruction (a thread storing its own row directly touches 32 different 128-byte lines per
-// instruction: 5 700 cycles per tile for the two outputs, tools/conv_probe.py).
+// instruction: 5 700 cycles per tile for the two outputs, measured on a B200).
 __device__ __forceinline__ uint4 ld_shared_u4(uint32_t addr) {
   uint4 v;
   asm volatile("ld.shared.v4.b32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "r"(addr) : "memory");
@@ -255,9 +254,6 @@ __device__ __forceinline__ uint64_t desc64(uint32_t lo) {
   return d;
 }
 
-// DBG: the switches of tools/conv_probe.py (p.dbg: 64 = no activation loads, 128 = no MMAs, 256 = no global traffic in
-// the epilogue); the shipped instantiation has none of it.
-template <bool DBG>
 __global__ void __launch_bounds__(PIX_THREADS, 1)
 conv_pix_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_w1,
                 const __grid_constant__ CUtensorMap tm_w2, const PixArgs p) {
@@ -284,7 +280,6 @@ conv_pix_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int n_chains = (p.taps + p.chain_taps - 1) / p.chain_taps;
-  const bool no_loads = DBG && (p.dbg & 64), no_mma = DBG && (p.dbg & 128), no_traffic = DBG && (p.dbg & 256);
 
   if (warp == 0 && lane == 0) {
     prefetch_tmap(&tm_a);
@@ -313,7 +308,7 @@ conv_pix_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
   // memory (the producer -- weights included: they may come from the kernel just before --, the epilogue warps) waits first.
   griddep_launch_dependents();
 
-  // What the measurements decided (tools/conv_probe.py, DESIGN.md 4.3, profiles/r02_conv_pix_probe.log):
+  // What the measurements decided (DESIGN.md 4.3, profiles/r02_conv_pix_probe.log):
   //  * no setmaxnreg (640 threads x 96 registers; the 56 / 224 split of the flat kernels made the issuer re-load its
   //    descriptors from local memory in front of every tcgen05.mma; and setmaxnreg.inc can only take what .dec released
   //    inside the CTA's launch allocation);
@@ -339,13 +334,9 @@ conv_pix_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
           for (int ty = 0; ty < p.ksize; ++ty)
             for (int tx = 0; tx < p.ksize; ++tx) {
               mbar_wait(empty_bar(stage), phase ^ 1);
-              if (no_loads) {
-                mbar_arrive(full_bar(stage));
-              } else {
-                mbar_expect_tx(full_bar(stage), p.box_bytes);
-                tma_load_4d(smem_base + (uint32_t)stage * A_STAGE, &tm_a, full_bar(stage), 0, (tx - half) * p.dil,
-                            t.h0 + (ty - half) * p.dil, t.n0);
-              }
+              mbar_expect_tx(full_bar(stage), p.box_bytes);
+              tma_load_4d(smem_base + (uint32_t)stage * A_STAGE, &tm_a, full_bar(stage), 0, (tx - half) * p.dil,
+                          t.h0 + (ty - half) * p.dil, t.n0);
               if (++stage == p.stages) { stage = 0; phase ^= 1; }
             }
         }
@@ -369,14 +360,12 @@ conv_pix_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
         tcgen05_fence_after();
         const uint32_t da = desc_lo(a2_base + (uint32_t)mt * A_MT), db = desc_lo(w2_base);
         const uint32_t d = tmem_base + ACC2_COL + (uint32_t)mt * 64;
-        if (!no_mma) {
-          umma_f16(desc64(da + KOFF_LO), desc64(db), d, IDESC_N64, 0u);
-          umma_f16(desc64(da), desc64(db + KOFF_LO), d, IDESC_N64, 1u);
-          umma_f16(desc64(da + KOFF_LO + KOFF_K1), desc64(db + KOFF_K1), d, IDESC_N64, 1u);
-          umma_f16(desc64(da + KOFF_K1), desc64(db + KOFF_LO + KOFF_K1), d, IDESC_N64, 1u);
-          umma_f16_scale11(desc64(da), desc64(db), d, IDESC_N64);
-          umma_f16(desc64(da + KOFF_K1), desc64(db + KOFF_K1), d, IDESC_N64, 1u);
-        }
+        umma_f16(desc64(da + KOFF_LO), desc64(db), d, IDESC_N64, 0u);
+        umma_f16(desc64(da), desc64(db + KOFF_LO), d, IDESC_N64, 1u);
+        umma_f16(desc64(da + KOFF_LO + KOFF_K1), desc64(db + KOFF_K1), d, IDESC_N64, 1u);
+        umma_f16(desc64(da + KOFF_K1), desc64(db + KOFF_LO + KOFF_K1), d, IDESC_N64, 1u);
+        umma_f16_scale11(desc64(da), desc64(db), d, IDESC_N64);
+        umma_f16(desc64(da + KOFF_K1), desc64(db + KOFF_K1), d, IDESC_N64, 1u);
         umma_commit(acc2full_bar);
       };
       for (long long tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
@@ -395,22 +384,18 @@ conv_pix_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
           uint32_t ph = phase;
           for (int tap = tap0; tap < tap1; ++tap) {       // cross terms of the whole chain first (lo' is scaled by 2^11)
             mbar_wait(full_bar(st), ph);
-            if (!no_mma) {
-              const uint32_t da = a_lo0 + (uint32_t)st * (A_STAGE >> 4), db = w_lo0 + (uint32_t)tap * (W1_TAP >> 4);
-              umma_f16(desc64(da + KOFF_LO), desc64(db), d, IDESC_N32, tap > tap0 ? 1u : 0u);
-              umma_f16(desc64(da), desc64(db + KOFF_LO), d, IDESC_N32, 1u);
-              umma_f16(desc64(da + KOFF_LO + KOFF_K1), desc64(db + KOFF_K1), d, IDESC_N32, 1u);
-              umma_f16(desc64(da + KOFF_K1), desc64(db + KOFF_LO + KOFF_K1), d, IDESC_N32, 1u);
-            }
+            const uint32_t da = a_lo0 + (uint32_t)st * (A_STAGE >> 4), db = w_lo0 + (uint32_t)tap * (W1_TAP >> 4);
+            umma_f16(desc64(da + KOFF_LO), desc64(db), d, IDESC_N32, tap > tap0 ? 1u : 0u);
+            umma_f16(desc64(da), desc64(db + KOFF_LO), d, IDESC_N32, 1u);
+            umma_f16(desc64(da + KOFF_LO + KOFF_K1), desc64(db + KOFF_K1), d, IDESC_N32, 1u);
+            umma_f16(desc64(da + KOFF_K1), desc64(db + KOFF_LO + KOFF_K1), d, IDESC_N32, 1u);
             if (++st == p.stages) { st = 0; ph ^= 1; }
           }
           for (int tap = tap0; tap < tap1; ++tap) {       // hi.hi: the first one rescales the accumulator by 2^-11
-            if (!no_mma) {
-              const uint32_t da = a_lo0 + (uint32_t)stage * (A_STAGE >> 4), db = w_lo0 + (uint32_t)tap * (W1_TAP >> 4);
-              if (tap == tap0) umma_f16_scale11(desc64(da), desc64(db), d, IDESC_N32);
-              else umma_f16(desc64(da), desc64(db), d, IDESC_N32, 1u);
-              umma_f16(desc64(da + KOFF_K1), desc64(db + KOFF_K1), d, IDESC_N32, 1u);
-            }
+            const uint32_t da = a_lo0 + (uint32_t)stage * (A_STAGE >> 4), db = w_lo0 + (uint32_t)tap * (W1_TAP >> 4);
+            if (tap == tap0) umma_f16_scale11(desc64(da), desc64(db), d, IDESC_N32);
+            else umma_f16(desc64(da), desc64(db), d, IDESC_N32, 1u);
+            umma_f16(desc64(da + KOFF_K1), desc64(db + KOFF_K1), d, IDESC_N32, 1u);
             umma_commit(empty_bar(stage));
             if (tap == tap1 - 1) umma_commit(tfull_bar(acc));
             if (++stage == p.stages) { stage = 0; phase ^= 1; }
@@ -454,7 +439,7 @@ conv_pix_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
     // bytes per instruction): issued at the top of their own tile they queued behind the previous tile's stores and their
     // latency showed (the gated block: 166 -> 15x us).
     uint4 pre[4];
-    const bool pre_on = (p.gated || x_vec) && !no_traffic;
+    const bool pre_on = p.gated || x_vec;
     const uint8_t* pre_base = p.gated ? reinterpret_cast<const uint8_t*>(p.out_f32) : reinterpret_cast<const uint8_t*>(p.x);
     const long long pre_pitch = p.gated ? p.ld_f32 * 4 : p.ldx * 4;
     const int pre_nch = p.gated ? 8 : (p.c_x >> 2);
@@ -476,9 +461,9 @@ conv_pix_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
     prefetch(blockIdx.x);
     for (long long tile = blockIdx.x; tile < p.n_tiles; tile += gridDim.x) {
       const Tile tl = decode_tile(p, tile);
-      const bool valid = t < tl.nvalid && !no_traffic;
+      const bool valid = t < tl.nvalid;
       int wrows = tl.nvalid - wrow0;                                  // valid rows of the pair's block
-      wrows = no_traffic ? 0 : wrows < 0 ? 0 : wrows > 32 ? 32 : wrows;
+      wrows = wrows < 0 ? 0 : wrows > 32 ? 32 : wrows;
       const long long r = tl.row0 + t, wr = tl.row0 + wrow0;
       float m[16];
       for (int c = 0; c < n_chains; ++c) {
@@ -691,8 +676,6 @@ inline size_t conv_pix_smem_bytes(int taps, int gated) {
          (gated ? convpix::W2_BYTES : 0) + convpix::A_STAGE + 1024 + 6144;
 }
 
-extern int g_pix_gate_at;               // chains of the next tile issued in front of a tile's gate contraction
-extern int g_pix_chain_taps;            // taps per accumulation chain (0 = auto; 3 = 96 K-elements; 2 = the flat engine's chain length)
 int launch_conv_pix(const usf_conv_pix_args* a, cudaStream_t st);
 int launch_pix_encode(const float* x, long long ldx, long long rows, int c, int hw, const float* mask, int relu, void* out16,
                       int* overflow_flag, cudaStream_t st);

@@ -3,9 +3,11 @@
 
 namespace usf {
 
-int g_pix_chain_taps = 0;              // 0 = auto: 3 for the gated block, 2 for a plain convolution (measured, tools/conv_probe.py)
-int g_pix_gate_at = 1;
-extern int g_dbg_flags;
+// taps per TMEM accumulation chain: 3 (96 K-elements) in the gated block, 2 (the flat engine's chain length) in a plain
+// convolution (measured on a B200, DESIGN.md 4.3)
+constexpr int PIX_CHAIN_TAPS_GATED = 3, PIX_CHAIN_TAPS_PLAIN = 2;
+// gated block: chains of the next tile issued in front of a tile's 1 x 1 gate contraction
+constexpr int PIX_GATE_AT = 1;
 
 static int make_pix_map(CUtensorMap* map, const void* ptr, long long n_images, int H, int W, int hr, int imgs) {
   PFN_encodeTiled enc = get_encode_tiled();
@@ -42,10 +44,10 @@ int launch_conv_pix(const usf_conv_pix_args* a, cudaStream_t st) {
   p.imgs = imgs; p.hr = hr; p.tiles_per_img = tpi;
   p.n_tiles = tpi == 1 ? (a->n_images + imgs - 1) / imgs : a->n_images * (long long)tpi;
   p.stages = stages;
-  p.chain_taps = g_pix_chain_taps < 1 ? (a->gated ? 3 : 2) : g_pix_chain_taps;
+  p.chain_taps = a->gated ? PIX_CHAIN_TAPS_GATED : PIX_CHAIN_TAPS_PLAIN;
   if (p.chain_taps > stages - 1) p.chain_taps = stages - 1;   // a chain holds its stages until its last product is issued
   if (p.chain_taps > taps) p.chain_taps = taps;
-  p.gate_at = g_pix_gate_at;
+  p.gate_at = PIX_GATE_AT;
   p.box_bytes = (unsigned)(convpix::PIX_BYTES * a->w * hr * imgs);
   p.gated = a->gated ? 1 : 0;
   p.bias1 = a->bias1; p.n1 = a->n1; p.relu1 = a->relu1;
@@ -55,12 +57,11 @@ int launch_conv_pix(const usf_conv_pix_args* a, cudaStream_t st) {
   p.x = a->x; p.ldx = a->ldx; p.inv_mask = a->inv_mask; p.sign = a->sign; p.c_x = a->c_x;
   p.bias2 = a->bias2; p.post_relu = a->post_relu;
   p.overflow_flag = a->overflow_flag;
-  p.dbg = g_dbg_flags;
 
-  auto kern = p.dbg ? convpix::conv_pix_kernel<true> : convpix::conv_pix_kernel<false>;
+  auto kern = convpix::conv_pix_kernel;
   const size_t smem = conv_pix_smem_bytes(taps, p.gated);
-  static size_t attr_bytes_dev[2][MAX_DEVICES] = {{0}};
-  size_t& attr_bytes = attr_bytes_dev[p.dbg ? 1 : 0][current_device_slot()];
+  static size_t attr_bytes_dev[MAX_DEVICES] = {0};
+  size_t& attr_bytes = attr_bytes_dev[current_device_slot()];
   if (smem > attr_bytes) {
     USF_CUDA_OK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     attr_bytes = smem;

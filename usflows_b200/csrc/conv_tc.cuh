@@ -44,7 +44,7 @@ template <int BLOCK_N>
 __global__ void __launch_bounds__(conv_threads(BLOCK_N), 1)
 conv_tc_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_w_lo,
                const float* __restrict__ act, long long ld_act, long long M, int H, int W, int Cin, int ksize, int dil,
-               const float* __restrict__ mask, int relu_in, int N, int K, int chunk_slabs, Epilogue ep, int dbg, int A_STAGES) {
+               const float* __restrict__ mask, int relu_in, int N, int K, int chunk_slabs, Epilogue ep, int A_STAGES) {
   using C = Config<BLOCK_N, 3, false>;
   constexpr int B_SLAB = BLOCK_N * SLAB_BYTES;      // one K-slab of one weight plane (multiple of 1024 B)
   constexpr int CONV_EPI_WARPS = conv_epi_warps(BLOCK_N), GATHER_TPR = conv_gather_tpr(BLOCK_N);
@@ -114,7 +114,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__
           if (lane == 0) {
             const uint32_t sa = smem_base + stage * A_STAGE_BYTES;
             const uint32_t sb = w_base + (uint32_t)ks * 2u * B_SLAB;
-            if (!(dbg & 128)) {
             const uint64_t da_hi = make_smem_desc(sa), da_lo = make_smem_desc(sa + A_TILE);
             const uint64_t db_hi = make_smem_desc(sb), db_lo = make_smem_desc(sb + B_SLAB);
 #pragma unroll
@@ -127,7 +126,6 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__
             for (int k = 0; k < SLAB_BYTES / UMMA_K_BYTES; ++k) {
               const uint64_t koff = (uint64_t)((k * UMMA_K_BYTES) >> 4);
               umma<false>(da_hi + koff, db_hi + koff, tmem_d, C::IDESC, 1u);
-            }
             }
             umma_commit(empty_bar(stage));
             if (ks == ks1 - 1) umma_commit(tfull_bar(acc));
@@ -180,24 +178,22 @@ conv_tc_kernel(const __grid_constant__ CUtensorMap tm_w, const __grid_constant__
     auto load_item = [&](const Item& it, float4 (&v)[CPT]) {
 #pragma unroll
       for (int j = 0; j < CPT; ++j)
-        v[j] = (it.src && !(dbg & 64)) ? *reinterpret_cast<const float4*>(it.src + 4 * j) : make_float4(0.f, 0.f, 0.f, 0.f);
+        v[j] = it.src ? *reinterpret_cast<const float4*>(it.src + 4 * j) : make_float4(0.f, 0.f, 0.f, 0.f);
     };
     auto store_item = [&](const Item& it, const float4 (&src)[CPT]) {
       mbar_wait(empty_bar(stage), phase ^ 1);
       const uint32_t sa = smem_base + stage * A_STAGE_BYTES + row_off;
-      if (!(dbg & 64)) {
 #pragma unroll
-        for (int j = 0; j < CPT; ++j) {
-          float4 v = src[j];
-          if (it.msk) {                                        // tiny (H*W*C floats): L1 resident
-            const float4 m = __ldg(reinterpret_cast<const float4*>(it.msk + 4 * j));
-            v.x *= m.x; v.y *= m.y; v.z *= m.z; v.w *= m.w;
-          }
-          if (relu_in) { v.x = fmaxf(v.x, 0.f); v.y = fmaxf(v.y, 0.f); v.z = fmaxf(v.z, 0.f); v.w = fmaxf(v.w, 0.f); }
-          const float hx = tf32_round(v.x), hy = tf32_round(v.y), hz = tf32_round(v.z), hw_ = tf32_round(v.w);
-          st_shared_v4(sa + col[j], hx, hy, hz, hw_);
-          st_shared_v4(sa + A_TILE + col[j], tf32_round(v.x - hx), tf32_round(v.y - hy), tf32_round(v.z - hz), tf32_round(v.w - hw_));
+      for (int j = 0; j < CPT; ++j) {
+        float4 v = src[j];
+        if (it.msk) {                                        // tiny (H*W*C floats): L1 resident
+          const float4 m = __ldg(reinterpret_cast<const float4*>(it.msk + 4 * j));
+          v.x *= m.x; v.y *= m.y; v.z *= m.z; v.w *= m.w;
         }
+        if (relu_in) { v.x = fmaxf(v.x, 0.f); v.y = fmaxf(v.y, 0.f); v.z = fmaxf(v.z, 0.f); v.w = fmaxf(v.w, 0.f); }
+        const float hx = tf32_round(v.x), hy = tf32_round(v.y), hz = tf32_round(v.z), hw_ = tf32_round(v.w);
+        st_shared_v4(sa + col[j], hx, hy, hz, hw_);
+        st_shared_v4(sa + A_TILE + col[j], tf32_round(v.x - hx), tf32_round(v.y - hy), tf32_round(v.z - hz), tf32_round(v.w - hw_));
       }
       fence_proxy_async();                 // generic-proxy stores -> visible to the tensor core's async-proxy reads
       __syncwarp();
@@ -260,7 +256,7 @@ struct ConvGeom {
   int relu_in;
 };
 
-// A stages: measured on the 32 -> 32 channel 3x3 convolution (tools/conv_probe.py): 3 stages 388 us, 4 stages 427 us
+// A stages: measured on the 32 -> 32 channel 3x3 convolution (B200): 3 stages 388 us, 4 stages 427 us
 // (the per-slab hand-over, not the pipeline depth, bounds the kernel), so 3 it is.  0 = the shape does not fit.
 inline int conv_tc_stages(int block_n, int K) {
   const long long w = (long long)((K + 31) / 32) * 2 * block_n * tc::SLAB_BYTES;
@@ -270,11 +266,10 @@ inline size_t conv_tc_smem_bytes(int block_n, int K) {
   return (size_t)conv_tc_stages(block_n, K) * convtc::A_STAGE_BYTES + (size_t)((K + 31) / 32) * 2 * block_n * tc::SLAB_BYTES + 1024 + 256;
 }
 
-extern int g_dbg_flags;
 // K-slabs (32 tf32 elements each) per TMEM accumulation chain of the convolution: 3 = 96 elements per chain (the chain
 // hand-over is what bounds the kernel: 388 us at 2, 363 us at 3, 356 us at 9 slabs for the 3x3 32->32 convolution; the
 // truncation bias of a 96-element chain is ~5e-7 relative, measured 5e-6 at 1024 elements)
-extern int g_conv_chunk_slabs;
+constexpr int CONV_CHUNK_SLABS = 3;
 template <int BLOCK_N>
 int launch_conv_tc_cfg(const usf_linear_args* a, const ConvGeom& g, const Epilogue& ep, cudaStream_t st) {
   auto kern = convtc::conv_tc_kernel<BLOCK_N>;
@@ -292,12 +287,11 @@ int launch_conv_tc_cfg(const usf_linear_args* a, const ConvGeom& g, const Epilog
   const long long tiles = (a->M + tc::BLOCK_M - 1) / tc::BLOCK_M;
   const int grid = (int)(tiles < num_sms() ? tiles : num_sms());
   kern<<<grid, convtc::conv_threads(BLOCK_N), smem, st>>>(mw, mwl, g.act, g.ld_act, a->M, g.H, g.W, g.Cin, g.ksize, g.dil, g.mask,
-                                                 g.relu_in, a->N, a->K, g_conv_chunk_slabs, ep, g_dbg_flags, conv_tc_stages(BLOCK_N, a->K));
+                                                 g.relu_in, a->N, a->K, CONV_CHUNK_SLABS, ep, conv_tc_stages(BLOCK_N, a->K));
   USF_CUDA_OK(cudaGetLastError());
   return USF_OK;
 }
 
-extern int g_dbg_flags;                 // debug (tools/conv_probe.py): 64 = gather skips loads / stores, 128 = no MMAs
 int launch_conv_tc(const usf_linear_args* a, const ConvGeom& g, const Epilogue& ep, cudaStream_t st);
 
 }  // namespace usf

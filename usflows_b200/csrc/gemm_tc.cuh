@@ -69,7 +69,7 @@ __device__ __forceinline__ bool mbar_test_wait(uint32_t bar, uint32_t parity) {
 }
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
   // fast path: the non-blocking test costs ~16 cycles on a completed phase, the (potentially suspending) try_wait ~180
-  // even when the phase is already complete (measured in-kernel, tools/conv_probe.py) -- and in a full pipeline most
+  // even when the phase is already complete (measured in-kernel on a B200) -- and in a full pipeline most
   // waits find their phase complete
   if (mbar_test_wait(bar, parity)) return;
 #if USF_WATCHDOG
@@ -246,7 +246,6 @@ __device__ __forceinline__ void epilogue_loop(int col0, int quarter, int lane, u
 }  // namespace tc
 
 // host side ---------------------------------------------------------------------------------------
-extern int g_chunk_slabs;  // K-slabs per TMEM accumulation chain in the 3xTF32 mode (usf_set_accum_chunk)
 typedef CUresult (*PFN_encodeTiled)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                     const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
                                     CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);

@@ -104,7 +104,6 @@ __device__ __forceinline__ TileCoord decode_tile(long long tile, int n_blocks, i
   return t;
 }
 
-constexpr int DBG_CHAINS = 512;   // timeline slots of a debug launch (usf_debug_gemm_timeline): 8 clock64 values each
 constexpr int KIND_TF32 = 0, KIND_BF16 = 1, KIND_F16 = 2;   // KIND_F16: fp16 split planes (x = hi + lo' 2^-11)
 
 // D = A.B + D * 2^-11 (kind::f16 with scale-input-d): folds the scaled-up cross terms of the fp16 split into the
@@ -234,7 +233,7 @@ __device__ __forceinline__ void stage_copy_out(uint32_t stage, int lane, uint8_t
 
 // The epilogue description, read ONCE per thread into registers.  Reading the fields from the kernel-parameter
 // constant bank where they are used costs a dependent constant load + compare + branch per feature and per group of
-// columns (~10^3 cycles per 32-column piece, measured with the clock64 timeline) -- the pieces must run on registers.
+// columns (~10^3 cycles per 32-column piece, measured with an in-kernel cycle-counter timeline) -- the pieces must run on registers.
 struct EpiRegs {
   uint32_t flags;
   float sign;
@@ -287,12 +286,9 @@ __device__ __forceinline__ EpiRegs load_epi_regs(const Epilogue& ep) {
 
 template <int W>
 __device__ __forceinline__ void store_chunk(const Epilogue& ep, const EpiRegs& er, float (&v)[W], long long row0, int lane,
-                                            long long M, int n0, int N, uint32_t stage, int dbg_flags,
-                                            unsigned long long* dbg_slot = nullptr) {
+                                            long long M, int n0, int N, uint32_t stage, int path_flags) {
   const long long m = row0 + lane;
   const uint32_t f = er.flags;
-  long long t0 = 0, t1 = 0, t2 = 0;
-  if (dbg_slot) t0 = clock64();
   if (m < M) {
     if (f & EF_RARE) {        // column scale / post-subtract / fp32 residual planes: the generic arithmetic
 #pragma unroll
@@ -357,13 +353,12 @@ __device__ __forceinline__ void store_chunk(const Epilogue& ep, const EpiRegs& e
       }
     }
   }
-  if (dbg_slot) t1 = clock64();
   if (f & EF_OUT16) {      // fp16 split planes: x = hi + lo' 2^-11
     constexpr int RB = W * 2;
     const uint32_t stage_lo = stage + 32 * RB;
     // debug flag 16: register-direct stores.  Unused, but deleting it shifts ptxas' register allocation and slowed the
     // BLOCK_N = 256 3xTF32 instantiation by 2% (1024 x 1024 over 65 536 rows, B200)
-    const bool direct = (dbg_flags & 16) != 0;
+    const bool direct = (path_flags & 16) != 0;
     uint4* gh = reinterpret_cast<uint4*>(er.oh + m * er.ld16 + n0);
     uint4* gl = reinterpret_cast<uint4*>(er.ol + m * er.ld16 + n0);
     __half2 amax2 = __float2half2_rn(0.f);      // running max |hi| (NaN-propagating): inf / NaN = the value left the fp16 range
@@ -394,17 +389,11 @@ __device__ __forceinline__ void store_chunk(const Epilogue& ep, const EpiRegs& e
       const float2 am = __half22float2(amax2);
       if (!(am.x <= F16_GUARD && am.y <= F16_GUARD) && m < M && ep.overflow_flag) *ep.overflow_flag = 1;
     }
-    if (dbg_slot) t2 = clock64();
     if (!direct) {
       __syncwarp();
       stage_copy_out<RB>(stage, lane, reinterpret_cast<uint8_t*>(er.oh), (long long)er.ld16 * 2, row0, M, n0 * 2, N * 2);
       stage_copy_out<RB>(stage_lo, lane, reinterpret_cast<uint8_t*>(er.ol), (long long)er.ld16 * 2, row0, M, n0 * 2, N * 2);
       __syncwarp();
-    }
-    if (dbg_slot) {
-      const long long t3 = clock64();
-      dbg_slot[6] += ((unsigned long long)(t1 - t0) << 32) | (unsigned long long)(t2 - t1);
-      dbg_slot[7] += (unsigned long long)(t3 - t2);
     }
   }
   if (f & EF_OUTF32) {
@@ -712,21 +701,19 @@ template <class C, int COLS, bool SPLITK>
 __device__ __forceinline__ void epilogue_loop(int col0, int quarter, int lane, uint32_t rank, uint32_t tmem_base,
                                               uint32_t tfull0, uint32_t tempty0_leader, uint8_t* stage_gen,
                                               uint32_t stage, long long n_tiles, int n_blocks, int k_slabs, int split_k, int split_per, int chunk_slabs, int lead,
-                                              long long M, int N, const Epilogue& ep, unsigned long long* dbg, int dbg_flags,
-                                              const StoreMaps& smaps) {
+                                              long long M, int N, const Epilogue& ep, int path_flags, const StoreMaps& smaps) {
   constexpr int BLOCK_N = C::kBlockN;
   int acc = 0;
   uint32_t acc_phase = 0;
   int n_chunks = chain_count(k_slabs, chunk_slabs, lead);   // (split_k == 1; recomputed per work item otherwise)
-  int dbg_chain = 0;   // timeline slot (debug launches only: dbg != nullptr on one warp of cluster 0's leader)
   float* patch = reinterpret_cast<float*>(stage_gen);
   // everything the tile loop needs lives in registers from here on (opaque to the compiler): re-deriving these from
   // special registers / the parameter bank inside the loop costs a dependent S2R / LDC per use
   asm volatile("" : "+r"(stage), "+r"(tfull0), "+r"(tempty0_leader), "+r"(tmem_base));
-  // the warp's in-box sits right behind its staging boxes (no register of its own); debug flag 256 switches it off
-  const uint32_t inbox = (C::INBOX && !(dbg_flags & 256)) ? stage + STAGE_EPI_BYTES : 0u;
+  // the warp's in-box sits right behind its staging boxes (no register of its own); path flag 256 switches it off
+  const uint32_t inbox = (C::INBOX && !(path_flags & 256)) ? stage + STAGE_EPI_BYTES : 0u;
   asm volatile("" : "+l"(M), "+r"(N), "+r"(lane), "+r"(quarter), "+r"(col0), "+r"(rank), "+r"(n_blocks), "+l"(n_tiles),
-               "+r"(n_chunks), "+r"(dbg_flags));
+               "+r"(n_chunks), "+r"(path_flags));
   const EpiRegs er = load_epi_regs(ep);
   const bool fast_store = ep.fast_store != 0;
   const bool async_store = ep.async_store != 0;
@@ -765,44 +752,37 @@ __device__ __forceinline__ void epilogue_loop(int col0, int quarter, int lane, u
       }
       mbar_wait(tfull0 + 8u * acc, acc_phase);
       tcgen05_fence_after();
-      if (dbg && dbg_chain < DBG_CHAINS) dbg[dbg_chain * 8 + 3] = clock64();
       const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + acc * C::ACC_STRIDE + col0;
-      if (!(dbg_flags & 1)) {
 #pragma unroll
-        for (int j = 0; j + 32 <= COLS; j += 32) {
-          if (n_idx + col0 + j < N) {      // columns past N hold no MMA result (the last tile of a row may be narrower)
-            float v[32];
-            tmem_ld32(taddr + j, v);
-            tmem_ld_wait();
+      for (int j = 0; j + 32 <= COLS; j += 32) {
+        if (n_idx + col0 + j < N) {      // columns past N hold no MMA result (the last tile of a row may be narrower)
+          float v[32];
+          tmem_ld32(taddr + j, v);
+          tmem_ld_wait();
 #pragma unroll
-            for (int i = 0; i < 32; ++i) master[j + i] += v[i];
-          }
+          for (int i = 0; i < 32; ++i) master[j + i] += v[i];
         }
-        if (COLS % 32) {
-          constexpr int j = COLS / 32 * 32;
-          if (n_idx + col0 + j < N) {
-            float v[16];
-            tmem_ld16(taddr + j, v);
-            tmem_ld_wait();
+      }
+      if (COLS % 32) {
+        constexpr int j = COLS / 32 * 32;
+        if (n_idx + col0 + j < N) {
+          float v[16];
+          tmem_ld16(taddr + j, v);
+          tmem_ld_wait();
 #pragma unroll
-            for (int i = 0; i < 16; ++i) master[j + i] += v[i];
-          }
+          for (int i = 0; i < 16; ++i) master[j + i] += v[i];
         }
       }
       tcgen05_fence_before();
       __syncwarp();
-      if (dbg && dbg_chain < DBG_CHAINS) dbg[dbg_chain * 8 + 4] = clock64();
       if (lane == 0) mbar_arrive_cluster(tempty0_leader + 8u * acc);
       if (++acc == 2) { acc = 0; acc_phase ^= 1; }
-      ++dbg_chain;
     }
-    if (dbg_flags & 2) continue;   // debug: no store phase
     const long long row0 = m_idx + quarter * 32;
     if (async_store) {
       if (row0 < M) {
         const long long m = row0 + lane;
         const bool row_ok = m < M;
-        const long long t_start = dbg ? clock64() : 0;
 #pragma unroll
         for (int c = 0; c < COLS / 32; ++c) {
           const int n0 = n_idx + col0 + c * 32;
@@ -827,7 +807,6 @@ __device__ __forceinline__ void epilogue_loop(int col0, int quarter, int lane, u
                               n0, N, row0, stage, hand, M, inbox);
           }
         }
-        if (dbg && dbg_chain - 1 < DBG_CHAINS) dbg[(dbg_chain - 1) * 8 + 6] = (unsigned long long)(clock64() - t_start) << 32;
       }
     } else if (fast_store) {
       if (row0 < M) {
@@ -835,12 +814,11 @@ __device__ __forceinline__ void epilogue_loop(int col0, int quarter, int lane, u
         for (int c = 0; c < COLS / 32; ++c) {
           const int n0 = n_idx + col0 + c * 32;
           if (n0 < N)
-            store_chunk<32>(ep, er, *reinterpret_cast<float(*)[32]>(&master[c * 32]), row0, lane, M, n0, N, stage, dbg_flags,
-                            (dbg && dbg_chain - 1 < DBG_CHAINS) ? dbg + (dbg_chain - 1) * 8 : nullptr);
+            store_chunk<32>(ep, er, *reinterpret_cast<float(*)[32]>(&master[c * 32]), row0, lane, M, n0, N, stage, path_flags);
         }
         if (COLS % 32) {
           const int n0 = n_idx + col0 + COLS / 32 * 32;
-          if (n0 < N) store_chunk<16>(ep, er, *reinterpret_cast<float(*)[16]>(&master[COLS / 32 * 32]), row0, lane, M, n0, N, stage, dbg_flags);
+          if (n0 < N) store_chunk<16>(ep, er, *reinterpret_cast<float(*)[16]>(&master[COLS / 32 * 32]), row0, lane, M, n0, N, stage, path_flags);
         }
       }
     } else {
@@ -872,7 +850,6 @@ __device__ __forceinline__ void epilogue_loop(int col0, int quarter, int lane, u
         __syncwarp();
       }
     }
-    if (dbg && dbg_chain - 1 < DBG_CHAINS) dbg[(dbg_chain - 1) * 8 + 5] = clock64();
   }
   if (async_store && lane == 0) bulk_wait0();   // staging memory and the stores outlive their reads / writes
   __syncwarp();
@@ -883,8 +860,7 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
 gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_a_lo,
                 const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_w_lo,
                 long long M, int N, int K, int chunk_slabs, int lead_chains, int split_k, int split_per,
-                const __grid_constant__ Epilogue ep, const __grid_constant__ StoreMaps smaps, unsigned long long* dbg_buf,
-                int dbg_flags) {
+                const __grid_constant__ Epilogue ep, const __grid_constant__ StoreMaps smaps, int path_flags) {
   using C = Config<BLOCK_N, NTERMS, KIND>;
   extern __shared__ uint8_t smem_raw[];
   uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;   // same offset in both CTAs of the pair
@@ -982,8 +958,6 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
       uint32_t phase = 0;
       int acc = 0;
       uint32_t acc_phase = 0;
-      int dbg_chain = 0;
-      unsigned long long* dbg_mma = cluster_id_x() == 0 ? dbg_buf : nullptr;
       for (long long tile = cluster_id_x(); tile < n_tiles; tile += num_clusters_x()) {
         const TileCoord tc = decode_tile<SPLITK>(tile, n_blocks, split_k, k_slabs, split_per);
         const uint32_t idesc = C::IDESC_NO_N | ((uint32_t)(tile_width(tc.n_blk * BLOCK_N) >> 3) << 17);
@@ -995,7 +969,6 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
           const int ks1 = ks0 + span < tc.nks ? ks0 + span : tc.nks;
           mbar_wait(tempty_bar(acc), acc_phase ^ 1);  // both CTAs' epilogues have drained this accumulator
           tcgen05_fence_after();
-          if (dbg_mma && dbg_chain < DBG_CHAINS) dbg_mma[dbg_chain * 8 + 0] = clock64();
           const uint32_t tmem_d = tmem_base + acc * C::ACC_STRIDE;
           constexpr int KSTEPS = SLAB_BYTES / UMMA_K_BYTES;
           if (NTERMS == 3 && KIND == KIND_F16) {
@@ -1024,7 +997,6 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
               }
               if (++st == C::STAGES) { st = 0; ph ^= 1; }
             }
-            if (dbg_mma && dbg_chain < DBG_CHAINS) dbg_mma[dbg_chain * 8 + 1] = clock64();
             for (int ks = ks0; ks < ks1; ++ks) {
               {
                 const uint32_t sa = smem_base + stage * C::STAGE_BYTES;
@@ -1048,7 +1020,6 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
             for (int ks = ks0; ks < ks1; ++ks) {
               mbar_wait(full_bar(stage), phase);
               tcgen05_fence_after();
-              if (dbg_mma && dbg_chain < DBG_CHAINS) dbg_mma[dbg_chain * 8 + 1] = clock64();
               {
                 const uint32_t sa = smem_base + stage * C::STAGE_BYTES;
                 const uint32_t sb = sa + C::NPLANES * C::A_TILE;
@@ -1079,8 +1050,6 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
             }
           }
           ks0 = ks1;
-          if (dbg_mma && dbg_chain < DBG_CHAINS) dbg_mma[dbg_chain * 8 + 2] = clock64();
-          ++dbg_chain;
           if (++acc == 2) { acc = 0; acc_phase ^= 1; }
         }
       }
@@ -1092,16 +1061,15 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
     uint8_t* stage = smem_gen + (stage_u32 - smem_base);
 
     const uint32_t tempty_leader = mapa(tempty_bar(0), 0);
-    unsigned long long* dbg_epi = (cluster_id_x() == 0 && rank == 0 && warp == FIRST_EPI_WARP && lane == 0) ? dbg_buf : nullptr;
     if (C::HALF0 == C::HALF1)     // one copy of the epilogue code serves both column halves
       epilogue_loop<C, C::HALF0, SPLITK>(warp < FIRST_EPI_WARP + 4 ? 0 : C::HALF0, warp & 3, lane, rank, tmem_base, tfull_bar(0),
-                                 tempty_leader, stage, stage_u32, n_tiles, n_blocks, k_slabs, split_k, split_per, chunk_slabs, lead_chains, M, N, ep, dbg_epi, dbg_flags, smaps);
+                                 tempty_leader, stage, stage_u32, n_tiles, n_blocks, k_slabs, split_k, split_per, chunk_slabs, lead_chains, M, N, ep, path_flags, smaps);
     else if (warp < FIRST_EPI_WARP + 4)
       epilogue_loop<C, C::HALF0, SPLITK>(0, warp & 3, lane, rank, tmem_base, tfull_bar(0), tempty_leader, stage, stage_u32, n_tiles,
-                                 n_blocks, k_slabs, split_k, split_per, chunk_slabs, lead_chains, M, N, ep, dbg_epi, dbg_flags, smaps);
+                                 n_blocks, k_slabs, split_k, split_per, chunk_slabs, lead_chains, M, N, ep, path_flags, smaps);
     else
       epilogue_loop<C, C::HALF1, SPLITK>(C::HALF0, warp & 3, lane, rank, tmem_base, tfull_bar(0), tempty_leader, stage, stage_u32,
-                                 n_tiles, n_blocks, k_slabs, split_k, split_per, chunk_slabs, lead_chains, M, N, ep, nullptr, dbg_flags, smaps);
+                                 n_tiles, n_blocks, k_slabs, split_k, split_per, chunk_slabs, lead_chains, M, N, ep, path_flags, smaps);
   }
 
   tcgen05_fence_before();
@@ -1115,11 +1083,19 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant_
 }  // namespace tc2
 
 // host side ---------------------------------------------------------------------------------------
-extern unsigned long long* g_dbg_buf;   // debug timeline buffer (usf_debug_gemm_timeline), normally null
-extern int g_lead_chains;               // leading double-length accumulation chains per tile (usf_set_accum_lead)
-extern int g_dbg_flags;                 // debug: 1 = epilogue skips the TMEM drain, 2 = no store phase
-extern int g_no_async_store;            // test hook: 1 = the epilogue warps store themselves (flag 32)
-extern int g_no_fast_store;             // test hook: 1 = always use the register/patch store path (usf_debug_gemm_timeline flag 4)
+// test hook (usf_debug_set_store_path): 4 = always the register/patch store path, 32 = the epilogue warps store their
+// staged boxes themselves (no TMA stores), 256 = the kernel reads the coupling residual lane-per-row (no in-box)
+extern int g_store_path;
+
+// 3xTF32 engine: K-slabs (32 elements each) accumulated in TMEM before the partial tile is added into fp32 registers with
+// round-to-nearest (the tensor core truncates when it accumulates: long chains carry a systematic toward-zero bias).  The
+// fp16-split engine closes a chain every slab (the kernel's rule); the single-pass engines accumulate the whole K.
+constexpr int CHUNK_SLABS = 2;
+// fp16-split engine: the first LEAD_CHAINS accumulation chains of every tile span twice the K-slabs, so the tensor core keeps
+// running on the next tile while the epilogue warps still store the previous one (two TMEM accumulators = two chains of
+// run-ahead).  Not for 3xTF32: its chains already hold 48 MMA steps, and the toward-zero bias of longer chains shows in
+// the gradients.
+constexpr int LEAD_CHAINS = 2;
 
 // fp16 output plane [rows, cols] (row pitch ld halves) for the TMA store path: box = 32 rows x box_cols (32: 64B swizzle,
 // 16: 32B swizzle) columns
@@ -1190,12 +1166,12 @@ int launch_gemm_tc2_cfg(const usf_linear_args* a, const Epilogue& ep_in, cudaStr
   // aligned output planes (16-byte aligned, pitch a 16-byte multiple, N a multiple of 8) leave through the staged,
   // coalesced store path; anything else through the generic register/patch path
   Epilogue ep = ep_in;
-  ep.fast_store = (ep.vec_ok && a->N % 8 == 0 && !g_no_fast_store) ? 1 : 0;
-  ep.async_store = (ep.fast_store && !g_no_async_store && ep.out_h16 && !ep.out_f32 && !ep.out_hi && !ep.out_bf16 &&
+  ep.fast_store = (ep.vec_ok && a->N % 8 == 0 && !(g_store_path & 4)) ? 1 : 0;
+  ep.async_store = (ep.fast_store && !(g_store_path & 32) && ep.out_h16 && !ep.out_f32 && !ep.out_hi && !ep.out_bf16 &&
                     !ep.colscale && !ep.postsub && !ep.resid_hi) ? 1 : 0;
   // mode 2: bf16 and / or fp32 planes (bf16 / tf32 precision modes), fp32 residual allowed
-  if (!ep.async_store && ep.fast_store && !g_no_async_store && !ep.out_h16 && !ep.out_hi && (ep.out_bf16 || ep.out_f32) &&
-      !ep.colscale && !ep.postsub && !ep.resid_h16 && !(SPLITK && a->split_k > 1) && !g_dbg_buf)
+  if (!ep.async_store && ep.fast_store && !(g_store_path & 32) && !ep.out_h16 && !ep.out_hi && (ep.out_bf16 || ep.out_f32) &&
+      !ep.colscale && !ep.postsub && !ep.resid_h16 && !(SPLITK && a->split_k > 1))
     ep.async_store = 2;
   tc2::StoreMaps sm;
   memset(&sm, 0, sizeof(sm));
@@ -1228,9 +1204,8 @@ int launch_gemm_tc2_cfg(const usf_linear_args* a, const Epilogue& ep_in, cudaStr
   const int pairs = num_sms() / 2;
   const int grid = 2 * (int)(tiles < pairs ? tiles : pairs);
   USF_CUDA_OK(launch_chain(kern, dim3(grid), dim3(tc::NUM_THREADS), (size_t)C::SMEM_BYTES, st, ma, mal, mw, mwl, (long long)a->M,
-                           (int)a->N, (int)a->K, NTERMS == 3 ? g_chunk_slabs : 0,
-                           (NTERMS == 3 && KIND == tc2::KIND_F16) ? g_lead_chains : 0, split_k, split_per, ep, sm, g_dbg_buf,
-                           g_dbg_flags));
+                           (int)a->N, (int)a->K, NTERMS == 3 ? CHUNK_SLABS : 0,
+                           (NTERMS == 3 && KIND == tc2::KIND_F16) ? LEAD_CHAINS : 0, split_k, split_per, ep, sm, g_store_path));
   return USF_OK;
 }
 
