@@ -219,6 +219,28 @@ int usf_base_sample(int64_t rows, int32_t d, const float* loc, const float* scal
                     uint64_t seed, uint64_t offset, float* out_f32, int64_t ld_f32, float* out_hi,
                     float* out_lo, int64_t ld_split, void* out_bf16, int64_t ld_bf16, void* stream);
 
+/* Philox key and counter base of one sampling call (usf_base_sample_at / usf_radial_sample_at).  Every counter that the
+ * plain entries key by the row index r within the call is keyed by the GLOBAL row row0 + r instead: counter
+ * ((row0 + r) * ceil(d / 4) + g, offset) for the 4-column group g of the coordinates, and (row0 + r, offset ^ tag [+ k]) for
+ * the radius, mixture component, rejection rounds and extremal coordinate of the radial sampler.  Rows [r0, r1) of one call
+ * therefore equal a call over r1 - r0 rows with row0 = r0, and usf_base_sample / usf_radial_sample are the row0 = 0 calls.
+ * When dev_params (device memory, 2 x int64) is given, the kernel reads {seed, row base} there at run time: seed is
+ * replaced, row base is added to row0 (a captured graph can then be replayed for the next chunk). */
+typedef struct usf_draw {
+  uint64_t seed;
+  uint64_t offset;
+  int64_t row0;
+  const int64_t* dev_params;
+} usf_draw;
+/* usf_base_sample with the draws of global rows draw->row0 .. draw->row0 + rows - 1 (row0 >= 0) */
+int usf_base_sample_at(int64_t rows, int32_t d, const float* loc, const float* scale, int32_t base_kind,
+                       const usf_draw* draw, float* out_f32, int64_t ld_f32, float* out_hi, float* out_lo,
+                       int64_t ld_split, void* out_bf16, int64_t ld_bf16, void* stream);
+
+/* 8-bit output, the inverse of usf_ingest_u8: out[r, j] = min(255, max(0, floor(256 y[r, j]))), NaN -> 0.  256 y is exact
+ * in fp32, so every value usf_ingest_u8 makes of k (either mode) quantises back to k. */
+int usf_quantize_u8(const float* y, int64_t ldy, int64_t rows, int32_t d, uint8_t* out, int64_t ldo, void* stream);
+
 /* Lp-radial base density:  out[r] = log f_R(r_r) - [dv_const + (d-1) log r_r] + add_const,  r_r = ||z[r,:] - loc||_p
  * (z = z [+ z_lo]); f_R is LogNormal(mu, sigma) or a K-component mixture (K <= 128) of Gammas, generalised Gammas or
  * log-normals, `norm_params` as listed at USF_NORM_*, already constrained (sigma, concentration, rate, scale, power > 0;
@@ -234,6 +256,10 @@ int usf_radial_logprob(const float* z, const float* z_lo, int64_t ldz, int64_t r
 int usf_radial_sample(int64_t rows, int32_t d, const float* loc, int32_t p_kind, int32_t norm_kind,
                       const float* norm_params, int32_t n_comp, uint64_t seed, uint64_t offset, float* out, int64_t ldo,
                       void* stream);
+/* usf_radial_sample with the draws of global rows draw->row0 .. draw->row0 + rows - 1 (usf_draw) */
+int usf_radial_sample_at(int64_t rows, int32_t d, const float* loc, int32_t p_kind, int32_t norm_kind,
+                         const float* norm_params, int32_t n_comp, const usf_draw* draw, float* out, int64_t ldo,
+                         void* stream);
 
 /* Row-wise glue of networks.ConvNet's vector branch (networks.py:205-245, 287-307) between two usf_linear calls:
  *   v = gated ? xres[r,j] + o[r,j] * sigmoid(o[r,n+j]) : o[r,j]        (GatedMLP: o = [val | gate], xres = x or proj(x))
@@ -252,6 +278,10 @@ int usf_gate_norm(const float* o, int64_t ldo, const float* xres, int64_t ldx, i
  * over [C, H, W] (transforms.py:105-125). */
 int usf_layout_transpose(const float* in, int64_t n, int32_t a, int32_t b, const float* scale, int32_t scale_mode,
                          int32_t scale_on_input, float* out, void* stream);
+/* the channels-last -> NCHW direction of usf_layout_transpose (scale_on_input = 0: `scale` indexed in NCHW order on the
+ * output side) writing 8-bit images: each fp32 value it would write is quantised as usf_quantize_u8 does */
+int usf_layout_transpose_to_u8(const float* in, int64_t n, int32_t a, int32_t b, const float* scale, int32_t scale_mode,
+                               uint8_t* out, void* stream);
 /* the NCHW -> channels-last direction of usf_layout_transpose (A = c, B = hw, scale on the input side) reading 8-bit images
  * in [n, c, hw], dequantised as usf_ingest_u8 does (j = c_index * hw + pixel, r = dq->row0 + image index) */
 int usf_layout_transpose_u8(const uint8_t* in, int64_t n, int32_t c, int32_t hw, const usf_dequant* dq, const float* scale,

@@ -11,7 +11,7 @@ from . import distributions, nn, transforms  # noqa: F401
 from .distributions import Chi, Gamma, GammaMM, LogNormalMM, WeibullMM, Independent, Laplace, LogNormal, Normal, RadialDistribution  # noqa: F401
 from .engine import get_precision, set_chunk_rows, set_precision  # noqa: F401
 from .flows import Flow, USFlow  # noqa: F401
-from .ops import dequantize  # noqa: F401
+from .ops import dequantize, quantize  # noqa: F401
 from .nn import (AdditiveAffineNN, BottleneckConv, CondConvNet, CondConvNet2D, ConditionalDenseNN, ConvNet, ConvNet2D, DenseNN, GatedConv, GatedConvND, GatedMLP,  # noqa: F401
                  LayerNormChannels, LayerNormChannelsND, LayerNormVector)
 from .optim import SophiaG  # noqa: F401

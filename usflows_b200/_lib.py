@@ -93,6 +93,12 @@ class Dequant(C.Structure):
     ]
 
 
+class Draw(C.Structure):
+    """Mirror of `usf_draw` (include/usflows_b200.h)."""
+
+    _fields_ = [("seed", C.c_uint64), ("offset", C.c_uint64), ("row0", C.c_int64), ("dev_params", C.c_void_p)]
+
+
 DEQUANT_UNIFORM, DEQUANT_MIDPOINT = 0, 1
 MODE_CODES = {"fp32": 0, "fp32_tf32": 1, "fp32_simt": 2, "tf32": 3, "bf16": 4}
 PLAN_SRC_STREAM, PLAN_SRC_HIDDEN = 0, 1
@@ -133,11 +139,15 @@ SIGNATURES = {
     "usf_base_logprob": (C.c_int, [_P, _P, _I64, _I64, _I32, _P, _P, _I32, _F, _P, _P]),
     "usf_flow_small": (C.c_int, [_P, _I64, _I64, _I32, _P, _I32, _P, _I32, _I32, _I32, _P, _I64, _P]),
     "usf_base_sample": (C.c_int, [_I64, _I32, _P, _P, _I32, _U64, _U64, _P, _I64, _P, _P, _I64, _P, _I64, _P]),
+    "usf_base_sample_at": (C.c_int, [_I64, _I32, _P, _P, _I32, C.POINTER(Draw), _P, _I64, _P, _P, _I64, _P, _I64, _P]),
+    "usf_quantize_u8": (C.c_int, [_P, _I64, _I64, _I32, _P, _I64, _P]),
     "usf_affine_couple": (C.c_int, [_P, _I64, _I64, _I32, _P, _I64, _P, _P, _I64, _P, _I64, _P, _P, _I64, _P, _F, _F, _F, _P, _P]),
     "usf_sub_rows": (C.c_int, [_P, _P, _I64, _P]),
     "usf_radial_logprob": (C.c_int, [_P, _P, _I64, _I64, _I32, _P, _I32, _I32, _P, _I32, _F, _F, _P, _P]),
     "usf_radial_sample": (C.c_int, [_I64, _I32, _P, _I32, _I32, _P, _I32, _U64, _U64, _P, _I64, _P]),
+    "usf_radial_sample_at": (C.c_int, [_I64, _I32, _P, _I32, _I32, _P, _I32, C.POINTER(Draw), _P, _I64, _P]),
     "usf_layout_transpose": (C.c_int, [_P, _I64, _I32, _I32, _P, _I32, _I32, _P, _P]),
+    "usf_layout_transpose_to_u8": (C.c_int, [_P, _I64, _I32, _I32, _P, _I32, _P, _P]),
     "usf_im2col": (C.c_int, [_P, _I64, _I64, _I32, _I32, _I32, _I32, _I32, _P, _I32, C.POINTER(Planes), _P, _P]),
     "usf_conv2d_rows": (C.c_int, [C.POINTER(LinearArgs), _P, _I64, _I64, _I32, _I32, _I32, _I32, _I32, _P, _I32, _P]),
     "usf_masked_add": (C.c_int, [_P, _I64, _P, _I64, _I64, _I32, _I32, _P, _F, _P]),

@@ -112,6 +112,11 @@ static OutPlanes to_out_planes(const usf_planes* p, int32_t* overflow_flag) {
   return o;
 }
 
+static inline DrawCtr to_draw(const usf_draw* d) {
+  return DrawCtr{(unsigned long long)d->seed, (unsigned long long)d->offset, (long long)d->row0,
+                 reinterpret_cast<const long long*>(d->dev_params)};
+}
+
 static inline bool dequant_ok(const usf_dequant* dq) {
   return dq && (dq->mode == USF_DEQUANT_UNIFORM || dq->mode == USF_DEQUANT_MIDPOINT);
 }
@@ -260,13 +265,34 @@ int usf_base_logprob(const float* z, const float* z_lo, int64_t ldz, int64_t row
 int usf_base_sample(int64_t rows, int32_t d, const float* loc, const float* scale, int32_t base_kind, uint64_t seed,
                     uint64_t offset, float* out_f32, int64_t ld_f32, float* out_hi, float* out_lo, int64_t ld_split,
                     void* out_bf16, int64_t ld_bf16, void* stream) {
+  const usf_draw dr{seed, offset, 0, nullptr};
+  return usf_base_sample_at(rows, d, loc, scale, base_kind, &dr, out_f32, ld_f32, out_hi, out_lo, ld_split, out_bf16, ld_bf16,
+                            stream);
+}
+
+int usf_base_sample_at(int64_t rows, int32_t d, const float* loc, const float* scale, int32_t base_kind, const usf_draw* draw,
+                       float* out_f32, int64_t ld_f32, float* out_hi, float* out_lo, int64_t ld_split, void* out_bf16,
+                       int64_t ld_bf16, void* stream) {
   USF_REQUIRE(loc && scale && d > 0 && rows >= 0, "bad input");
+  USF_REQUIRE(draw && draw->row0 >= 0, "bad draw (null, or negative row0)");
   USF_REQUIRE(base_kind == USF_BASE_LAPLACE || base_kind == USF_BASE_NORMAL, "unknown base distribution");
   USF_REQUIRE((out_hi == nullptr) == (out_lo == nullptr), "out_hi and out_lo come as a pair");
   if (rows == 0) return USF_OK;
   OutPlanes o{out_f32, out_hi, out_lo, reinterpret_cast<__nv_bfloat16*>(out_bf16), ld_f32, ld_split, ld_bf16};
   const int vec = planes_vec_ok(o) ? 1 : 0;
-  base_sample_kernel<<<ew_grid(rows * ((d + 3) / 4), 256), 256, 0, S(stream)>>>(rows, d, loc, scale, base_kind, seed, offset, o, vec);
+  base_sample_kernel<<<ew_grid(rows * ((d + 3) / 4), 256), 256, 0, S(stream)>>>(rows, d, loc, scale, base_kind, to_draw(draw), o, vec);
+  USF_CUDA_OK(cudaGetLastError());
+  return USF_OK;
+}
+
+int usf_quantize_u8(const float* y, int64_t ldy, int64_t rows, int32_t d, uint8_t* out, int64_t ldo, void* stream) {
+  USF_REQUIRE(y && out && rows >= 0 && d > 0 && ldy >= d && ldo >= d, "bad input");
+  if (rows == 0) return USF_OK;
+  const bool vec = aligned16(y) && ldy % 4 == 0 && d % 4 == 0 && (reinterpret_cast<uintptr_t>(out) & 3u) == 0 && ldo % 4 == 0;
+  if (vec)
+    quantize_u8_kernel<true><<<ew_grid(rows * (d / 4), 256), 256, 0, S(stream)>>>(y, ldy, rows, d, out, ldo);
+  else
+    quantize_u8_kernel<false><<<ew_grid(rows * d, 256), 256, 0, S(stream)>>>(y, ldy, rows, d, out, ldo);
   USF_CUDA_OK(cudaGetLastError());
   return USF_OK;
 }
@@ -308,13 +334,21 @@ int usf_radial_logprob(const float* z, const float* z_lo, int64_t ldz, int64_t r
 int usf_radial_sample(int64_t rows, int32_t d, const float* loc, int32_t p_kind, int32_t norm_kind,
                       const float* norm_params, int32_t n_comp, uint64_t seed, uint64_t offset, float* out, int64_t ldo,
                       void* stream) {
+  const usf_draw dr{seed, offset, 0, nullptr};
+  return usf_radial_sample_at(rows, d, loc, p_kind, norm_kind, norm_params, n_comp, &dr, out, ldo, stream);
+}
+
+int usf_radial_sample_at(int64_t rows, int32_t d, const float* loc, int32_t p_kind, int32_t norm_kind,
+                         const float* norm_params, int32_t n_comp, const usf_draw* draw, float* out, int64_t ldo,
+                         void* stream) {
   USF_REQUIRE(loc && norm_params && out && d > 0 && rows >= 0 && ldo >= d, "bad input");
+  USF_REQUIRE(draw && draw->row0 >= 0, "bad draw (null, or negative row0)");
   USF_REQUIRE(p_kind == USF_LP_INF || p_kind == USF_LP_1 || p_kind == USF_LP_2, "p must be 1, 2 or inf");
   USF_REQUIRE(norm_kind == USF_NORM_LOGNORMAL ||
               (norm_kind >= USF_NORM_GAMMA_MIXTURE && norm_kind <= USF_NORM_LOGNORMAL_MIXTURE && n_comp >= 1 && n_comp <= RAD_MAX_COMP),
               "unknown norm distribution / too many mixture components");
   if (rows == 0) return USF_OK;
-  radial_sample_kernel<<<ew_grid(rows * 32, RAD_THREADS), RAD_THREADS, 0, S(stream)>>>(rows, d, loc, p_kind, norm_kind, norm_params, n_comp, seed, offset, out, ldo);
+  radial_sample_kernel<<<ew_grid(rows * 32, RAD_THREADS), RAD_THREADS, 0, S(stream)>>>(rows, d, loc, p_kind, norm_kind, norm_params, n_comp, to_draw(draw), out, ldo);
   USF_CUDA_OK(cudaGetLastError());
   return USF_OK;
 }
@@ -359,6 +393,18 @@ int usf_layout_transpose(const float* in, int64_t n, int32_t a, int32_t b, const
   const long long tiles = (long long)n * ((a + 31) / 32) * ((b + 31) / 32);
   layout_kernel<float><<<ew_grid(tiles * 256, 256), 256, 0, S(stream)>>>(in, n, a, b, scale, scale_mode, scale_on_input, out,
                                                                          LayoutU8{0, 0, nullptr, 0});
+  USF_CUDA_OK(cudaGetLastError());
+  return USF_OK;
+}
+
+int usf_layout_transpose_to_u8(const float* in, int64_t n, int32_t a, int32_t b, const float* scale, int32_t scale_mode,
+                               uint8_t* out, void* stream) {
+  USF_REQUIRE(in && out && n >= 0 && a > 0 && b > 0, "bad input");
+  USF_REQUIRE(scale_mode >= 0 && scale_mode <= 2 && (scale_mode == 0 || scale), "scale_mode 0 (none), 1 (multiply) or 2 (divide)");
+  if (n == 0) return USF_OK;
+  const long long tiles = (long long)n * ((a + 31) / 32) * ((b + 31) / 32);
+  layout_kernel<float, uint8_t><<<ew_grid(tiles * 256, 256), 256, 0, S(stream)>>>(in, n, a, b, scale, scale_mode, 0, out,
+                                                                                  LayoutU8{0, 0, nullptr, 0});
   USF_CUDA_OK(cudaGetLastError());
   return USF_OK;
 }

@@ -257,16 +257,31 @@ base_logprob_kernel(const float* __restrict__ z, const float* __restrict__ z_lo,
 // (24 bits + 1/2 would round up to 1.0 for the top value and give log1p(-1) = -inf in the Laplace inverse CDF)
 __device__ __forceinline__ float u01_open(uint32_t x) { return ((float)(x >> 9) + 0.5f) * (1.0f / 8388608.0f); }
 
+// Philox key and counter base of one sampling call (usf_draw): local row r draws as GLOBAL row row0 + r, so a chunk of
+// rows [r0, r1) of a larger call reproduces exactly those rows.  `params` (device {seed, row base}) replaces the seed and
+// adds to row0 at run time, so one captured graph serves every chunk.
+struct DrawCtr {
+  unsigned long long seed, offset;
+  long long row0;
+  const long long* params;
+  __device__ __forceinline__ void init() {
+    if (params) { seed = (unsigned long long)__ldg(params); row0 += __ldg(params + 1); }
+  }
+};
+
 __global__ void __launch_bounds__(256)
 base_sample_kernel(long long rows, int d, const float* __restrict__ loc, const float* __restrict__ scale, int kind,
-                   uint64_t seed, uint64_t offset, OutPlanes o, int vec) {
+                   DrawCtr dc, OutPlanes o, int vec) {
+  dc.init();
+  const uint64_t seed = dc.seed, offset = dc.offset;
   const int d4 = (d + 3) >> 2;
   const long long total = rows * d4;
+  const uint64_t ctr0 = (uint64_t)dc.row0 * (uint64_t)d4;        // counter of the call's row r, group g: (row0 + r) * d4 + g
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
     const long long r = i / d4;
     const int j = (int)(i - r * d4) * 4;
     uint32_t rnd[4], rnd2[4];
-    philox4x32_10(seed, (uint64_t)i, offset, rnd);
+    philox4x32_10(seed, ctr0 + (uint64_t)i, offset, rnd);
     float e[4];
     if (kind == USF_BASE_LAPLACE) {
       // inverse CDF on u in (-1, 1): eps = -sign(u) * log1p(-|u|)  (torch.distributions.Laplace.rsample)
@@ -276,7 +291,7 @@ base_sample_kernel(long long rows, int d, const float* __restrict__ loc, const f
         e[t] = -copysignf(1.f, u) * log1pf(-fabsf(u));
       }
     } else {
-      philox4x32_10(seed, (uint64_t)i, offset ^ 0x8000000000000000ull, rnd2);
+      philox4x32_10(seed, ctr0 + (uint64_t)i, offset ^ 0x8000000000000000ull, rnd2);
 #pragma unroll
       for (int t = 0; t < 4; t += 2) {  // Box-Muller
         const float u1 = u01_open(rnd[t]), u2 = u01_open(rnd2[t]);
@@ -293,6 +308,36 @@ base_sample_kernel(long long rows, int d, const float* __restrict__ loc, const f
     if (vec && j + 3 < d) store_planes4(o, r, j, v);
     else
       for (int t = 0; t < 4 && j + t < d; ++t) store_planes1(o, r, j + t, v[t]);
+  }
+}
+
+// ---- 8-bit output (usf_quantize_u8): q = min(255, max(0, floor(256 y))), NaN -> 0 ------------------------------------
+// 256 y is exact in fp32, so q is the k that usf_ingest_u8 dequantises into (k/256, (k+1)/256), in either mode.
+__device__ __forceinline__ uint32_t quantize_value(float y) {
+  const float t = floorf(256.f * y);
+  return t >= 255.f ? 255u : t >= 0.f ? (uint32_t)t : 0u;      // a NaN fails both comparisons
+}
+
+template <bool VEC>
+__global__ void __launch_bounds__(256)
+quantize_u8_kernel(const float* __restrict__ y, long long ldy, long long rows, int d, uint8_t* __restrict__ out, long long ldo) {
+  if (VEC) {
+    const int d4 = d >> 2;
+    const long long total = rows * d4;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+      const long long r = i / d4;
+      const int j = (int)(i - r * d4) * 4;
+      const float4 v = __ldcs(reinterpret_cast<const float4*>(y + r * ldy + j));
+      const uint32_t q = quantize_value(v.x) | (quantize_value(v.y) << 8) | (quantize_value(v.z) << 16) | (quantize_value(v.w) << 24);
+      *reinterpret_cast<uint32_t*>(out + r * ldo + j) = q;
+    }
+  } else {
+    const long long total = rows * d;
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
+      const long long r = i / d;
+      const int j = (int)(i - r * d);
+      out[r * ldo + j] = (uint8_t)quantize_value(y[r * ldy + j]);
+    }
   }
 }
 

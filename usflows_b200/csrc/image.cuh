@@ -24,10 +24,10 @@ struct LayoutU8 {
   const long long* params;
   int mode;
 };
-template <class T>
+template <class T, class OutT = float>
 __global__ void __launch_bounds__(256)
 layout_kernel(const T* __restrict__ in, long long N, int A, int B, const float* __restrict__ s, int s_mode, int s_on_input,
-              float* __restrict__ out, LayoutU8 dq) {
+              OutT* __restrict__ out, LayoutU8 dq) {
   __shared__ float tile[32][33];
   if (sizeof(T) == 1 && dq.params) { dq.seed = (unsigned long long)__ldg(dq.params); dq.row0 += __ldg(dq.params + 1); }
   const int ta = (A + 31) >> 5, tb = (B + 31) >> 5;
@@ -38,7 +38,7 @@ layout_kernel(const T* __restrict__ in, long long N, int A, int B, const float* 
     const int rem = (int)(t - n * (ta * tb));
     const int a0 = (rem / tb) << 5, b0 = (rem % tb) << 5;
     const T* src = in + n * (long long)A * B;
-    float* dst = out + n * (long long)A * B;
+    OutT* dst = out + n * (long long)A * B;
 #pragma unroll
     for (int i = 0; i < 32; i += 8) {
       const int a = a0 + ty + i, b = b0 + tx;
@@ -63,7 +63,10 @@ layout_kernel(const T* __restrict__ in, long long N, int A, int B, const float* 
 #pragma unroll
     for (int i = 0; i < 32; i += 8) {
       const int b = b0 + ty + i, a = a0 + tx;
-      if (a < A && b < B) dst[(long long)b * A + a] = tile[tx][ty + i];
+      if (a < A && b < B) {
+        if (sizeof(OutT) == 1) dst[(long long)b * A + a] = (OutT)quantize_value(tile[tx][ty + i]);
+        else dst[(long long)b * A + a] = tile[tx][ty + i];
+      }
     }
     __syncthreads();
   }

@@ -175,15 +175,18 @@ __device__ float gamma_mt(float a, uint64_t seed, uint64_t ctr, uint64_t off) {
 
 __global__ void __launch_bounds__(RAD_THREADS)
 radial_sample_kernel(long long rows, int d, const float* __restrict__ loc, int p_kind, int norm_kind,
-                     const float* __restrict__ params, int n_comp, uint64_t seed, uint64_t offset,
-                     float* __restrict__ out, long long ldo) {
+                     const float* __restrict__ params, int n_comp, DrawCtr dc, float* __restrict__ out, long long ldo) {
   __shared__ GammaMixSmem sm;
   if (norm_kind != USF_NORM_LOGNORMAL) gamma_mix_prepare(sm, params, n_comp, norm_kind);
+  dc.init();
+  const uint64_t seed = dc.seed, offset = dc.offset;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int wpb = RAD_THREADS / 32;
   const int d4 = (d + 3) >> 2;
   const uint64_t RTAG = 0x4000000000000000ull;
-  for (long long r = (long long)blockIdx.x * wpb + warp; r < rows; r += (long long)gridDim.x * wpb) {
+  for (long long lr = (long long)blockIdx.x * wpb + warp; lr < rows; lr += (long long)gridDim.x * wpb) {
+    const long long r = dc.row0 + lr;          // every counter below is keyed by the GLOBAL row (usf_draw)
+    float* __restrict__ orow = out + lr * ldo;
     float radius = 0.f;
     int extremal = -1;
     if (lane == 0) {
@@ -255,7 +258,7 @@ radial_sample_kernel(long long rows, int d, const float* __restrict__ loc, int p
 #pragma unroll
       for (int t = 0; t < 4; ++t) {
         const int j = g * 4 + t;
-        if (j < d) out[r * ldo + j] = fmaf(mul, j == extremal ? 1.f : e[t], __ldg(loc + j));
+        if (j < d) orow[j] = fmaf(mul, j == extremal ? 1.f : e[t], __ldg(loc + j));
       }
     }
   }

@@ -56,9 +56,13 @@ class DistributionModule(Module):
         loc, scale = self._prepared() if perm is None else self._permuted(perm)
         ops.base_logprob(z, loc, scale, self.base_kind, add_const, out)
 
-    def _sample_into(self, out: torch.Tensor, seed: int, offset: int) -> None:
+    def _sample_into(self, out: torch.Tensor, draw: "ops.Draw") -> None:
         loc, scale = self._prepared()
-        ops.base_sample(ops.Act(out.shape[0], out.shape[1], f32=out), loc, scale, self.base_kind, seed, offset)
+        a = ops.Act(out.shape[0], out.shape[1], f32=out)
+        if draw.plain:
+            ops.base_sample(a, loc, scale, self.base_kind, draw.seed, draw.offset)
+        else:
+            ops.base_sample_at(a, loc, scale, self.base_kind, draw)
 
     @property
     def event_shape(self) -> torch.Size:
@@ -581,9 +585,12 @@ class RadialDistribution(Module):
             loc = self._perm_loc
         ops.radial_logprob(z, loc, self._p_kind, kind, params, K, self.log_delta_volume_const(), add_const, out)
 
-    def _sample_into(self, out: torch.Tensor, seed: int, offset: int) -> None:
+    def _sample_into(self, out: torch.Tensor, draw: "ops.Draw") -> None:
         loc, kind, K, params = self._prepared()
-        ops.radial_sample(out, loc, self._p_kind, kind, params, K, seed, offset)
+        if draw.plain:
+            ops.radial_sample(out, loc, self._p_kind, kind, params, K, draw.seed, draw.offset)
+        else:
+            ops.radial_sample_at(out, loc, self._p_kind, kind, params, K, draw)
 
     def forward(self, x: torch.Tensor) -> torch.Tensor:
         return self.log_prob(x)

@@ -1018,7 +1018,7 @@ def base_sample(base, sample_shape=None) -> torch.Tensor:
     out = torch.empty(rows, d, dtype=torch.float32, device=base._prepared()[0].device)
     seed, offset = philox_call_stream(out.device)
     with ops.on_device(out):
-        base._sample_into(out, seed, offset)
+        base._sample_into(out, ops.Draw(seed, offset=offset))
     return out.reshape(*shape, *base.event_shape)
 
 

@@ -113,6 +113,22 @@ def _wave_aligned_chunk_rows(prog, device) -> int:
     return 256 * unit * k
 
 
+def sample_host_bounds(n: int, unit: int, uniform: bool = False):
+    """Chunks of `sample_host`.  There the LAST device-to-host copy is the exposed one (the reverse of `log_prob_host`), so
+    the chunks shrink towards the end: HOST_CHUNK_UNITS read from the end, in wave-aligned units; the first chunk takes the
+    remainder.  `uniform`: chunks of `unit` rows from the start."""
+    if uniform:
+        return [(r0, min(n, r0 + unit)) for r0 in range(0, n, unit)]
+    bounds, r1 = [], n
+    while r1 > 0:
+        take = min(unit * HOST_CHUNK_UNITS[min(len(bounds), len(HOST_CHUNK_UNITS) - 1)], r1)
+        if r1 - take < unit // 2:                 # do not leave a sliver for a launch sequence of its own
+            take = r1
+        bounds.append((r1 - take, r1))
+        r1 -= take
+    return bounds[::-1]
+
+
 class Flow(torch.nn.Module):
     """Base flow: a list of bijective layers over a base distribution (flows.py:22-292)."""
 
@@ -523,17 +539,199 @@ class Flow(torch.nn.Module):
             main.synchronize()
         return out_host
 
-    def sample(self, sample_shape: Iterable[int] = None, context: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """Draw from the base and push through the layers (flows.py:247-265)."""
+    def sample(self, sample_shape: Iterable[int] = None, context: Optional[torch.Tensor] = None, *, seed: Optional[int] = None,
+               quantize: bool = False) -> torch.Tensor:
+        """Draw from the base and push through the layers (flows.py:247-265).
+
+        With `seed`, the base draws are keyed by (seed, global row) alone (ops.Draw): the result does not depend on
+        `torch.manual_seed`, and row r equals row r of `sample_host(n, seed=seed)`.  With `quantize`, the result is uint8
+        `[*sample_shape, *event]`: the 8-bit pixels `usflows_b200.quantize` makes of the samples."""
         if sample_shape is None:
             sample_shape = [1]
         shape = [int(s) for s in sample_shape]
         with ops.on_device(next(self.parameters())):
-            z = self.base_distribution.sample(shape)
             ev = len(self._event_shape())
-            z = z.reshape(-1, *z.shape[z.dim() - ev:])
+            if seed is None:
+                z = self.base_distribution.sample(shape)
+                z = z.reshape(-1, *z.shape[z.dim() - ev:])
+            else:
+                rows = math.prod(shape)
+                z = self._draw(rows, ops.Draw(int(seed))).reshape(rows, *self._event_shape())
             y = self._run("forward", z, self._zero_ctx) if context is None else self._with_context("forward", z, context)
+            if quantize:
+                y = ops.quantize(y)
         return y.reshape(*shape, *y.shape[1:])
+
+    def _draw(self, rows: int, draw: ops.Draw, out: Optional[torch.Tensor] = None) -> torch.Tensor:
+        """Base draws [rows, d] of the global rows draw.row0 .. draw.row0 + rows - 1, into `out` when given."""
+        if out is None:
+            out = torch.empty(rows, math.prod(self._event_shape()), dtype=torch.float32, device=next(self.parameters()).device)
+        if rows:
+            with torch.no_grad():
+                self._base_module()._sample_into(out, draw)
+        return out
+
+    def sample_host(self, n: int, out_host: Optional[torch.Tensor] = None, *, seed: Optional[int] = None,
+                    quantize: bool = False, row_offset: int = 0, chunk_rows: Optional[int] = None) -> torch.Tensor:
+        """`n` samples [n, *event] streamed into HOST memory (`out_host`, allocated pinned when None) in chunks, returned.
+        The device holds two chunks of output whatever `n` is, and the device-to-host copy of chunk i runs on a side stream
+        under the kernels of the next chunk.  Row r is global row `row_offset + r` of the stream of `seed` (the rows
+        `sample(seed=seed)` draws from 0 on), so a caller that splits one draw over several calls or devices passes each
+        part's offset and one seed; `seed=None` draws one from torch.default_generator.  With `quantize`, the result is
+        uint8 pixels (see `sample`): a quarter of the bytes cross to the host.  `chunk_rows` gives uniform chunks."""
+        n, row_offset = int(n), int(row_offset)
+        if n < 0 or row_offset < 0:
+            raise ValueError(f"usflows_b200: sample_host needs n >= 0 and row_offset >= 0, got {n}, {row_offset}")
+        ev = tuple(self._event_shape())
+        dtype = torch.uint8 if quantize else torch.float32
+        if out_host is None:
+            out_host = torch.empty(n, *ev, dtype=dtype, pin_memory=torch.cuda.is_available())
+        elif out_host.is_cuda:
+            raise RuntimeError("sample_host writes host memory; use sample for device tensors")
+        elif out_host.dtype != dtype or tuple(out_host.shape) != (n, *ev) or not out_host.is_contiguous():
+            raise ValueError(f"usflows_b200: out_host must be a contiguous {dtype} tensor of shape {(n, *ev)}, got "
+                             f"{out_host.dtype} {tuple(out_host.shape)}")
+        draw = ops.Draw(ops.draw_seed() if seed is None else int(seed), row_offset)
+        if n:
+            with ops.on_device(next(self.parameters())), torch.no_grad():
+                self._sample_host(out_host.view(n, -1), draw, quantize, chunk_rows)
+        return out_host
+
+    def _sample_graph(self, prog, base, slot: int, buf: torch.Tensor, quantize: bool) -> dict:
+        """CUDA graph of one full-size chunk of `sample_host` writing output buffer `slot`: the base draws at the {seed, row
+        base} read from its `params` tensor (written before a replay), the launch program, the quantisation."""
+        cache = prog.__dict__.setdefault("_sample_graphs", {})   # on the Program: see _log_prob_small_batch
+        rows, d = buf.shape
+        key = (slot, buf.data_ptr(), rows, quantize)
+        ent = cache.get(key)
+        if ent is not None and ent["gen"] == engine._workspace.generation:
+            return ent
+        dev = buf.device
+        flag = torch.zeros(1, dtype=torch.int32, device=dev) if prog.uses_range_flag else None
+        params = torch.zeros(2, dtype=torch.int64, device=dev)
+        z = engine._workspace.planes(dev, f"sample_z{slot}", 1, rows * d, "f32").view(rows, d)
+        fin = prog.final_buffer(dev, f"final_q{slot}", rows, d) if quantize else buf
+        draw = ops.Draw(0, 0, params)
+
+        def body():
+            base._sample_into(z, draw)
+            prog._run_chunk(z, fin, flag)
+            if quantize:
+                ops.quantize_u8(fin, buf)
+        ent = dict(graph=_capture(dev, body), flag=flag, params=params, gen=engine._workspace.generation)
+        for k in [k for k in cache if cache[k]["gen"] != ent["gen"] or (k[0] == slot and k[1] != key[1] and k[3] == quantize)]:
+            del cache[k]                                  # graphs of stale workspaces / of a replaced output buffer
+        while len(cache) >= 8:                            # a few chunk sizes per buffer; drop the oldest
+            del cache[next(iter(cache))]
+        cache[key] = ent
+        return ent
+
+    def _sample_host(self, flat: torch.Tensor, draw: ops.Draw, quantize: bool, chunk_rows: Optional[int]) -> None:
+        dev = next(self.parameters()).device
+        cuda = dev.type == "cuda"
+        n, d = flat.shape
+        base = self._base_module()
+        base._prepared()                  # parameter-side work happens here, outside any graph capture
+        prog = None if self._layer_route else self._program("forward", self._zero_ctx)[0]
+        images = isinstance(prog, image_engine.ImageProgram)
+        launch = prog is not None and not images and prog.small is None       # the flat launch program, chunk by chunk
+        if prog is not None and prog.force_fallback:
+            prog = prog._fallback()
+        if launch:
+            unit = min(chunk_rows or _wave_aligned_chunk_rows(prog, dev), n)
+            bounds = sample_host_bounds(n, unit, uniform=bool(chunk_rows))
+        else:                             # images: eager chunks; single-launch and layer-route flows: plain chunks
+            step = chunk_rows or (prog._chunk_bounds(n, None)[0][1] if images else HOST_CHUNK_ROWS)
+            bounds = [(r0, min(n, r0 + step)) for r0 in range(0, n, step)]
+        chunk = max(r1 - r0 for r0, r1 in bounds)
+        # two output buffers used in turn; fp32 and uint8 calls in turn keep their own buffers and captured graphs
+        attr = "_sample_stage_u8" if quantize else "_sample_stage"
+        stage = getattr(self, attr, None)
+        if stage is None or stage.shape[1] < chunk or stage.shape[2] != d or stage.device != dev:
+            stage = torch.empty(2, chunk, d, dtype=flat.dtype, device=dev)
+            setattr(self, attr, stage)
+        if cuda and (getattr(self, "_sample_stream", None) is None or self._sample_stream.device != dev):
+            self._sample_stream = torch.cuda.Stream(device=dev)
+        main = torch.cuda.current_stream(dev) if cuda else None
+        side = self._sample_stream if cuda else None
+        ready = [torch.cuda.Event() for _ in range(2)] if cuda else None
+        copied = [torch.cuda.Event() for _ in range(2)] if cuda else None
+        issued = [0]
+
+        def emit(r0, r1, run):
+            """run(buf) fills an output buffer with rows [r0, r1); its D2H copy follows on the side stream, and the buffer's
+            next use waits for that copy."""
+            slot = issued[0] % 2
+            issued[0] += 1
+            buf = stage[slot][:r1 - r0]
+            if not cuda:
+                run(buf)
+                flat[r0:r1].copy_(buf)
+                return
+            main.wait_event(copied[slot])
+            run(buf)
+            ready[slot].record(main)
+            with torch.cuda.stream(side):
+                side.wait_event(ready[slot])
+                flat[r0:r1].copy_(buf, non_blocking=True)
+                copied[slot].record(side)
+
+        def compute(p, buf, r0, r1, flag):
+            rows, dr = r1 - r0, draw.shifted(r0)
+            if p is None or p.small is not None:          # what `sample` runs
+                z = self._draw(rows, dr).reshape(rows, *self._event_shape())
+                y = self._run("forward", z, self._zero_ctx).reshape(rows, d)
+                if quantize:
+                    ops.quantize_u8(y, buf)
+                else:
+                    buf.copy_(y)
+                return
+            z = engine._workspace.planes(dev, "sample_z", 1, rows * d, "f32").view(rows, d)
+            base._sample_into(z, dr)
+            if images:
+                p._run_chunk(z, buf, flag, nchw_out=True, quantize=quantize)
+                return
+            fin = p.final_buffer(dev, "final_q", rows, d) if quantize else buf
+            p._run_chunk(z, fin, flag)
+            if quantize:
+                ops.quantize_u8(fin, buf)
+
+        graphs = {}
+        if cuda and launch and HOST_CUDA_GRAPHS and not prog.force_fallback and n >= unit:
+            sizes = [r1 - r0 for r0, r1 in bounds]
+            for _ in range(2):                            # a workspace that grew while capturing invalidates earlier graphs
+                for i in sorted(range(len(sizes)), key=lambda j: -sizes[j]):
+                    if sizes[i] >= unit // 2:
+                        graphs[(i % 2, sizes[i])] = self._sample_graph(prog, base, i % 2, stage[i % 2][:sizes[i]], quantize)
+                if all(g["gen"] == engine._workspace.generation for g in graphs.values()):
+                    break
+            for g in graphs.values():
+                if g["flag"] is not None:
+                    g["flag"].zero_()
+            wrap = lambda v: (v + 2**63) % 2**64 - 2**63                     # noqa: E731  (uint64 bits as int64)
+            params = torch.tensor([[wrap(draw.seed), draw.row0 + r0] for r0, _ in bounds], dtype=torch.int64).to(dev)
+
+        def first(i, r0, r1, flag):
+            g = graphs.get((i % 2, r1 - r0))
+            if g is None:
+                emit(r0, r1, lambda buf: compute(prog, buf, r0, r1, flag))
+                return
+
+            def replay(buf):
+                g["params"].copy_(params[i])
+                g["graph"].replay()
+            emit(r0, r1, replay)
+
+        def again(i, r0, r1):                             # the same rows of the noise on the tf32-split program
+            emit(r0, r1, lambda buf: compute(prog._fallback(), buf, r0, r1, None))
+
+        guarded = prog is not None and prog.small is None and prog.uses_range_flag and not prog.force_fallback
+        if cuda:
+            side.wait_stream(main)
+        # a graph's flag is not per chunk: when one is set, every chunk is recomputed
+        engine.run_chunks(bounds, dev, guarded, first, again, shared_flags=[g["flag"] for g in graphs.values()])
+        if cuda:
+            side.synchronize()
 
     def fit(self, data_train, optim=None, optim_params: Optional[Dict[str, Any]] = None, batch_size: int = 32,
             shuffle: bool = True, gradient_clip: Optional[float] = None, device=None, epochs: int = 1, **kw):

@@ -302,11 +302,13 @@ class ImageProgram(engine.ProgramCore):
 
     # ----------------------------------------------------------------------------------------------
     def _run_chunk(self, x: torch.Tensor, out: torch.Tensor, flag, dq: Optional[ops.Dequant] = None, *,
-                   nchw_out: bool = False) -> None:
+                   nchw_out: bool = False, quantize: bool = False) -> None:
         """x [n, C*H*W] (NCHW, read-only) -> out [n, C*H*W]: channels-last ([n, H*W*C]), or NCHW when `nchw_out`.  With
-        `dq`, x is uint8 and the NCHW -> channels-last conversion dequantises it."""
+        `dq`, x is uint8 and the NCHW -> channels-last conversion dequantises it.  With `quantize` (NCHW only), out is uint8
+        and the channels-last -> NCHW conversion writes the quantised pixels (ops.quantize)."""
         dev, n = x.device, x.shape[0]
         rows, C, HW = n * self.HW, self.C, self.HW
+        nchw_out = nchw_out or quantize
         direct = not nchw_out and self.exit_scale is None    # the channels-last stream itself is the result
         bufs = [_dense(dev, "img_x0", rows, C), _dense(dev, "img_x1", rows, C)]
         which, cur = 0, bufs[0]
@@ -342,7 +344,9 @@ class ImageProgram(engine.ProgramCore):
                 out.view(rows, C).copy_(cur)
             return
         xs = self.exit_scale
-        if nchw_out:
+        if quantize:
+            ops.layout_transpose_to_u8(cur, n, HW, C, out, scale=None if xs is None else xs[0], scale_mode=0 if xs is None else xs[1])
+        elif nchw_out:
             ops.layout_transpose(cur, n, HW, C, out, scale=None if xs is None else xs[0], scale_mode=0 if xs is None else xs[1],
                                  scale_on_input=False)
         else:                                                # channels-last result with a trailing scale: two conversions

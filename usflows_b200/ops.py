@@ -238,6 +238,65 @@ def base_sample(out: Act, loc, scale, kind: int, seed: int, offset: int) -> None
         _ptr(out.bf16), _ld(out.bf16) if out.bf16 is not None else 0, _stream()))
 
 
+@dataclass(frozen=True)
+class Draw:
+    """Which Philox draws a sampling call makes (usf_draw): key `seed`, sub-stream `offset`, the global row of local row 0
+    `row0`, and optionally `params`, a device int64 [2] tensor {seed, row base} read at run time (seed replaced, row base
+    added to row0) so that one captured graph serves every chunk.  Rows [r0, r1) of a call are the call `shifted(r0)` over
+    r1 - r0 rows."""
+
+    seed: int
+    row0: int = 0
+    params: Optional[torch.Tensor] = None
+    offset: int = 0
+
+    def shifted(self, rows: int) -> "Draw":
+        return Draw(self.seed, self.row0 + int(rows), self.params, self.offset)
+
+    @property
+    def plain(self) -> bool:
+        """The draws of the row0 = 0 entries (usf_base_sample / usf_radial_sample)."""
+        return self.row0 == 0 and self.params is None
+
+    def struct(self):
+        s = _lib.Draw()
+        s.seed, s.offset, s.row0 = self.seed & (2**64 - 1), self.offset & (2**64 - 1), self.row0
+        s.dev_params = _ptr(self.params)
+        return s
+
+
+def base_sample_at(out: Act, loc, scale, kind: int, draw: Draw) -> None:
+    """`base_sample` drawing the global rows draw.row0 .. draw.row0 + out.rows - 1; see usf_base_sample_at."""
+    s = draw.struct()
+    check(_lib.load().usf_base_sample_at(
+        out.rows, out.width, _ptr(loc), _ptr(scale), kind, C.byref(s),
+        _ptr(out.f32), _ld(out.f32) if out.f32 is not None else 0,
+        _ptr(out.hi), _ptr(out.lo), _ld(out.hi) if out.hi is not None else 0,
+        _ptr(out.bf16), _ld(out.bf16) if out.bf16 is not None else 0, _stream()))
+
+
+def quantize_u8(y: torch.Tensor, out: torch.Tensor) -> None:
+    """out [rows, d] uint8 = min(255, max(0, floor(256 y))), NaN -> 0, from fp32 y [rows, d]; see usf_quantize_u8."""
+    global LAUNCHES
+    LAUNCHES += 1
+    rows, d = y.shape
+    check(_lib.load().usf_quantize_u8(_ptr(y), _ld(y), rows, d, _ptr(out), _ld(out), _stream()))
+
+
+def quantize(y: torch.Tensor) -> torch.Tensor:
+    """8-bit values of the fp32 CUDA tensor `y` [rows, *event] (a 1-D tensor is one row): min(255, max(0, floor(256 y))),
+    NaN -> 0 -- the inverse of `dequantize` in both modes, and the pixels `Flow.sample(..., quantize=True)` returns."""
+    require_cuda(y, "y")
+    y2 = y.reshape(1, -1) if y.dim() <= 1 else y.reshape(y.shape[0], math.prod(y.shape[1:]))
+    if y2.shape[1] > 0 and y2.stride(1) != 1:
+        y2 = y2.contiguous()
+    out = torch.empty(y2.shape, dtype=torch.uint8, device=y.device)
+    if out.numel():
+        with on_device(y):
+            quantize_u8(y2, out)
+    return out.reshape(y.shape)
+
+
 def flow_small(x: torch.Tensor, prog_i32: torch.Tensor, blob: torch.Tensor, n_ops: int, D: int, H: int,
                out: torch.Tensor) -> None:
     """Whole layer stack in one launch (d <= 8, conditioner width <= 64); see usf_flow_small."""
@@ -278,6 +337,15 @@ def radial_sample(out: torch.Tensor, loc, p_kind: int, norm_kind: int, norm_para
     rows, d = out.shape
     check(_lib.load().usf_radial_sample(rows, d, _ptr(loc), p_kind, norm_kind, _ptr(norm_params), n_comp,
                                         seed & (2**64 - 1), offset & (2**64 - 1), _ptr(out), _ld(out), _stream()))
+
+
+def radial_sample_at(out: torch.Tensor, loc, p_kind: int, norm_kind: int, norm_params: torch.Tensor, n_comp: int,
+                     draw: Draw) -> None:
+    """`radial_sample` drawing the global rows draw.row0 .. draw.row0 + rows - 1; see usf_radial_sample_at."""
+    rows, d = out.shape
+    s = draw.struct()
+    check(_lib.load().usf_radial_sample_at(rows, d, _ptr(loc), p_kind, norm_kind, _ptr(norm_params), n_comp, C.byref(s),
+                                           _ptr(out), _ld(out), _stream()))
 
 
 def _planes_struct(a: Optional[Act]):
@@ -326,6 +394,14 @@ def layout_transpose_u8(x: torch.Tensor, dq: Dequant, n: int, c: int, hw: int, o
     s = dq.struct()
     check(_lib.load().usf_layout_transpose_u8(_ptr(x), n, c, hw, C.byref(s), _ptr(scale), scale_mode if scale is not None else 0,
                                               _ptr(out), _stream()))
+
+
+def layout_transpose_to_u8(x: torch.Tensor, n: int, a: int, b: int, out: torch.Tensor, scale=None, scale_mode: int = 0) -> None:
+    """Channels-last fp32 x [n, a*b] -> 8-bit NCHW out[n, b, a] (x| /) scale, quantised; see usf_layout_transpose_to_u8."""
+    global LAUNCHES
+    LAUNCHES += 1
+    check(_lib.load().usf_layout_transpose_to_u8(_ptr(x), n, a, b, _ptr(scale), scale_mode if scale is not None else 0,
+                                                 _ptr(out), _stream()))
 
 
 def im2col(x: torch.Tensor, n_images: int, h: int, w: int, c: int, k: int, dilation: int, out: Act, *, mask=None,

@@ -27,7 +27,7 @@ import torch
 from . import engine, ops
 
 _UNCOPIED = ("_programs", "_host_stage", "_host_stage_u8", "_host_out", "_copy_stream", "_cl_perm",
-             "_cl_perm_key", "_sharded")
+             "_cl_perm_key", "_sharded", "_sample_stage", "_sample_stage_u8", "_sample_stream")
 
 
 def shard_bounds(n: int, rank: int, world: int):
@@ -117,8 +117,13 @@ class ShardedFlow:
         self._map(work, rows)
         return out_host
 
-    def sample(self, n: int, out_host: Optional[torch.Tensor] = None) -> torch.Tensor:
-        """`n` samples [n, *event] in host memory; every device draws from its own Philox stream."""
+    def sample(self, n: int, out_host: Optional[torch.Tensor] = None, *, seed: Optional[int] = None,
+               quantize: bool = False) -> torch.Tensor:
+        """`n` samples [n, *event] in host memory; every device draws from its own Philox stream.  With `seed` or
+        `quantize` (see Flow.sample_host), one seed serves all devices and device i streams its block [lo, hi) as global
+        rows lo .. hi - 1 of that seed's stream, so the result does not depend on the number of devices."""
+        if seed is not None or quantize:
+            return self._sample_stream(n, out_host, ops.draw_seed() if seed is None else int(seed), quantize)
         self.sync_weights()
         ev = tuple(self.flow._event_shape())
         if out_host is None:
@@ -133,6 +138,20 @@ class ShardedFlow:
                     engine.philox_salt.value = 0
                 out_host[lo:hi].copy_(y, non_blocking=True)
                 torch.cuda.current_stream(self.devices[i]).synchronize()
+        self._map(work, n)
+        return out_host
+
+    def _sample_stream(self, n: int, out_host: Optional[torch.Tensor], seed: int, quantize: bool) -> torch.Tensor:
+        if n < 0:
+            raise ValueError("usflows_b200: the number of samples must be >= 0")
+        self.sync_weights()
+        if out_host is None:
+            out_host = torch.empty(n, *self.flow._event_shape(), dtype=torch.uint8 if quantize else torch.float32,
+                                   pin_memory=True)
+
+        def work(i, rep, lo, hi):
+            if hi > lo:
+                rep.sample_host(hi - lo, out_host[lo:hi], seed=seed, quantize=quantize, row_offset=lo)
         self._map(work, n)
         return out_host
 
@@ -179,6 +198,8 @@ def log_prob_sharded(flow, x_host: torch.Tensor, devices: Optional[Sequence] = N
     return _sharded(flow, devices).log_prob(x_host, out_host, dequantize=dequantize, seed=seed)
 
 
-def sample_sharded(flow, n: int, devices: Optional[Sequence] = None, out_host: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """`n` samples of `flow` in host memory, drawn on `devices` (default: all visible GPUs)."""
-    return _sharded(flow, devices).sample(n, out_host)
+def sample_sharded(flow, n: int, devices: Optional[Sequence] = None, out_host: Optional[torch.Tensor] = None, *,
+                   seed: Optional[int] = None, quantize: bool = False) -> torch.Tensor:
+    """`n` samples of `flow` in host memory, drawn on `devices` (default: all visible GPUs); `seed` / `quantize` as in
+    ShardedFlow.sample."""
+    return _sharded(flow, devices).sample(n, out_host, seed=seed, quantize=quantize)
