@@ -209,7 +209,7 @@ def test_image_flow_outside_the_fp16_range_falls_back_per_chunk():
     assert rel_err(z[:4], z_ref[:4]) <= 3e-6 and not torch.equal(z[:4], z_ref[:4])     # the others: the fp16-split engine
 
 
-def test_small_image_batches_replay_one_graph():
+def test_small_image_batches_replay_one_cached_graph():
     """`log_prob` of an image-shaped flow on a small batch: the ~100 launches of the step are captured once per batch size
     and replayed; same bits as the launch-by-launch route, follows new inputs and new weights, and a batch outside the
     fp16 range falls through to the launch-by-launch route (which re-runs the chunk on the tf32-split program)."""
@@ -225,9 +225,9 @@ def test_small_image_batches_replay_one_graph():
     finally:
         flows.SMALL_BATCH_GRAPH_IMAGES = old
     prog, _ = flow._program("backward")
-    assert torch.equal(flow.log_prob(x), want) and len(prog.__dict__.get("_lp_graphs", {})) == 1
+    assert torch.equal(flow.log_prob(x), want) and sum(k[0] == "small" for k in prog.__dict__.get("_graphs", {})) == 1
     assert torch.equal(flow.log_prob(x.flip(0)), want2)                 # replay on new inputs
-    assert torch.equal(flow.log_prob(x[:7]), want[:7]) and len(prog.__dict__["_lp_graphs"]) == 2
+    assert torch.equal(flow.log_prob(x[:7]), want[:7]) and sum(k[0] == "small" for k in prog._graphs) == 2
     big = x.clone()
     big[3] *= 1e6
     lp_big = flow.log_prob(big)

@@ -149,7 +149,7 @@ def test_chunking_and_host_path_do_not_change_results():
     assert torch.equal(lp_ref.cpu(), lp_host)
 
 
-def test_host_path_growing_chunk_schedule_is_bit_identical():
+def test_host_path_growing_chunk_schedule_replays_bit_identical():
     """`log_prob_host` streams a growing chunk schedule (first copy small, later chunks larger), one captured CUDA graph
     per (staging buffer, chunk size): same bits as the device-resident pass, also on replay and for other row counts."""
     spec, params, arr = load_case("d100_h50_hh")
@@ -161,13 +161,13 @@ def test_host_path_growing_chunk_schedule_is_bit_identical():
     assert torch.equal(flow.log_prob_host(xp), want)
     assert torch.equal(flow.log_prob_host(xp), want)                          # graph replay
     prog, _ = flow._program("backward")
-    assert len({k[2] for k in prog._host_graphs}) >= 2                        # more than one chunk size was captured
+    assert len({k[3] for k in prog._graphs if k[0] == "host"}) >= 2          # more than one chunk size was captured
     assert torch.equal(flow.log_prob_host(xp[:45001]), want[:45001])          # other schedule, cached + new graphs
     assert torch.equal(flow.log_prob_host(xp, chunk_rows=8192), want)         # explicit uniform chunks
     assert torch.equal(flow.log_prob_host(xp), want)
 
 
-def test_graph_caches_follow_the_weight_version():
+def test_graph_cache_follows_the_weight_version():
     """ADVICE r1 (high): captured graphs hold raw pointers into a Program's operand planes, so they must die with it.
     Alternate in-place weight updates with `log_prob_host` / small-batch `log_prob` (both replay captured graphs) and
     compare with the launch-by-launch pass of the same weight version."""
@@ -197,8 +197,57 @@ def test_graph_caches_follow_the_weight_version():
         assert torch.equal(flow.log_prob_host(xp), want), it
         assert torch.equal(flow.log_prob(xs), want_small), it
         assert torch.equal(flow.log_prob_host(xp), want), it
-        assert all(k[0] in range(8) for k in prog._host_graphs)
-    assert not hasattr(flow, "_host_graphs") and not hasattr(flow, "_lp_graphs")
+        assert all(k[1] in range(8) for k in prog._graphs if k[0] == "host")
+    assert not hasattr(flow, "_graphs")
+
+
+def test_each_kind_of_host_call_captures_once(monkeypatch):
+    """fp32 and 8-bit `log_prob_host`, fp32 and quantised `sample_host` and the small-batch `log_prob` in turn keep each
+    other's captured graphs and staging buffers: only the first call of each kind captures, later ones replay with the same
+    result.  A first flow of the same shapes sizes the process-wide workspaces, whose growth would invalidate every graph."""
+    from usflows_b200 import flows
+    spec, params, _ = load_case("d100_h50_hh")
+    x = torch.rand(70000, 100, generator=torch.Generator().manual_seed(13))
+    xp, xq, xs = x.pin_memory(), (x * 256).to(torch.uint8).pin_memory(), x[:700].cuda()
+    kinds = {"host": lambda f: f.log_prob_host(xp), "host_u8": lambda f: f.log_prob_host(xq, dequantize="uniform", seed=5),
+             "sample": lambda f: f.sample_host(70000, seed=3), "sample_q": lambda f: f.sample_host(70000, seed=3, quantize=True),
+             "small": lambda f: f.log_prob(xs)}
+    order = ["host", "host_u8", "host", "host_u8", "sample", "sample_q", "sample", "small", "small"]
+    warm = build_flow(spec, params)
+    for kind in order:
+        kinds[kind](warm)
+    flow = build_flow(spec, params)
+    capture, n = flows._capture, [0]
+
+    def counting(dev, body):
+        n[0] += 1
+        return capture(dev, body)
+    monkeypatch.setattr(flows, "_capture", counting)
+    first = {}
+    for kind in order:
+        before = n[0]
+        out = kinds[kind](flow).clone()
+        if kind in first:
+            assert n[0] == before and torch.equal(out, first[kind]), kind
+        else:
+            assert n[0] > before, kind
+            first[kind] = out
+
+
+def test_weights_outside_the_fp16_range_stream_through_graphs_of_the_tf32_split():
+    """A conditioner weight past the fp16 range (one hidden layer rescaled, the function unchanged): the "fp32" program
+    always runs as its tf32-split program, and `log_prob_host` replays captured graphs of that program."""
+    spec, params, _ = load_case("d100_h50_hh")
+    c = "trainable_layers.1.conditioner.layers."
+    params = dict(params, **{c + "1.weight": params[c + "1.weight"] * 1e6, c + "1.bias": params[c + "1.bias"] * 1e6,
+                             c + "2.weight": params[c + "2.weight"] * 1e-6})
+    f16, tf = build_flow(spec, params, precision="fp32"), build_flow(spec, params, precision="fp32_tf32")
+    prog, _ = f16._program("backward")
+    assert prog.force_fallback
+    x = torch.rand(70000, 100, generator=torch.Generator().manual_seed(14)).pin_memory()
+    got = f16.log_prob_host(x)
+    assert any(k[0] == "host" for k in prog._fallback().__dict__.get("_graphs", {}))
+    assert torch.isfinite(got).all() and torch.equal(got, tf.log_prob_host(x))
 
 
 def test_row_shard_driver_matches_the_single_device_pass():

@@ -30,7 +30,7 @@ for chunk in (None, 9472, 18944, 16384):
 from usflows_b200 import _lib
 for pdl in (0, 1):
     _lib.load().usf_debug_set_pdl(pdl)
-    flow._host_graphs = {}                                  # re-capture with / without programmatic edges
+    flow._program("backward")[0]._graphs.clear()            # re-capture with / without programmatic edges
     ms_dev = timed(lambda: flow.log_prob(x))
     ms = timed(lambda: flow.log_prob_host(x_host, out_host))
     print(f"pdl={pdl}: device log_prob {ms_dev:.3f} ms, log_prob_host {ms:.3f} ms = {rows/ms/1e3:.2f} M rows/s")

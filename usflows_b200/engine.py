@@ -324,6 +324,12 @@ class ProgramCore:
             self._fallback_prog = self._in_mode("fp32_tf32")
         return self._fallback_prog
 
+    @property
+    def guarded(self) -> bool:
+        """Chunks run launch by launch on fp16 split planes under a range flag (the single-launch program has none, the
+        always-tf32-split one needs none)."""
+        return self.uses_range_flag and self.small is None and not self.force_fallback
+
     def run(self, x: torch.Tensor, *, out: Optional[torch.Tensor] = None, sink=None, chunk_rows: Optional[int] = None,
             ladj_rows: Optional[torch.Tensor] = None, dq: Optional[ops.Dequant] = None) -> Optional[torch.Tensor]:
         """Evaluate the program on x [rows, d] chunk by chunk into `out` (allocated when None).  With `sink`, the result of

@@ -113,20 +113,71 @@ def _wave_aligned_chunk_rows(prog, device) -> int:
     return 256 * unit * k
 
 
+def _uniform_bounds(n: int, step: int):
+    """Chunks of `step` rows from the start; the last one takes the rest."""
+    return [(r0, min(n, r0 + step)) for r0 in range(0, n, step)]
+
+
+def growing_bounds(n: int, unit: int, units):
+    """Chunks of `log_prob_host`: `units` (the last entry repeats) in multiples of `unit` rows from the start.  Its H2D copy
+    of chunk i+1 hides under the kernels of chunk i (a row copies faster than it computes), so only the FIRST copy is
+    exposed: start with the smallest wave-aligned chunk and let the later ones grow (fewer kernel boundaries, fuller
+    tails).  Fewer than unit // 2 rows left join the last chunk instead of making a launch sequence of their own."""
+    bounds, r0 = [], 0
+    while r0 < n:
+        take = min(unit * units[min(len(bounds), len(units) - 1)], n - r0)
+        if n - r0 - take < unit // 2:
+            take = n - r0
+        bounds.append((r0, r0 + take))
+        r0 += take
+    return bounds
+
+
 def sample_host_bounds(n: int, unit: int, uniform: bool = False):
-    """Chunks of `sample_host`.  There the LAST device-to-host copy is the exposed one (the reverse of `log_prob_host`), so
-    the chunks shrink towards the end: HOST_CHUNK_UNITS read from the end, in wave-aligned units; the first chunk takes the
-    remainder.  `uniform`: chunks of `unit` rows from the start."""
+    """Chunks of `sample_host`.  There the LAST device-to-host copy is the exposed one, so the chunks are those of
+    `log_prob_host` mirrored: they shrink towards the end, and the first chunk takes the remainder.  `uniform`: chunks of
+    `unit` rows from the start."""
     if uniform:
-        return [(r0, min(n, r0 + unit)) for r0 in range(0, n, unit)]
-    bounds, r1 = [], n
-    while r1 > 0:
-        take = min(unit * HOST_CHUNK_UNITS[min(len(bounds), len(HOST_CHUNK_UNITS) - 1)], r1)
-        if r1 - take < unit // 2:                 # do not leave a sliver for a launch sequence of its own
-            take = r1
-        bounds.append((r1 - take, r1))
-        r1 -= take
-    return bounds[::-1]
+        return _uniform_bounds(n, unit)
+    return [(n - r1, n - r0) for r0, r1 in reversed(growing_bounds(n, unit, HOST_CHUNK_UNITS))]
+
+
+def _cached_graph(prog, key, build) -> dict:
+    """The graph entry of `key` = (route, slot, staging buffer data_ptr, rows, variant) from `build()` (the graph, its range
+    `flag` and the buffers a replay uses), unless one captured since the last workspace reallocation (`gen`) is cached.  On
+    insert, stale entries and those of the same (route, slot, variant) over another buffer go; at most 8 stay per (route,
+    slot).  The cache lives ON the Program (one per weight version and mode): graphs point into its operand planes and die
+    with it instead of surviving under a recycled id()."""
+    cache = prog.__dict__.setdefault("_graphs", {})
+    ent = cache.get(key)
+    if ent is not None and ent["gen"] == engine._workspace.generation:
+        return ent
+    ent = build()
+    ent["gen"] = engine._workspace.generation
+    for k in [k for k, e in cache.items() if e["gen"] != ent["gen"] or (k[:2] == key[:2] and k[4] == key[4] and k[2] != key[2])]:
+        del cache[k]
+    while sum(1 for k in cache if k[:2] == key[:2]) >= 8:        # a few row counts per staging slot; drop the oldest
+        del cache[next(k for k in cache if k[:2] == key[:2])]
+    cache[key] = ent
+    return ent
+
+
+def _capture_chunks(bounds, n_slots: int, unit: int, capture) -> dict:
+    """{(slot, rows): capture(slot, rows)} for every chunk i of `bounds` of at least unit // 2 rows, with slot = i % n_slots.
+    Largest first, so that the shared workspaces are sized once; a second pass recaptures what a workspace that grew
+    meanwhile invalidated.  The flags are zeroed at the end: the eager pass of a capture may have set them."""
+    sizes = [r1 - r0 for r0, r1 in bounds]
+    graphs = {}
+    for _ in range(2):
+        for i in sorted(range(len(sizes)), key=lambda j: -sizes[j]):
+            if sizes[i] >= unit // 2:
+                graphs[(i % n_slots, sizes[i])] = capture(i % n_slots, sizes[i])
+        if all(g["gen"] == engine._workspace.generation for g in graphs.values()):
+            break
+    for g in graphs.values():
+        if g["flag"] is not None:
+            g["flag"].zero_()
+    return graphs
 
 
 class Flow(torch.nn.Module):
@@ -328,14 +379,10 @@ class Flow(torch.nn.Module):
         encoding), not by the kernels: the launch program + base density of a given row count is captured ONCE into a CUDA
         graph over fixed staging buffers and replayed (input copied in, result cloned out).  Returns None when a value
         left the fp16 range (the caller then takes the launch-by-launch route, which handles the tf32-split re-run)."""
-        # the cache lives ON the Program (one Program per weight version and mode): graphs of a replaced weight version die
-        # with their Program instead of surviving under a recycled id() with dangling operand pointers
-        cache = prog.__dict__.setdefault("_lp_graphs", {})
         rows, d = x2.shape
         dev = x2.device
-        key = (rows, str(dev))
-        ent = cache.get(key)
-        if ent is None or ent["gen"] != engine._workspace.generation:
+
+        def build():
             base = self._base_module()
             base._prepared()                  # parameter-side work happens here, outside any graph capture
             xin = torch.empty(rows, d, dtype=torch.float32, device=dev)
@@ -346,13 +393,10 @@ class Flow(torch.nn.Module):
             def body():
                 prog._run_chunk(xin, fin, flag)
                 base._density_into(ops.Act(rows, fin.shape[1], f32=fin), -ladj, out, perm=perm)
-            with torch.no_grad():
-                xin.copy_(x2)
-                graph = _capture(dev, body)
-            if len(cache) >= 8:                               # a few row counts per weight version; drop the oldest
-                cache.pop(next(iter(cache)))
-            ent = cache[key] = dict(graph=graph, x=xin, out=out, flag=flag, gen=engine._workspace.generation)
+            xin.copy_(x2)
+            return dict(graph=_capture(dev, body), x=xin, out=out, flag=flag)
         with torch.no_grad():
+            ent = _cached_graph(prog, ("small", None, None, rows, None), build)
             ent["x"].copy_(x2)
             if ent["flag"] is not None:
                 ent["flag"].zero_()
@@ -361,27 +405,21 @@ class Flow(torch.nn.Module):
                 return None
             return ent["out"].clone()
 
-    def _chunk_graph(self, prog, slot: int, buf: torch.Tensor, d: int, dq_mode: Optional[str] = None) -> dict:
-        """CUDA graph of the launch program of one full-size chunk reading host-staging buffer `slot`.  With `dq_mode`, the
-        buffer holds 8-bit rows; the graph reads their {seed, global row} from its `params` tensor, written before a replay."""
-        cache = prog.__dict__.setdefault("_host_graphs", {})     # on the Program: see _log_prob_small_batch
-        key = (slot, buf.data_ptr(), tuple(buf.shape), dq_mode)
-        ent = cache.get(key)
-        if ent is not None and ent["gen"] == engine._workspace.generation:
-            return ent
-        dev = buf.device
-        flag = torch.zeros(1, dtype=torch.int32, device=dev) if prog.uses_range_flag else None
-        fin = prog.final_buffer(dev, f"final_host{slot}", buf.shape[0], d)
-        params = None if dq_mode is None else torch.zeros(2, dtype=torch.int64, device=dev)
-        dq = None if dq_mode is None else ops.Dequant(dq_mode, 0, 0, params)
-        graph = _capture(dev, lambda: prog._run_chunk(buf, fin, flag, dq))
-        ent = dict(graph=graph, fin=fin, flag=flag, params=params, gen=engine._workspace.generation)
-        for k in [k for k in cache if k[0] == slot and ((k[1] != key[1] and k[3] == dq_mode) or cache[k]["gen"] != ent["gen"])]:
-            del cache[k]                                  # graphs of a replaced staging buffer / of stale workspaces
-        while sum(1 for k in cache if k[0] == slot) >= 6:  # a few chunk sizes per staging buffer; drop the oldest
-            del cache[next(k for k in cache if k[0] == slot)]
-        cache[key] = ent
-        return ent
+    def _staging(self, name: str, rows: int, width: int, dtype: torch.dtype, dev) -> torch.Tensor:
+        """The device buffer [>= rows, width] this flow keeps for `name` and `dtype` (fp32 and 8-bit calls in turn keep their
+        own buffers, and the graphs captured over them); reallocated when it has too few rows, another width or device."""
+        bufs = self.__dict__.setdefault("_stage", {})
+        buf = bufs.get((name, dtype))
+        if buf is None or buf.shape[0] < rows or buf.shape[1] != width or buf.device != dev:
+            buf = bufs[(name, dtype)] = torch.empty(rows, width, dtype=dtype, device=dev)
+        return buf
+
+    def _side_stream(self, dev) -> "torch.cuda.Stream":
+        """The stream the host copies of `log_prob_host` / `sample_host` run on, under the kernels of the next chunk."""
+        s = self.__dict__.get("_side")
+        if s is None or s.device != dev:
+            s = self._side = torch.cuda.Stream(device=dev)
+        return s
 
     def log_prob_host(self, x_host: torch.Tensor, out_host: Optional[torch.Tensor] = None,
                       chunk_rows: Optional[int] = None, *, dequantize: Optional[str] = None, seed: Optional[int] = None,
@@ -409,61 +447,41 @@ class Flow(torch.nn.Module):
                                                            None if dq is None else dq.shifted(r0)))
             return out
         prog, ladj = self._program("backward", self._zero_ctx)
+        prog = prog._fallback() if prog.force_fallback else prog
         base = self._base_module()
         base._prepared()                  # parameter-side work happens here, outside any graph capture
         x2 = x_host.reshape(-1, math.prod(self._event_shape()))
         rows, d = x2.shape
         if out_host is None:
             out_host = torch.empty(rows, dtype=torch.float32, pin_memory=True)
-        # 8-bit rows are staged as they are (a quarter of the bytes), in a buffer of their own: fp32 and uint8 calls in turn
-        # keep their staging buffers and captured graphs
-        sdt, attr = (torch.float32, "_host_stage") if dq is None else (torch.uint8, "_host_stage_u8")
+        sdt = torch.float32 if dq is None else torch.uint8      # 8-bit rows are staged as they are (a quarter of the bytes)
         images = len(self._event_shape()) == 3
         if images:
             # image-shaped events: uniform chunks in two staging buffers in turn, each through `_log_prob` (whose routes
             # guard their own chunks); the H2D copy of chunk i + 1 is issued before chunk i is enqueued
-            step = max(1, chunk_rows or HOST_CHUNK_ROWS)
-            bounds = [(r0, min(rows, r0 + step)) for r0 in range(0, rows, step)]
+            bounds = _uniform_bounds(rows, max(1, chunk_rows or HOST_CHUNK_ROWS))
             whole, ahead = False, 1
         else:
-            # Chunk schedule.  The H2D copy of chunk i+1 hides under the kernels of chunk i (a row copies faster than it
-            # computes), so only the FIRST copy is exposed: start with the smallest wave-aligned chunk and let the later
-            # ones grow (fewer kernel boundaries, fuller tails).  An explicit `chunk_rows` gives uniform chunks.
+            # an explicit `chunk_rows` gives uniform chunks
             unit = min(chunk_rows or _wave_aligned_chunk_rows(prog, dev), max(rows, 1))
-            bounds, r0 = [], 0
-            while r0 < rows:
-                mult = 1 if chunk_rows else HOST_CHUNK_UNITS[min(len(bounds), len(HOST_CHUNK_UNITS) - 1)]
-                take = min(unit * mult, rows - r0)
-                if rows - r0 - take < unit // 2:         # do not leave a sliver for a last launch sequence
-                    take = rows - r0
-                bounds.append((r0, r0 + take))
-                r0 += take
+            bounds = growing_bounds(rows, unit, (1,) if chunk_rows else HOST_CHUNK_UNITS)
             # staging: one device buffer per chunk (slices of one allocation holding the whole batch) when that fits -- the
             # copies then run back to back on the copy stream, independent of the kernels --, else two buffers used in turn
             whole = rows * d * sdt.itemsize <= HOST_STAGE_BYTES and len(bounds) <= HOST_MAX_STAGE_SLICES
             ahead = 0
-        sizes = [r1 - r0 for r0, r1 in bounds]
-        chunk = max(sizes, default=1)
-        need = max(rows, 1) if whole else 2 * chunk
-        stage = getattr(self, attr, None)
-        if stage is None or stage.shape[0] < need or stage.shape[1] != d or stage.device != dev:
-            stage = torch.empty(need, d, dtype=sdt, device=dev)
-            setattr(self, attr, stage)
-            self._host_out = torch.empty(0, dtype=torch.float32, device=dev)
-            self._copy_stream = torch.cuda.Stream(device=dev)
+        chunk = max([r1 - r0 for r0, r1 in bounds], default=1)
+        stage = self._staging("host", max(rows, 1) if whole else 2 * chunk, d, sdt, dev)
         if whole:
             bufs = [stage[r0:r1] for r0, r1 in bounds] or [stage[:0]]
         else:
             bufs = [stage[:chunk], stage[chunk:2 * chunk]]
         n_buf = len(bufs)
-        if self._host_out.numel() < rows:
-            self._host_out = torch.empty(rows, dtype=torch.float32, device=dev)
-        out_dev = self._host_out[:rows]
+        out_dev = self._staging("out", rows, 1, torch.float32, dev).view(-1)[:rows]
+        side = self._side_stream(dev)
         main = torch.cuda.current_stream(dev)
         copied = [torch.cuda.Event() for _ in range(n_buf)]
         consumed = [torch.cuda.Event() for _ in range(n_buf)]
-        # chunks run `_run_chunk` under a range flag; the single-launch and the always-tf32-split programs have none
-        guarded = not images and prog.uses_range_flag and prog.small is None and not prog.force_fallback
+        guarded = not images and prog.guarded
         row_ladj = torch.zeros(rows, dtype=torch.float32, device=dev) if prog.has_row_ladj else None
         lr = lambda r0, r1: None if row_ladj is None else row_ladj[r0:r1]     # noqa: E731
         shifted = lambda r0: None if dq is None else dq.shifted(r0)           # noqa: E731
@@ -474,11 +492,24 @@ class Flow(torch.nn.Module):
         def issue_copy(i):
             r0, r1 = bounds[i]
             slot = i % n_buf
-            with torch.cuda.stream(self._copy_stream):
+            with torch.cuda.stream(side):
                 if i >= n_buf:
-                    self._copy_stream.wait_event(consumed[slot])
+                    side.wait_event(consumed[slot])
                 bufs[slot][:r1 - r0].copy_(x2[r0:r1], non_blocking=True)
-                copied[slot].record(self._copy_stream)
+                copied[slot].record(side)
+
+        def capture(slot, size):
+            """The launch program of one chunk reading staging buffer `slot`.  With `dq`, the buffer holds 8-bit rows; the
+            graph reads their {seed, global row} from its `params` tensor, written before every replay."""
+            buf = bufs[slot][:size]
+
+            def build():
+                flag = torch.zeros(1, dtype=torch.int32, device=dev) if prog.uses_range_flag else None
+                fin = prog.final_buffer(dev, f"final_host{slot}", size, d)
+                params = None if dq is None else torch.zeros(2, dtype=torch.int64, device=dev)
+                dqg = None if dq is None else ops.Dequant(dq.mode, 0, 0, params)
+                return dict(graph=_capture(dev, lambda: prog._run_chunk(buf, fin, flag, dqg)), fin=fin, flag=flag, params=params)
+            return _cached_graph(prog, ("host", slot, buf.data_ptr(), size, None if dq is None else dq.mode), build)
 
         def first(i, r0, r1, flag):
             if i + ahead < len(bounds):
@@ -512,22 +543,11 @@ class Flow(torch.nn.Module):
 
         with torch.no_grad():
             graphs = {}
-            if not images and HOST_CUDA_GRAPHS and not prog.force_fallback and rows >= unit and prog.small is None \
-                    and not prog.has_row_ladj:
-                # one graph per (staging buffer, chunk size), largest first so that the shared workspaces are sized once
-                for _ in range(2):                        # a workspace that grew while capturing invalidates earlier graphs
-                    for i in sorted(range(len(sizes)), key=lambda j: -sizes[j]):
-                        if sizes[i] >= unit // 2:
-                            graphs[(i % n_buf, sizes[i])] = self._chunk_graph(prog, i % n_buf, bufs[i % n_buf][:sizes[i]], d,
-                                                                              None if dq is None else dq.mode)
-                    if all(g["gen"] == engine._workspace.generation for g in graphs.values()):
-                        break
-                for g in graphs.values():
-                    if g["flag"] is not None:
-                        g["flag"].zero_()
+            if not images and HOST_CUDA_GRAPHS and rows >= unit and prog.small is None and not prog.has_row_ladj:
+                graphs = _capture_chunks(bounds, n_buf, unit, capture)
             if graphs and dq is not None:                 # {seed, global row} of every chunk, read by the graphs' ingest
                 params = torch.tensor([[dq.seed, dq.row0 + r0] for r0, _ in bounds], dtype=torch.int64).to(dev)
-            self._copy_stream.wait_stream(main)
+            side.wait_stream(main)
             if ahead and bounds:
                 issue_copy(0)
             # a graph's flag is not per chunk: when one is set, every chunk is recomputed
@@ -597,35 +617,6 @@ class Flow(torch.nn.Module):
                 self._sample_host(out_host.view(n, -1), draw, quantize, chunk_rows)
         return out_host
 
-    def _sample_graph(self, prog, base, slot: int, buf: torch.Tensor, quantize: bool) -> dict:
-        """CUDA graph of one full-size chunk of `sample_host` writing output buffer `slot`: the base draws at the {seed, row
-        base} read from its `params` tensor (written before a replay), the launch program, the quantisation."""
-        cache = prog.__dict__.setdefault("_sample_graphs", {})   # on the Program: see _log_prob_small_batch
-        rows, d = buf.shape
-        key = (slot, buf.data_ptr(), rows, quantize)
-        ent = cache.get(key)
-        if ent is not None and ent["gen"] == engine._workspace.generation:
-            return ent
-        dev = buf.device
-        flag = torch.zeros(1, dtype=torch.int32, device=dev) if prog.uses_range_flag else None
-        params = torch.zeros(2, dtype=torch.int64, device=dev)
-        z = engine._workspace.planes(dev, f"sample_z{slot}", 1, rows * d, "f32").view(rows, d)
-        fin = prog.final_buffer(dev, f"final_q{slot}", rows, d) if quantize else buf
-        draw = ops.Draw(0, 0, params)
-
-        def body():
-            base._sample_into(z, draw)
-            prog._run_chunk(z, fin, flag)
-            if quantize:
-                ops.quantize_u8(fin, buf)
-        ent = dict(graph=_capture(dev, body), flag=flag, params=params, gen=engine._workspace.generation)
-        for k in [k for k in cache if cache[k]["gen"] != ent["gen"] or (k[0] == slot and k[1] != key[1] and k[3] == quantize)]:
-            del cache[k]                                  # graphs of stale workspaces / of a replaced output buffer
-        while len(cache) >= 8:                            # a few chunk sizes per buffer; drop the oldest
-            del cache[next(iter(cache))]
-        cache[key] = ent
-        return ent
-
     def _sample_host(self, flat: torch.Tensor, draw: ops.Draw, quantize: bool, chunk_rows: Optional[int]) -> None:
         dev = next(self.parameters()).device
         cuda = dev.type == "cuda"
@@ -633,27 +624,22 @@ class Flow(torch.nn.Module):
         base = self._base_module()
         base._prepared()                  # parameter-side work happens here, outside any graph capture
         prog = None if self._layer_route else self._program("forward", self._zero_ctx)[0]
-        images = isinstance(prog, image_engine.ImageProgram)
-        launch = prog is not None and not images and prog.small is None       # the flat launch program, chunk by chunk
         if prog is not None and prog.force_fallback:
             prog = prog._fallback()
+        images = isinstance(prog, image_engine.ImageProgram)
+        launch = prog is not None and not images and prog.small is None       # the flat launch program, chunk by chunk
         if launch:
             unit = min(chunk_rows or _wave_aligned_chunk_rows(prog, dev), n)
             bounds = sample_host_bounds(n, unit, uniform=bool(chunk_rows))
         else:                             # images: eager chunks; single-launch and layer-route flows: plain chunks
-            step = chunk_rows or (prog._chunk_bounds(n, None)[0][1] if images else HOST_CHUNK_ROWS)
-            bounds = [(r0, min(n, r0 + step)) for r0 in range(0, n, step)]
+            bounds = _uniform_bounds(n, chunk_rows or (prog._chunk_bounds(n, None)[0][1] if images else HOST_CHUNK_ROWS))
         chunk = max(r1 - r0 for r0, r1 in bounds)
         # two output buffers used in turn; fp32 and uint8 calls in turn keep their own buffers and captured graphs
-        attr = "_sample_stage_u8" if quantize else "_sample_stage"
-        stage = getattr(self, attr, None)
-        if stage is None or stage.shape[1] < chunk or stage.shape[2] != d or stage.device != dev:
-            stage = torch.empty(2, chunk, d, dtype=flat.dtype, device=dev)
-            setattr(self, attr, stage)
-        if cuda and (getattr(self, "_sample_stream", None) is None or self._sample_stream.device != dev):
-            self._sample_stream = torch.cuda.Stream(device=dev)
+        stage = self._staging("sample", 2 * chunk, d, flat.dtype, dev)
+        half = stage.shape[0] // 2
+        bufs = [stage[:half], stage[half:2 * half]]
         main = torch.cuda.current_stream(dev) if cuda else None
-        side = self._sample_stream if cuda else None
+        side = self._side_stream(dev) if cuda else None
         ready = [torch.cuda.Event() for _ in range(2)] if cuda else None
         copied = [torch.cuda.Event() for _ in range(2)] if cuda else None
         issued = [0]
@@ -663,7 +649,7 @@ class Flow(torch.nn.Module):
             next use waits for that copy."""
             slot = issued[0] % 2
             issued[0] += 1
-            buf = stage[slot][:r1 - r0]
+            buf = bufs[slot][:r1 - r0]
             if not cuda:
                 run(buf)
                 flat[r0:r1].copy_(buf)
@@ -696,18 +682,29 @@ class Flow(torch.nn.Module):
             if quantize:
                 ops.quantize_u8(fin, buf)
 
+        def capture(slot, rows):
+            """One chunk writing output buffer `slot`: the base draws at the {seed, row base} read from its `params` tensor
+            (written before every replay), the launch program, the quantisation."""
+            buf = bufs[slot][:rows]
+
+            def build():
+                flag = torch.zeros(1, dtype=torch.int32, device=dev) if prog.uses_range_flag else None
+                params = torch.zeros(2, dtype=torch.int64, device=dev)
+                z = engine._workspace.planes(dev, f"sample_z{slot}", 1, rows * d, "f32").view(rows, d)
+                fin = prog.final_buffer(dev, f"final_q{slot}", rows, d) if quantize else buf
+                dr = ops.Draw(0, 0, params)
+
+                def body():
+                    base._sample_into(z, dr)
+                    prog._run_chunk(z, fin, flag)
+                    if quantize:
+                        ops.quantize_u8(fin, buf)
+                return dict(graph=_capture(dev, body), flag=flag, params=params)
+            return _cached_graph(prog, ("sample", slot, buf.data_ptr(), rows, quantize), build)
+
         graphs = {}
-        if cuda and launch and HOST_CUDA_GRAPHS and not prog.force_fallback and n >= unit:
-            sizes = [r1 - r0 for r0, r1 in bounds]
-            for _ in range(2):                            # a workspace that grew while capturing invalidates earlier graphs
-                for i in sorted(range(len(sizes)), key=lambda j: -sizes[j]):
-                    if sizes[i] >= unit // 2:
-                        graphs[(i % 2, sizes[i])] = self._sample_graph(prog, base, i % 2, stage[i % 2][:sizes[i]], quantize)
-                if all(g["gen"] == engine._workspace.generation for g in graphs.values()):
-                    break
-            for g in graphs.values():
-                if g["flag"] is not None:
-                    g["flag"].zero_()
+        if cuda and launch and HOST_CUDA_GRAPHS and n >= unit:
+            graphs = _capture_chunks(bounds, 2, unit, capture)
             wrap = lambda v: (v + 2**63) % 2**64 - 2**63                     # noqa: E731  (uint64 bits as int64)
             params = torch.tensor([[wrap(draw.seed), draw.row0 + r0] for r0, _ in bounds], dtype=torch.int64).to(dev)
 
@@ -725,11 +722,11 @@ class Flow(torch.nn.Module):
         def again(i, r0, r1):                             # the same rows of the noise on the tf32-split program
             emit(r0, r1, lambda buf: compute(prog._fallback(), buf, r0, r1, None))
 
-        guarded = prog is not None and prog.small is None and prog.uses_range_flag and not prog.force_fallback
         if cuda:
             side.wait_stream(main)
         # a graph's flag is not per chunk: when one is set, every chunk is recomputed
-        engine.run_chunks(bounds, dev, guarded, first, again, shared_flags=[g["flag"] for g in graphs.values()])
+        engine.run_chunks(bounds, dev, prog is not None and prog.guarded, first, again,
+                          shared_flags=[g["flag"] for g in graphs.values()])
         if cuda:
             side.synchronize()
 

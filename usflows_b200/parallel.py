@@ -26,8 +26,7 @@ import torch
 
 from . import engine, ops
 
-_UNCOPIED = ("_programs", "_host_stage", "_host_stage_u8", "_host_out", "_copy_stream", "_cl_perm",
-             "_cl_perm_key", "_sharded", "_sample_stage", "_sample_stage_u8", "_sample_stream")
+_UNCOPIED = ("_programs", "_stage", "_side", "_cl_perm", "_cl_perm_key", "_sharded")
 
 
 def shard_bounds(n: int, rank: int, world: int):
